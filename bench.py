@@ -2,6 +2,7 @@
 """bench.py — game-steps/sec of the batched Hironaka env step on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this engine
+    python bench.py ... --dump-outputs DIR                          # also write the last timed step's outputs
     python bench.py --impl reference [--gpus N] [--steps K] ...     # CPU arm: the unmodified reference (baseline/_ref)
     torchrun --nproc-per-node N ... bench.py --gpus N ...           # one rank per GPU
 
@@ -40,6 +41,7 @@ GAMES_PER_GPU = 1 << 20
 CPU_SAMPLE_GAMES = int(os.environ.get("HK_BENCH_CPU_SAMPLE", 1 << 19))  # bounded sample of the C2 workload for the C port (state 126 MB, ~1 s per 40 steps)
 REF_SAMPLE_GAMES = int(os.environ.get("HK_BENCH_REF_SAMPLE", 1 << 14))  # games per step of the real reference (its [B,N,N,d] temporaries: 79 MB each)
 MAX_RESIDENT_ROLLOUTS = 10  # distinct pre-generated batches; beyond K = 200 they are restored from pristine copies
+DUMP_SAMPLE_GAMES = 1 << 17  # games whose state --dump-outputs writes (31.5 MB of float32)
 BYTES_PER_GAME_STEP = 8 * N_POINTS * DIM + 13  # SURVEY.md 8(d): int32 state r+w, 2 x int32 action, u8 done, f32 reward
 OPS_PER_GAME_STEP = N_POINTS * (N_POINTS - 1) * (DIM + 1) + 3 * N_POINTS * DIM + N_POINTS
 
@@ -302,6 +304,8 @@ def run_gpu_arm(args):
     barrier()
     total_ms = ev[0].elapsed_time(ev[K])
     per_launch_ms = [ev[i].elapsed_time(ev[i + 1]) for i in range(K)]
+    # what the last timed step returned (batch r), read back before the launches below overwrite done / reward
+    outputs = last_step_outputs(torch, batches[r].points, done, reward) if args.dump_outputs and rank == 0 else None
     # keep the device busy a little longer so that NVML has samples under load
     t_end = time.perf_counter() + 0.4
     i = 0
@@ -388,10 +392,26 @@ def run_gpu_arm(args):
         "cpu_baseline": cpu, "e2e": e2e, "gpu_launches": K, "clocks": clocks,
         "library": os.path.relpath(hb.LIB_PATH, ROOT), "collective": collective, "secondary": secondary,
     }
+    if outputs is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
     return 0
+
+
+def last_step_outputs(torch, points, done, reward) -> dict:
+    """What a caller of the timed step receives, as float32 host arrays for --dump-outputs: the per-game done
+    flags and rewards in full, and the new state of a fixed, seeded sample of DUMP_SAMPLE_GAMES games with their
+    indices (the whole state, 252 MB, exceeds the 64 MB a dump may take)."""
+    games = np.sort(np.random.default_rng(0).choice(points.shape[0], DUMP_SAMPLE_GAMES, replace=False))
+    sample = points.index_select(0, torch.from_numpy(games).to(points.device))
+    out = {"points": sample.cpu().numpy().astype(np.float32), "points_games": games.astype(np.float64),
+           "done": done.cpu().numpy().astype(np.float32), "reward": reward.cpu().numpy().astype(np.float32)}
+    assert sum(a.nbytes for a in out.values()) <= 64_000_000
+    return out
 
 
 def executed_issue(avg_launch_s):
@@ -934,10 +954,15 @@ def main():
     ap.add_argument("--no-secondary", action="store_true", help="skip the other BASELINE configs (profiling runs)")
     ap.add_argument("--no-pdl", action="store_true", help="disable programmatic dependent launch (A/B tuning)")
     ap.add_argument("--no-collective", action="store_true", help="skip the rollout all-gather leg (N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed on rank 0 (done, reward, a seeded sample of the "
+                         "new states) as DIR/<name>.npy, to compare builds output for output")
     args = ap.parse_args()
     if args.steps < 1:
         raise SystemExit("--steps must be >= 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes the GPU arm's outputs; --impl reference has none")
         return run_reference_arm(args)
     return run_gpu_arm(args)
 

@@ -164,19 +164,36 @@ def test_bench_reference_arm_runs_on_cpu():
         assert k in line
 
 
-def test_reference_arm_matches_the_oracle():
+def test_reference_arm_matches_the_oracle(golden_dir):
     """Parity gate of the reference arm (BASELINE.md section 3): what bench.py times as "the reference" — the
-    unmodified hironaka.core.TensorPoints from baseline/_ref playing the bench's own C2 inputs — gives, step by
-    step, the states, done flags and rewards of the oracle's torch flavour on the same inputs (the GPU arm is
-    held to the same oracle by tests/test_gpu_parity.py, and to this arm directly by
-    test_reference_arm_matches_the_gpu)."""
+    unmodified hironaka.core.TensorPoints playing C2 random games, shift -> reposition -> newton ->
+    ended_batch_in_tensor -> reward — gives, step by step, the states, done flags and rewards of the oracle's torch
+    flavour on the same inputs (the GPU arm is held to the same oracle by tests/test_gpu_parity.py, and to this arm
+    directly by test_reference_arm_matches_the_gpu).  The reference's side is stored: ref_rollout_c2_20x3*.npz,
+    recorded from the unmodified reference by oracle/gen_golden.py (rollout_torch plays that composition), tiled
+    here to 1024 games.  Where baseline/_ref is installed, the live reference also plays the bench's own inputs."""
     from baseline import reference_arm as R
+    from oracle import cport, hk_oracle as O
+    flags = O.F_NOOP_INVALID | O.F_FREEZE_ENDED | O.F_ACT_DISCRETE
+    for name in ("c2_20x3", "c2_20x3_repos"):
+        g = np.load(os.path.join(golden_dir, f"ref_rollout_{name}.npz"))
+        _, B, _, _, T, _, _, repos = g["meta"].tolist()
+        reps = -(-1024 // B)
+
+        def tile(a):
+            return np.tile(a, (reps,) + (1,) * (a.ndim - 1))
+        ops = O.OP_SHIFT | O.OP_NEWTON | (O.OP_REPOSITION if repos else 0)
+        o = cport.step(tile(g["init"]).astype(np.int32), None, None, O.OP_NEWTON, 0)[0]
+        assert np.array_equal(o.astype(np.float32), tile(g["states"][0])), name
+        for t in range(T):
+            o, od, orw, _ = cport.step(o, tile(g["host_ids"][t]), tile(g["axes"][t]), ops, flags)
+            assert np.array_equal(o.astype(np.float32), tile(g["states"][t + 1])), (name, t)
+            assert np.array_equal(od.astype(bool), tile(g["dones"][t + 1])), (name, t)
+            assert np.array_equal(orw, tile(g["dones"][t + 1] & ~g["dones"][t]).astype(np.float32)), (name, t)
     if not R.available():
-        pytest.skip("baseline/_ref is not installed (baseline/install_ref.sh needs /root/reference)")
-    import numpy as np
+        return
     sys.path.insert(0, ROOT)
     import bench
-    from oracle import cport, hk_oracle as O
     torch, TensorPoints, HostActionEncoder = R.import_reference()
     B, T = 1024, 12
     pts, ha, ax = bench.make_inputs(99, B, 1)
@@ -185,7 +202,6 @@ def test_reference_arm_matches_the_oracle():
     assert np.array_equal(tp.points.numpy(), o.astype(np.float32))
     rec = []
     counts = R.play(tp, HostActionEncoder(3), torch, ha[0, :T], ax[0, :T], True, record=rec)
-    flags = O.F_NOOP_INVALID | O.F_FREEZE_ENDED | O.F_ACT_DISCRETE
     for t in range(T):
         o, od, orw, _ = cport.step(o, ha[0, t], ax[0, t], O.OP_SHIFT | O.OP_REPOSITION | O.OP_NEWTON, flags)
         assert np.array_equal(rec[t][0], o.astype(np.float32)), t

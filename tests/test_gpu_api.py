@@ -698,17 +698,40 @@ def test_cuda_graph_capture_of_step():
     assert eq(state, o) and eq(r.done, O.get_dones(o.astype(np.float32)))
 
 
-def test_reference_arm_matches_the_gpu():
-    """The unmodified reference (baseline/_ref, what `bench.py --impl reference` times) against the CUDA path on
-    the bench's own C2 inputs, bit for bit: states, done flags, rewards after every step.  The reference's torch
+def test_reference_arm_matches_the_gpu(golden_dir):
+    """The unmodified reference (what `bench.py --impl reference` times) against the CUDA path the bench times
+    (in-place census steps), bit for bit: states, done flags, rewards after every step.  The reference's torch
     ops treat an invalid action as a no-op and freeze ended games (hironaka/src/_torch_ops.py:90-93), so the
-    kernel runs with those two flags here; the headline's JAX flavour is pinned by the JAX-source goldens."""
-    import sys
+    kernel runs with those two flags here; the headline's JAX flavour is pinned by the JAX-source goldens.  The
+    reference's side is stored: ref_rollout_c2_20x3*.npz, C2 random play recorded from the unmodified
+    TensorPoints by oracle/gen_golden.py, tiled here to 4096 games.  Where baseline/_ref is installed, the live
+    reference also plays the bench's own C2 inputs."""
+    import os
     from baseline import reference_arm as R
-    if not R.available():
-        pytest.skip("baseline/_ref did not travel")
-    import bench
     from hironaka_b200 import constants as C, ops
+    flags = C.TORCH_SEMANTICS | C.HK_F_ACT_DISCRETE
+    for name in ("c2_20x3", "c2_20x3_repos"):
+        gd = np.load(os.path.join(golden_dir, f"ref_rollout_{name}.npz"))
+        _, B, _, _, Tn, _, _, repos = gd["meta"].tolist()
+        reps = -(-4096 // B)
+
+        def tile(a):
+            return np.tile(a, (reps,) + (1,) * (a.ndim - 1))
+        step_ops = C.HK_OP_SHIFT | C.HK_OP_NEWTON | (C.HK_OP_REPOSITION if repos else 0)
+        g = T(tile(gd["init"]).astype(np.int32))
+        census = ops.new_census(g)
+        ops.step(g, ops=C.HK_OP_NEWTON, inplace=True, census=census)
+        assert np.array_equal(g.cpu().numpy().astype(np.float32), tile(gd["states"][0])), name
+        for t in range(Tn):
+            r = ops.step(g, T(tile(gd["host_ids"][t])), T(tile(gd["axes"][t])), ops=step_ops, flags=flags, inplace=True,
+                         want_done=True, want_reward=True, census=census)
+            assert np.array_equal(g.cpu().numpy().astype(np.float32), tile(gd["states"][t + 1])), (name, t)
+            assert np.array_equal(r.done.cpu().numpy(), tile(gd["dones"][t + 1])), (name, t)
+            assert np.array_equal(r.reward.cpu().numpy(),
+                                  tile(gd["dones"][t + 1] & ~gd["dones"][t]).astype(np.float32)), (name, t)
+    if not R.available():
+        return
+    import bench
     rtorch, TensorPoints, HostActionEncoder = R.import_reference()
     B, Tn = 4096, 20
     pts, ha, ax = bench.make_inputs(7, B, 1)
