@@ -694,6 +694,13 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
             }
             // ---- dedupe alone (remove_repeated _fn.py:192-213) ----
             if ((kops & HK_OP_DEDUPE) && cnt >= 2) {
+                // A row that died in an earlier step of a rollout still holds its old values in the slot (dead rows
+                // are padded on the way out): whether row j is live comes from the warp's live masks, not its data.
+                _Pragma("unroll UNR")
+                for (int r = 0; r < R; ++r) {
+                    const uint32_t bal = __ballot_sync(0xffffffffu, (mylive >> r) & 1u);
+                    if (lane == 0) lmw[r] = bal;
+                }
                 __syncwarp();
                 uint32_t kill = 0;
                 _Pragma("unroll UNR")
@@ -702,7 +709,7 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
                     const int i = lane + 32 * r;
                     bool rep = false;
                     for (int j = 0; j < i; ++j) {
-                        bool eq = x[j * D] >= Elem<T>::zero();
+                        bool eq = (lmw[j >> 5] >> (j & 31)) & 1u;
 #pragma unroll
                         for (int k = 0; k < D; ++k) eq = eq && (x[i * D + k] == x[j * D + k]);
                         rep = rep || eq;
