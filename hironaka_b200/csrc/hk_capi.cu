@@ -125,6 +125,11 @@ int run(StepParams& p, int dtype, int force_generic, cudaStream_t stream) {
     }
     // remove_repeated alone is not on the step path: it runs on the warp-per-game kernel for every shape
     const bool small = hk::is_small_shape(p.N, p.d) && !force_generic && !(p.ops & HK_OP_DEDUPE);
+    if (p.obs_t || p.host_mask_t || p.axis_played_t) {  // a recorded rollout: instantiations of its own
+        if (dtype == HK_DTYPE_I32)
+            return small ? hk::launch_small_i32_rec(p, dev, stream) : hk::launch_generic_i32_rec(p, dev, stream);
+        return small ? hk::launch_small_f32_rec(p, dev, stream) : hk::launch_generic_f32_rec(p, dev, stream);
+    }
     if (dtype == HK_DTYPE_I32)
         return small ? hk::launch_small_i32(p, obs, dev, stream) : hk::launch_generic_i32(p, obs, dev, stream);
     return small ? hk::launch_small_f32(p, obs, dev, stream) : hk::launch_generic_f32(p, obs, dev, stream);
@@ -374,6 +379,32 @@ int hk_rollout_seeded(const void* state_in, void* state_out, const int32_t* host
     p.flags = flags;
     p.seed = seed;
     p.step_offset = step_offset;
+    return run(p, dtype, g_force_generic.load(), (cudaStream_t)stream);
+}
+
+int hk_rollout_record(const void* state_in, void* state_out, const int32_t* host_action_t, const int32_t* axis_t,
+                      float* obs_t, int32_t agent_obs, int32_t* host_mask_t, int32_t* axis_played_t, uint8_t* done_t,
+                      float* reward_t, int32_t* done_count, int32_t* length, int64_t B, int32_t N, int32_t d, int32_t T,
+                      int32_t dtype, uint32_t ops, uint32_t flags, float padding_value, uint64_t seed, int32_t step_offset,
+                      void* stream) {
+    if (T < 1 || (agent_obs && !obs_t)) return HK_ERR_BAD_ARG;
+    const bool random = flags & (HK_F_HOST_RANDOM | HK_F_AGENT_RANDOM);
+    StepParams p = make_params(state_in, state_out, B, N, d, padding_value);
+    p.host_action = (flags & HK_F_HOST_RANDOM) ? nullptr : host_action_t;
+    p.axis = (flags & HK_F_AGENT_RANDOM) ? nullptr : axis_t;
+    p.obs_t = obs_t;
+    p.agent_obs = agent_obs ? 1 : 0;
+    p.host_mask_t = host_mask_t;
+    p.axis_played_t = axis_played_t;
+    p.done = done_t;
+    p.reward = reward_t;
+    p.done_count = done_count;
+    p.length = length;
+    p.T = T;
+    p.ops = ops;
+    p.flags = flags;
+    p.seed = random ? seed : 0;
+    p.step_offset = random ? step_offset : 0;
     return run(p, dtype, g_force_generic.load(), (cudaStream_t)stream);
 }
 

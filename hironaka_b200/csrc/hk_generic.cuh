@@ -46,6 +46,79 @@ constexpr uint32_t GENERIC_HOT_FLAGS = HK_F_ACT_DISCRETE;
 // count so that a pair of rows is a whole number of 16-byte words
 __host__ __device__ constexpr int generic_compact_stride(int D) { return (D + 2) & ~1; }
 
+// Observation features of one game as it stands (live rows from the bits of `mylive`, lane l owning rows l, l + 32, ...)
+// into its row `gobs` of an obs array; `f` is the warp's feature buffer (N*d floats).  The recorded rollouts call it before
+// every step.  It computes what the step's observation phase at the end of hk_generic_kernel computes; that phase keeps
+// its own copy because calling this function there changes the instruction schedule of the step + features kernels.
+template <typename T, int D, int RT>
+__device__ __forceinline__ void generic_features(const T* x, uint32_t mylive, float* f, float* gobs, int N, int R, int lane,
+                                                 uint32_t kflags, float pad) {
+    constexpr int UNR = RT > 0 ? RT : 1;
+    float mx = -1.0f;
+    _Pragma("unroll UNR")
+    for (int r = 0; r < R; ++r) {
+        if (!((mylive >> r) & 1u)) continue;
+        const int i = lane + 32 * r;
+#pragma unroll
+        for (int k = 0; k < D; ++k) mx = fmaxf(mx, Elem<T>::to_float(x[i * D + k]));
+    }
+    mx = warp_maxf(mx);
+    if (mx == 0.0f || ((kflags & HK_F_RESCALE_EPS) && mx > 0.0f && mx <= 1e-8f)) mx = 1.0f;
+    const bool resc = (kflags & HK_F_OBS_RESCALE) && (mx > 0.0f);
+    _Pragma("unroll UNR")
+    for (int r = 0; r < R; ++r) {
+        const int i = lane + 32 * r;
+        if (i >= N) continue;
+        const bool lv = (mylive >> r) & 1u;
+#pragma unroll
+        for (int k = 0; k < D; ++k) {
+            float v = Elem<T>::to_float(x[i * D + k]);
+            v = (resc && lv && v != 0.0f) ? __fdiv_rn(v, mx) : v;
+            f[i * D + k] = lv ? v : pad;
+        }
+    }
+    __syncwarp();
+    const bool sorted = kflags & (HK_F_OBS_SORT_COORD0 | HK_F_OBS_SORT_LEX | HK_F_OBS_SORT_LEX_FIRST);
+    const bool lex = kflags & HK_F_OBS_SORT_LEX;
+    const bool lexf = kflags & HK_F_OBS_SORT_LEX_FIRST;
+    _Pragma("unroll UNR")
+    for (int r = 0; r < R; ++r) {
+        const int i = lane + 32 * r;
+        if (i >= N) continue;
+        float fi[D];
+#pragma unroll
+        for (int k = 0; k < D; ++k) fi[k] = f[i * D + k];
+        int rank = i;
+        if (sorted) {
+            rank = 0;
+            for (int j = 0; j < N; ++j) {
+                bool gt = f[j * D] > fi[0];
+                bool eq = f[j * D] == fi[0];
+                if (lex) {
+#pragma unroll
+                    for (int k = 1; k < D; ++k) {
+                        const float fj = f[j * D + k];
+                        gt = (fj > fi[k]) || ((fj == fi[k]) && gt);
+                        eq = eq && (fj == fi[k]);
+                    }
+                } else if (lexf) {
+                    gt = f[j * D + D - 1] > fi[D - 1];
+                    eq = f[j * D + D - 1] == fi[D - 1];
+#pragma unroll
+                    for (int k = D - 2; k >= 0; --k) {
+                        const float fj = f[j * D + k];
+                        gt = (fj > fi[k]) || ((fj == fi[k]) && gt);
+                        eq = eq && (fj == fi[k]);
+                    }
+                }
+                rank += (gt || (eq && j < i)) ? 1 : 0;
+            }
+        }
+#pragma unroll
+        for (int k = 0; k < D; ++k) gobs[rank * D + k] = fi[k];
+    }
+}
+
 // smem per warp: DEPTH + 1 state buffers x[DEPTH + 1][Wpad] (the games up to DEPTH iterations ahead are in
 // flight while the current one is processed), then (OBS) f[Wpad] floats, then lmw[ceil(N/32)] (padded to
 // 4 words), then the compact list of live rows, (N + 1) * generic_compact_stride(D) words
@@ -53,7 +126,10 @@ __host__ __device__ constexpr int generic_compact_stride(int D) { return (D + 2)
 // guards become predication) or 0 for any N (run-time loops).
 // CENSUS: the instantiation that serves hk_step_census (plain in-place single steps); it is separate so that
 // the census bookkeeping costs the other calls nothing (the kernel is bound by instruction issue).
-template <typename T, int D, bool OBS, int RT, int DEPTH, bool HOT, bool CENSUS = false>
+// REC: recorded rollouts (hk_rollout_record, with OBS for the feature buffer): every game takes the padded route,
+// whose step loop writes the features of the state before each step to row st of p.obs_t and the played actions after
+// the shift.
+template <typename T, int D, bool OBS, int RT, int DEPTH, bool HOT, bool CENSUS = false, bool REC = false>
 __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(const StepParams p, int warps_per_cta, int slot_words) {
     constexpr int NBUF = DEPTH + 1;
     // HOT: the plain random-play step (shift + reposition + newton, discrete host ids, int32 action arrays,
@@ -80,13 +156,13 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
     const bool vec_in = aligned16(p.in) && ((W & 3) == 0);
     const bool vec_out = aligned16(p.out) && ((W & 3) == 0);
     const T padv = Elem<T>::pad(p.pad);
-    const int OW = W + (p.obs_coord ? D : 0);
+    const int OW = W + ((REC ? p.agent_obs : p.obs_coord != nullptr) ? D : 0);
     const bool inplace = (gout == gin) && !(kflags & HK_F_STORE_ALL);
     // the short path for ended games covers plain single steps only
-    const bool ended_fast_path =
+    const bool ended_fast_path = !REC &&
         kT == 1 && !(OBS && p.obs) && !p.host_out && !(kops & ~(HK_OP_SHIFT | HK_OP_REPOSITION | HK_OP_NEWTON)) &&
         !(kflags & (HK_F_HOST_ALL_COORD | HK_F_HOST_ZEILLINGER | HK_F_AGENT_FIRST | HK_F_AGENT_LAST));
-    const bool compact_path =
+    const bool compact_path = !REC &&
         !(OBS && p.obs) && !p.host_out && !(kops & HK_OP_DEDUPE) &&
         !(kflags & (HK_F_HOST_ALL_COORD | HK_F_HOST_ZEILLINGER | HK_F_AGENT_FIRST | HK_F_AGENT_LAST));
 
@@ -561,6 +637,13 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
         }
         int32_t len = (cnt < 2) ? 0 : kT + 1;
         for (int st = 0; st < kT; ++st) {
+            float* gobs_t = nullptr;
+            if constexpr (REC) {
+                if (p.obs_t) {
+                    gobs_t = p.obs_t + ((long long)st * p.B + g) * OW;
+                    generic_features<T, D, RT>(x, mylive, f, gobs_t, N, R, lane, kflags, p.pad);
+                }
+            }
             int32_t ha_n = 3, ax_n = 0;
             if ((kops & HK_OP_SHIFT) && st + 1 < kT) {
                 load_actions(p, kflags, g, st + 1, ha_n, ax_n);
@@ -569,6 +652,15 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
 
             // ---- shift ----
             if ((kops & HK_OP_SHIFT) && cnt == 0 && p.host_out && lane == 0) p.host_out[g] = 0;
+            uint32_t played_cm = 0, played_ax = 0;  // (REC) what the shift used, 0 without one
+            if constexpr (REC) {
+                if ((kops & HK_OP_SHIFT) && cnt == 0) {  // nothing moves; the players answer as on any other game
+                    const uint32_t cm = (kflags & HK_F_HOST_ALL_COORD) ? ((1u << D) - 1u)
+                                        : (kflags & HK_F_HOST_ZEILLINGER) ? decode_host_action(0) : action_mask(ha, kflags);
+                    played_cm = (kflags & (HK_F_HOST_ALL_COORD | HK_F_HOST_ZEILLINGER)) ? 0u : cm;
+                    played_ax = (uint32_t)agent_policy_axis(cm, ax, kflags, D);
+                }
+            }
             if ((kops & HK_OP_SHIFT) && cnt > 0) {
                 uint32_t cm;
                 if (kflags & HK_F_HOST_ALL_COORD) {
@@ -632,6 +724,10 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
                     cm = action_mask(ha, kflags);
                 }
                 ax = agent_policy_axis(cm, ax, kflags, D);
+                if constexpr (REC) {
+                    played_cm = cm;
+                    played_ax = (uint32_t)ax;
+                }
                 bool apply = (ax >= 0) && (ax < D);
                 if (p.host_out) {  // hk_host_policy: report the host's choice, move nothing
                     if (lane == 0) p.host_out[g] = (int32_t)cm;
@@ -651,6 +747,14 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
                         x[i * D + ax] = s;
                     }
                 }
+            }
+            if constexpr (REC) {
+                if (lane == 0) {
+                    const long long o = (long long)st * p.B + g;
+                    if (p.host_mask_t) p.host_mask_t[o] = (int32_t)played_cm;
+                    if (p.axis_played_t) p.axis_played_t[o] = (int32_t)played_ax;
+                }
+                if (gobs_t && p.agent_obs && lane < D) gobs_t[W + lane] = (float)((played_cm >> lane) & 1u);
             }
             // ---- reposition ----
             if ((kops & HK_OP_REPOSITION) && cnt == 1) {

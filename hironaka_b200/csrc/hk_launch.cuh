@@ -63,5 +63,10 @@ inline bool rows_shape(int N, int d) { return N <= 64 && d >= 2 && d <= 5; }
 // warp-per-game family (hk_generic.cuh)
 int launch_generic_i32(const StepParams& p, bool obs, int dev, cudaStream_t stream);
 int launch_generic_f32(const StepParams& p, bool obs, int dev, cudaStream_t stream);
+// recorded rollouts (hk_rollout_record), instantiations of their own in both families
+int launch_small_i32_rec(const StepParams& p, int dev, cudaStream_t stream);
+int launch_small_f32_rec(const StepParams& p, int dev, cudaStream_t stream);
+int launch_generic_i32_rec(const StepParams& p, int dev, cudaStream_t stream);
+int launch_generic_f32_rec(const StepParams& p, int dev, cudaStream_t stream);
 
 }  // namespace hk

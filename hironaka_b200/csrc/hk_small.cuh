@@ -331,9 +331,11 @@ __device__ __forceinline__ uint32_t zeillinger_rows(const T (&y)[K * D], uint32_
 }
 
 // POLICY: instantiation that can evaluate the fixed players (kept out of the ordinary step kernels)
-template <typename T, int N, int D, int RS = 0, bool POLICY = false>
+// REC: recorded rollouts; `played` receives the coordinate bitmask and the axis the shift used (a fixed host on a game
+// without live rows records 0, as hk_host_policy reports it)
+template <typename T, int N, int D, int RS = 0, bool POLICY = false, bool REC = false>
 __device__ __forceinline__ uint32_t game_step(T (&x)[N * D], uint32_t lm, uint32_t ops, uint32_t flags, int32_t ha,
-                                              int32_t ax_in, uint32_t* scratch = nullptr) {
+                                              int32_t ax_in, uint32_t* scratch = nullptr, uint32_t* played = nullptr) {
     if (ops & HK_OP_SHIFT) {
         uint32_t cm;
         int ax = ax_in;
@@ -348,6 +350,10 @@ __device__ __forceinline__ uint32_t game_step(T (&x)[N * D], uint32_t lm, uint32
             ax = agent_policy_axis(cm, ax_in, flags, D);
         } else {
             cm = action_mask(ha, flags);
+        }
+        if constexpr (REC) {
+            played[0] = (POLICY && (flags & (HK_F_HOST_ALL_COORD | HK_F_HOST_ZEILLINGER)) && lm == 0) ? 0u : cm;
+            played[1] = (uint32_t)ax;
         }
         bool apply = (ax >= 0) && (ax < D);
         if (flags & HK_F_NOOP_INVALID) apply = apply && ((cm >> (ax & 31)) & 1u);
@@ -391,6 +397,7 @@ struct LaneState {
     int cnt;
     int32_t len;
     bool origin;  // census only: no live row, or the lone live row sits at the origin (a fixed point of every op)
+    uint32_t played[2];  // recorded rollouts: the host's coordinate bitmask and the axis of the last step (0 without a shift)
 };
 
 __host__ __device__ constexpr int next_lower_tier(int K) {
@@ -398,9 +405,9 @@ __host__ __device__ constexpr int next_lower_tier(int K) {
 }
 
 // Runs steps [st, T) of one tile on K compact rows; returns the step index at which it stopped
-// (T, or earlier when every game of the warp fits the next lower tier).  The lane's game area in
+// (T, or earlier when every game of the warp fits the next lower tier; REC: after one step).  The lane's game area in
 // shared memory (`row`) holds the current state on entry and on exit.
-template <typename T, int N, int D, int K, bool POLICY>
+template <typename T, int N, int D, int K, bool POLICY, bool REC = false>
 __device__ __forceinline__ int tier_steps(const StepParams& p, LaneState& ls, uint32_t* row, uint32_t lm, int st,
                                           bool& exceed, bool& chg) {
     const long long B = p.B;
@@ -452,7 +459,8 @@ __device__ __forceinline__ int tier_steps(const StepParams& p, LaneState& ls, ui
             load_actions(p, p.flags, ls.g, st + 1, ha_n, ax_n);
         }
         const bool prev_done = ls.cnt < 2;
-        clm = game_step<T, K, D, RS, POLICY>(y, clm, p.ops, p.flags, ls.ha, ls.ax, row);
+        if constexpr (REC) ls.played[0] = ls.played[1] = 0u;
+        clm = game_step<T, K, D, RS, POLICY, REC>(y, clm, p.ops, p.flags, ls.ha, ls.ax, row, ls.played);
         if (K <= 4 && p.T == 1) {
             bool diff = (clm != clm_before) || (clm_before > 1u);  // compact rows fill from 0: > 1 means two or more rows
 #pragma unroll
@@ -476,6 +484,7 @@ __device__ __forceinline__ int tier_steps(const StepParams& p, LaneState& ls, ui
         ls.ha = ha_n;
         ls.ax = ax_n;
         ++st;
+        if constexpr (REC) break;  // the recorder reads the state in the lane's game area after every step
         if constexpr (LOWER > 0) {
             if (st < p.T && __reduce_max_sync(0xffffffffu, ls.valid ? ls.cnt : 0) <= LOWER) break;  // re-tier
         }
@@ -1134,16 +1143,27 @@ __device__ __noinline__ void features_rolled(const uint32_t* row, uint32_t lm, i
 // `gdst` (optional, with `release`): the lane's game in global memory of an in-place call whose stage may be refilled
 // as soon as the packed tiers have gathered their rows (tier_packed, DIRECT); returns true when that route was taken
 // (the stage has been released, the game is already in global memory, `row` is stale).
-template <typename T, int N, int D, bool POLICY, bool PACKED = true, typename Release = NoRelease>
+// `rec` (recorded rollouts): rec(st, false) before step st with the state in `row`, rec(st, true) after it with
+// ls.played set; the tiers then stop after every step.
+struct NoRec {
+    __device__ __forceinline__ void operator()(int, bool) const {}
+};
+
+template <typename T, int N, int D, bool POLICY, bool PACKED = true, typename Release = NoRelease, typename Rec = NoRec>
 __device__ __forceinline__ bool small_process_tile(const StepParams& p, LaneState& ls, uint32_t* row, bool& exceed,
-                                                   bool& chg, uint32_t* gdst = nullptr, Release release = Release()) {
+                                                   bool& chg, uint32_t* gdst = nullptr, Release release = Release(),
+                                                   Rec rec = Rec()) {
     constexpr int W = N * D;
+    constexpr bool REC = !std::is_same<Rec, NoRec>::value;
+    static_assert(!(REC && PACKED), "a recorded rollout steps on the exact tiers only");
     const T padv = Elem<T>::pad(p.pad);
     const bool mutate = p.ops != 0;
     bool normalised = false;
     ls.len = -1;
     int st = 0;
     do {
+        const int st0 = st;
+        if constexpr (REC) rec(st0, false);
         bool any_junk = false;
         uint32_t lm;
         {
@@ -1254,25 +1274,26 @@ __device__ __forceinline__ bool small_process_tile(const StepParams& p, LaneStat
         }
         if (N > 2 && p.T == 1 && lmax <= 2) {  // the tail of a rollout driven step by step: ended games and two-point games only
             prestore();
-            st = tier_steps<T, N, D, (N > 2 ? 2 : N), POLICY>(p, ls, row, lm, st, exceed, chg);
+            st = tier_steps<T, N, D, (N > 2 ? 2 : N), POLICY, REC>(p, ls, row, lm, st, exceed, chg);
         } else if (N > 4 && lmax <= 4) {
             prestore();
-            st = tier_steps<T, N, D, (N > 4 ? 4 : N), POLICY>(p, ls, row, lm, st, exceed, chg);
+            st = tier_steps<T, N, D, (N > 4 ? 4 : N), POLICY, REC>(p, ls, row, lm, st, exceed, chg);
         } else if (N > 8 && lmax <= 8) {
             prestore();
-            st = tier_steps<T, N, D, (N > 8 ? 8 : N), POLICY>(p, ls, row, lm, st, exceed, chg);
+            st = tier_steps<T, N, D, (N > 8 ? 8 : N), POLICY, REC>(p, ls, row, lm, st, exceed, chg);
         } else if (N > 12 && lmax <= 12) {
             if (W % 4 != 0) prestore();
-            st = tier_steps<T, N, D, (N > 12 ? 12 : N), POLICY>(p, ls, row, lm, st, exceed, chg);
+            st = tier_steps<T, N, D, (N > 12 ? 12 : N), POLICY, REC>(p, ls, row, lm, st, exceed, chg);
             normalised = normalised || (W % 4 == 0);
         } else if (N > 16 && lmax <= 16) {
             if (W % 4 != 0) prestore();
-            st = tier_steps<T, N, D, (N > 16 ? 16 : N), POLICY>(p, ls, row, lm, st, exceed, chg);
+            st = tier_steps<T, N, D, (N > 16 ? 16 : N), POLICY, REC>(p, ls, row, lm, st, exceed, chg);
             normalised = normalised || (W % 4 == 0);
         } else {
-            st = tier_steps<T, N, D, N, POLICY>(p, ls, row, lm, st, exceed, chg);
+            st = tier_steps<T, N, D, N, POLICY, REC>(p, ls, row, lm, st, exceed, chg);
             normalised = true;
         }
+        if constexpr (REC) rec(st0, true);
     } while (st < p.T);
     return false;
 }
@@ -1283,10 +1304,12 @@ __device__ __forceinline__ void warp_copy_words(uint32_t* dst, const uint32_t* s
 }
 
 // PACKED = false: the instantiation of the one-launch rollouts (p.T > 1), which never take the packed tiers and are bound
-// by instruction fetch: they do not carry that code
-template <typename T, int N, int D, bool OBS, bool POLICY, int WARPS, int STAGES, bool PACKED = true>
-__global__ void __launch_bounds__(WARPS * 32) hk_small_kernel(const StepParams p) {
-    using L = SmallLayout<N, D, OBS, WARPS, STAGES>;
+// by instruction fetch: they do not carry that code.
+// REC: recorded rollouts (hk_small_record_kernel): before every step the features of the state go to the warp's obs
+// tile, after it the played actions are written and the tile leaves with one bulk store into row st of p.obs_t.
+template <typename T, int N, int D, bool OBS, bool POLICY, int WARPS, int STAGES, bool PACKED, bool REC>
+__device__ __forceinline__ void small_kernel_body(const StepParams& p) {
+    using L = SmallLayout<N, D, OBS || REC, WARPS, STAGES>;
     constexpr int SMALL_WARPS = WARPS;
     constexpr int SMALL_STAGES = STAGES;
     constexpr bool DELAYED_REFILL = (STAGES >= 3) && !OBS;  // the single obs tile needs its store drained first
@@ -1304,7 +1327,7 @@ __global__ void __launch_bounds__(WARPS * 32) hk_small_kernel(const StepParams p
     const uint32_t* gin = reinterpret_cast<const uint32_t*>(p.in);
     uint32_t* gout = reinterpret_cast<uint32_t*>(p.out);
     const bool tma_base = aligned16(p.in) && aligned16(p.out);
-    const int OW = W + (p.obs_coord ? D : 0);
+    const int OW = W + ((REC ? p.agent_obs : p.obs_coord != nullptr) ? D : 0);
     const bool obs_tma = aligned16(p.obs);
     const T padv = Elem<T>::pad(p.pad);
     const bool write = (gout != nullptr);
@@ -1374,7 +1397,56 @@ __global__ void __launch_bounds__(WARPS * 32) hk_small_kernel(const StepParams p
         // (everything is when out != in).
         bool chg = !inplace;
         bool released = false;  // the stage has been handed back (and refilled) in the middle of the step
-        if constexpr (HK_SMALL_DIRECT && PACKED && !OBS && !POLICY && SMALL_STAGES == 1 && !Elem<T>::is_float) {
+        if constexpr (REC) {
+            const int nrows = words / W;
+            auto rec = [&](int st, bool after) {
+                if (!after) {
+                    if (p.obs_t == nullptr) return;
+                    if (lane == 0) bulk_wait_read<0>();  // the previous row's store has read the obs tile
+                    __syncwarp();
+                    T z[W];
+                    load_game<T, W>(row, z);
+                    if constexpr (Elem<T>::is_float) {
+#pragma unroll
+                        for (int q = 0; q < W; ++q) z[q] = z[q] + 0.0f;
+                    }
+                    const uint32_t zl = live_mask<T, N, D>(z);
+                    const int zmax = __reduce_max_sync(0xffffffffu, ls.valid ? __popc(zl) : 0);
+                    bool built = false;
+                    if constexpr (D <= 6) built = features_network<T, N, D>(z, zl, zmax, p.flags, p.pad, orow);
+                    if (!built) {
+                        const int gpow = (OW & -OW) > 32 ? 32 : (OW & -OW);
+                        features_rolled<T, N, D>(row, zl, zmax, p.flags, p.pad, orow, (lane * gpow) >> 5);
+                    }
+                    return;
+                }
+                if (ls.valid) {
+                    const long long o = (long long)st * B + ls.g;
+                    if (p.host_mask_t) p.host_mask_t[o] = (int32_t)ls.played[0];
+                    if (p.axis_played_t) p.axis_played_t[o] = (int32_t)ls.played[1];
+                }
+                if (p.obs_t == nullptr) return;
+                if (p.agent_obs) {
+#pragma unroll
+                    for (int k = 0; k < D; ++k) orow[W + k] = (float)((ls.played[0] >> k) & 1u);
+                }
+                const int owords = nrows * OW;
+                float* gobs = p.obs_t + ((long long)st * B + (t << 5)) * OW;
+                if (aligned16(gobs) && (owords & 3) == 0) {
+                    fence_async_smem();
+                    __syncwarp();
+                    if (lane == 0) {
+                        bulk_store(gobs, obs_tile, (uint32_t)owords * 4u);
+                        bulk_commit();
+                    }
+                } else {
+                    __syncwarp();
+                    warp_copy_words(reinterpret_cast<uint32_t*>(gobs), reinterpret_cast<uint32_t*>(obs_tile), owords, lane);
+                    __syncwarp();
+                }
+            };
+            small_process_tile<T, N, D, POLICY, PACKED, NoRelease, decltype(rec)>(p, ls, row, exceed, chg, nullptr, NoRelease(), rec);
+        } else if constexpr (HK_SMALL_DIRECT && PACKED && !OBS && !POLICY && SMALL_STAGES == 1 && !Elem<T>::is_float) {
             // packed tiers, direct route (tier_packed, DIRECT) of an in-place single step: the stage is refilled as soon as
             // the rows are gathered and the changed rows go straight to global memory
             if (inplace && tma && p.T == 1) {  // (warp-uniform)
@@ -1502,6 +1574,17 @@ __global__ void __launch_bounds__(WARPS * 32) hk_small_kernel(const StepParams p
         s = (s + 1 == SMALL_STAGES) ? 0 : s + 1;
     }
     if (lane == 0) bulk_wait_all<0>();  // all bulk stores globally complete before the warp retires
+}
+
+template <typename T, int N, int D, bool OBS, bool POLICY, int WARPS, int STAGES, bool PACKED = true>
+__global__ void __launch_bounds__(WARPS * 32) hk_small_kernel(const StepParams p) {
+    small_kernel_body<T, N, D, OBS, POLICY, WARPS, STAGES, PACKED, false>(p);
+}
+
+// hk_rollout_record on the thread-per-game shapes: the rollout kernel's tile loop with the recorder, one stage per warp
+template <typename T, int N, int D, bool POLICY, int WARPS>
+__global__ void __launch_bounds__(WARPS * 32) hk_small_record_kernel(const StepParams p) {
+    small_kernel_body<T, N, D, false, POLICY, WARPS, 1, false, true>(p);
 }
 
 }  // namespace hk

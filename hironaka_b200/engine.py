@@ -124,6 +124,22 @@ class GameBatch:
         self.reset_census()  # the one-launch rollout does not keep it
         return done, reward, dcount, length
 
+    def record(self, steps: Optional[int] = None, host_actions: Optional[torch.Tensor] = None,
+               axes: Optional[torch.Tensor] = None, *, scale_observation: bool = True, sort: str = "lex",
+               agent_obs: bool = False) -> _ops.Trajectory:
+        """T game-steps in ONE launch that also record the trajectory (ops.rollout_record): obs [T, B, N*d (+d)] of the
+        state before each step, with the observation options of `features` (agent_obs appends the host's coordinates
+        of the step), the played host bitmasks and axes [T, B], done / reward [T, B], done_count [T] and length [B].
+        The observation after the last step is features() of the batch afterwards."""
+        obs_flags = (C.HK_F_OBS_RESCALE if scale_observation else 0) | \
+            {"lex": C.HK_F_OBS_SORT_LEX, "coord0": C.HK_F_OBS_SORT_COORD0, "none": 0}[sort]
+        traj = _ops.rollout_record(self.points, steps, host_actions, axes, ops=self.ops, flags=self.flags | obs_flags,
+                                   seed=self.seed, step_offset=self.steps_played, agent_obs=agent_obs, inplace=True)
+        if self.flags & (C.HK_F_HOST_RANDOM | C.HK_F_AGENT_RANDOM):
+            self.steps_played += traj.done_count.shape[0]
+        self.reset_census()  # the one-launch rollout does not keep it
+        return traj
+
     def step_host(self, host_action_host: torch.Tensor, axis_host: torch.Tensor) -> int:
         """One game-step driven from HOST buffers: copies this step's actions (int32 [B], ideally
         pinned) to the device, runs the step in place and returns the number of finished games

@@ -239,6 +239,59 @@ def rollout_random(state: torch.Tensor, steps: int, seed: int, *, ops: int, flag
     return dst, (None if done is None else done.view(torch.bool)), reward, dcount, length
 
 
+class Trajectory(NamedTuple):
+    state: torch.Tensor                  # [B,N,d] state after the last step (the input tensor itself when in place)
+    obs: Optional[torch.Tensor]          # [T, B, N*d (+d)] float32: features of the state BEFORE each step
+    host_mask: Optional[torch.Tensor]    # [T, B] int32 coordinate bitmask each step's shift used
+    axis: Optional[torch.Tensor]         # [T, B] int32 axis each step's shift used
+    done: Optional[torch.Tensor]         # [T, B] bool
+    reward: Optional[torch.Tensor]       # [T, B] float32
+    done_count: Optional[torch.Tensor]   # [T] int32 finished games after each step
+    length: Optional[torch.Tensor]       # [B] int32
+
+
+def rollout_record(state: torch.Tensor, steps: Optional[int] = None, host_actions: Optional[torch.Tensor] = None,
+                   axes: Optional[torch.Tensor] = None, *, ops: int, flags: int = 0, seed: int = 0, step_offset: int = 0,
+                   want_obs: bool = True, agent_obs: bool = False, want_actions: bool = True, want_done: bool = True,
+                   want_reward: bool = True, want_length: bool = True, inplace: bool = True,
+                   padding_value: float = -1.0) -> Trajectory:
+    """T fused steps in one launch that also record the trajectory (hk_rollout_record): obs[t] are the features of the
+    state the players see at step t (the observation flags of `features`), host_mask / axis what step t played, as
+    bitmasks and axes (replayed through `rollout` without HK_F_ACT_DISCRETE and the player flags they give the same
+    rollout).  `agent_obs` appends step t's host coordinates to obs[t] as d floats 0/1.  The players are [T, B] int32
+    streams, fixed-player flags, or the in-kernel random players (HK_F_HOST_RANDOM / HK_F_AGENT_RANDOM, keyed by `seed`
+    and `step_offset`); `steps` gives T when no stream does.  The features after the last step are
+    features(trajectory.state)."""
+    dt = _require_state(state)
+    B, N, d = state.shape
+    dev = state.device
+    streams = [t for t in (host_actions, axes) if t is not None]
+    if any(t.dim() != 2 or t.shape[1] != B for t in streams) or len({tuple(t.shape) for t in streams}) > 1:
+        raise ValueError("host_actions and axes must be [T, B]")
+    T = int(steps) if steps is not None else (streams[0].shape[0] if streams else 0)
+    if T < 1 or (streams and streams[0].shape[0] != T):
+        raise ValueError("steps must be >= 1 and match the action streams")
+    if agent_obs and not want_obs:
+        raise ValueError("agent_obs needs want_obs")
+    ha = None if host_actions is None else host_actions.to(device=dev, dtype=torch.int32).contiguous()
+    ax = None if axes is None else axes.to(device=dev, dtype=torch.int32).contiguous()
+    dst = state if inplace else torch.empty_like(state)
+    obs = torch.empty((T, B, N * d + (d if agent_obs else 0)), dtype=torch.float32, device=dev) if want_obs else None
+    hmask = torch.empty((T, B), dtype=torch.int32, device=dev) if want_actions else None
+    axis = torch.empty((T, B), dtype=torch.int32, device=dev) if want_actions else None
+    done = torch.empty((T, B), dtype=torch.uint8, device=dev) if want_done else None
+    reward = torch.empty((T, B), dtype=torch.float32, device=dev) if want_reward else None
+    dcount = torch.zeros(T, dtype=torch.int32, device=dev)
+    length = torch.empty(B, dtype=torch.int32, device=dev) if want_length else None
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        rc = lib().hk_rollout_record(_ptr(state), _ptr(dst), _ptr(ha), _ptr(ax), _ptr(obs), 1 if agent_obs else 0, _ptr(hmask),
+                                     _ptr(axis), _ptr(done), _ptr(reward), _ptr(dcount), _ptr(length), B, N, d, T, dt, ops,
+                                     flags, float(padding_value), int(seed) & (2 ** 64 - 1), int(step_offset), stream)
+    check(rc, "hk_rollout_record")
+    return Trajectory(dst, obs, hmask, axis, None if done is None else done.view(torch.bool), reward, dcount, length)
+
+
 def random_actions(B: int, d: int, steps: int, seed: int, step_offset: int = 0, device="cuda"):
     """The action streams the in-kernel random players draw, written out: (host ids [T, B], axes [T, B]) int32."""
     dev = torch.device(device)

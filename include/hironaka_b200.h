@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define HK_VERSION 100 /* major*100 + minor */
+#define HK_VERSION 101 /* major*100 + minor */
 
 /* ---- status codes ---------------------------------------------------------------- */
 #define HK_OK 0
@@ -242,6 +242,27 @@ int hk_rollout_seeded(const void* state_in, void* state_out, const int32_t* host
                       uint64_t seed, int32_t step_offset, void* stream);
 int hk_random_actions(int32_t* host_action_t, int32_t* axis_t, int64_t B, int32_t d, int32_t T, uint64_t seed,
                       int32_t step_offset, void* stream);
+
+/* ---- recorded rollout -----------------------------------------------------------------------
+ * hk_rollout / hk_rollout_seeded that also writes the trajectory, for training data: what the players saw before
+ * every step and what they played.  seed / step_offset are read only with HK_F_HOST_RANDOM / HK_F_AGENT_RANDOM.
+ * Every output is nullable; with obs_t, host_mask_t and axis_played_t all null the call is hk_rollout(_seeded).
+ *   obs_t         [T,B,OW] float: row t = the features of the state BEFORE step t, as hk_features computes them with the
+ *                 same flags (sort mode, HK_F_OBS_RESCALE, HK_F_RESCALE_EPS), bit for bit; row 0 = hk_features(state_in),
+ *                 and hk_features(state_out) is the observation after the last step.  OW = N*d, or N*d + d with
+ *                 agent_obs != 0: the host's coordinate set of step t appended as d floats 0/1 (make_agent_obs,
+ *                 hironaka/jax/util.py:22-31).  agent_obs without obs_t is HK_ERR_BAD_ARG.
+ *   host_mask_t   [T,B] int32: the coordinate bitmask step t's shift used (discrete ids decoded, packed and nibble
+ *                 streams unpacked, the choices of fixed and random players as made; a fixed host on a game without
+ *                 live rows records 0, as hk_host_policy does)
+ *   axis_played_t [T,B] int32: the axis step t's shift used
+ * Both are 0 without HK_OP_SHIFT.  Fed back to hk_rollout as bitmask / int32 streams (HK_F_ACT_DISCRETE cleared, the
+ * player flags removed) they replay the rollout bit for bit.  The other outputs are hk_rollout's. */
+int hk_rollout_record(const void* state_in, void* state_out, const int32_t* host_action_t, const int32_t* axis_t,
+                      float* obs_t, int32_t agent_obs, int32_t* host_mask_t, int32_t* axis_played_t, uint8_t* done_t,
+                      float* reward_t, int32_t* done_count, int32_t* length, int64_t B, int32_t N, int32_t d, int32_t T,
+                      int32_t dtype, uint32_t ops, uint32_t flags, float padding_value, uint64_t seed, int32_t step_offset,
+                      void* stream);
 
 /* ---- experience writer (SURVEY 8f rank 2) --------------------------------------------------------
  * Appends the rows with skip[b] == 0, IN BATCH ORDER, to circular replay buffers at
