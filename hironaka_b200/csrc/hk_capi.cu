@@ -6,6 +6,7 @@
 #include <cuda_runtime.h>
 
 #include <atomic>
+#include <cmath>
 #include <cstdio>
 #include <cstring>
 #include <new>
@@ -125,6 +126,12 @@ int run(StepParams& p, int dtype, int force_generic, cudaStream_t stream) {
     }
     // remove_repeated alone is not on the step path: it runs on the warp-per-game kernel for every shape
     const bool small = hk::is_small_shape(p.N, p.d) && !force_generic && !(p.ops & HK_OP_DEDUPE);
+    if (p.over_step || p.stop_at_threshold) {  // a rollout with a value threshold, recorded or not: instantiations of their own
+        const bool rec = p.obs_t || p.host_mask_t || p.axis_played_t;
+        if (dtype == HK_DTYPE_I32)
+            return small ? hk::launch_small_i32_thr(p, rec, dev, stream) : hk::launch_generic_i32_thr(p, rec, dev, stream);
+        return small ? hk::launch_small_f32_thr(p, rec, dev, stream) : hk::launch_generic_f32_thr(p, rec, dev, stream);
+    }
     if (p.obs_t || p.host_mask_t || p.axis_played_t) {  // a recorded rollout: instantiations of its own
         if (dtype == HK_DTYPE_I32)
             return small ? hk::launch_small_i32_rec(p, dev, stream) : hk::launch_generic_i32_rec(p, dev, stream);
@@ -146,6 +153,31 @@ StepParams make_params(const void* in, void* out, long long B, int N, int d, flo
     p.T = 1;
     p.pad = pad;
     p.threshold = 1e8f;
+    return p;
+}
+
+// the parameters of hk_rollout_record (and of hk_rollout_threshold before its threshold)
+StepParams record_params(const void* state_in, void* state_out, const int32_t* host_action_t, const int32_t* axis_t,
+                         float* obs_t, int32_t agent_obs, int32_t* host_mask_t, int32_t* axis_played_t, uint8_t* done_t,
+                         float* reward_t, int32_t* done_count, int32_t* length, long long B, int N, int d, int T,
+                         uint32_t ops, uint32_t flags, float padding_value, uint64_t seed, int32_t step_offset) {
+    const bool random = flags & (HK_F_HOST_RANDOM | HK_F_AGENT_RANDOM);
+    StepParams p = make_params(state_in, state_out, B, N, d, padding_value);
+    p.host_action = (flags & HK_F_HOST_RANDOM) ? nullptr : host_action_t;
+    p.axis = (flags & HK_F_AGENT_RANDOM) ? nullptr : axis_t;
+    p.obs_t = obs_t;
+    p.agent_obs = agent_obs ? 1 : 0;
+    p.host_mask_t = host_mask_t;
+    p.axis_played_t = axis_played_t;
+    p.done = done_t;
+    p.reward = reward_t;
+    p.done_count = done_count;
+    p.length = length;
+    p.T = T;
+    p.ops = ops;
+    p.flags = flags;
+    p.seed = random ? seed : 0;
+    p.step_offset = random ? step_offset : 0;
     return p;
 }
 
@@ -388,23 +420,28 @@ int hk_rollout_record(const void* state_in, void* state_out, const int32_t* host
                       int32_t dtype, uint32_t ops, uint32_t flags, float padding_value, uint64_t seed, int32_t step_offset,
                       void* stream) {
     if (T < 1 || (agent_obs && !obs_t)) return HK_ERR_BAD_ARG;
-    const bool random = flags & (HK_F_HOST_RANDOM | HK_F_AGENT_RANDOM);
-    StepParams p = make_params(state_in, state_out, B, N, d, padding_value);
-    p.host_action = (flags & HK_F_HOST_RANDOM) ? nullptr : host_action_t;
-    p.axis = (flags & HK_F_AGENT_RANDOM) ? nullptr : axis_t;
-    p.obs_t = obs_t;
-    p.agent_obs = agent_obs ? 1 : 0;
-    p.host_mask_t = host_mask_t;
-    p.axis_played_t = axis_played_t;
-    p.done = done_t;
-    p.reward = reward_t;
-    p.done_count = done_count;
-    p.length = length;
-    p.T = T;
-    p.ops = ops;
-    p.flags = flags;
-    p.seed = random ? seed : 0;
-    p.step_offset = random ? step_offset : 0;
+    StepParams p = record_params(state_in, state_out, host_action_t, axis_t, obs_t, agent_obs, host_mask_t, axis_played_t,
+                                 done_t, reward_t, done_count, length, B, N, d, T, ops, flags, padding_value, seed,
+                                 step_offset);
+    return run(p, dtype, g_force_generic.load(), (cudaStream_t)stream);
+}
+
+int hk_rollout_threshold(const void* state_in, void* state_out, const int32_t* host_action_t, const int32_t* axis_t,
+                         float* obs_t, int32_t agent_obs, int32_t* host_mask_t, int32_t* axis_played_t, uint8_t* done_t,
+                         float* reward_t, int32_t* done_count, int32_t* length, int64_t B, int32_t N, int32_t d, int32_t T,
+                         int32_t dtype, uint32_t ops, uint32_t flags, float padding_value, uint64_t seed, int32_t step_offset,
+                         float value_threshold, int32_t stop_at_threshold, int32_t* over_step, void* stream) {
+    if (T < 1 || (agent_obs && !obs_t) || value_threshold != value_threshold) return HK_ERR_BAD_ARG;
+    const bool never = value_threshold == INFINITY;
+    // int32 state: inputs below the threshold give shift sums below 2^30, the range in which the kernels are exact
+    if (dtype == HK_DTYPE_I32 && !never && d >= 1 && (double)value_threshold > (double)((1 << 30) / d)) return HK_ERR_BAD_ARG;
+    StepParams p = record_params(state_in, state_out, host_action_t, axis_t, obs_t, agent_obs, host_mask_t, axis_played_t,
+                                 done_t, reward_t, done_count, length, B, N, d, T, ops, flags, padding_value, seed,
+                                 step_offset);
+    // without over_step and without a stop (+inf stops nothing) the call is the recorded rollout as it is
+    p.threshold = value_threshold;
+    p.over_step = over_step;
+    p.stop_at_threshold = (stop_at_threshold && !never) ? 1 : 0;
     return run(p, dtype, g_force_generic.load(), (cudaStream_t)stream);
 }
 

@@ -129,7 +129,11 @@ __device__ __forceinline__ void generic_features(const T* x, uint32_t mylive, fl
 // REC: recorded rollouts (hk_rollout_record, with OBS for the feature buffer): every game takes the padded route,
 // whose step loop writes the features of the state before each step to row st of p.obs_t and the played actions after
 // the shift.
-template <typename T, int D, bool OBS, int RT, int DEPTH, bool HOT, bool CENSUS = false, bool REC = false>
+// THR: rollouts with a value threshold (hk_rollout_threshold, recorded with REC): the crossing step of every game, from
+// its live entries on entry and after every step (one vote over the rows the warp holds), goes to p.over_step; with
+// p.stop_at_threshold a game that has crossed sits out the later steps of both routes and writes its per-step outputs
+// as an ended game that does not change: its done flag again, no reward, (REC) no action.
+template <typename T, int D, bool OBS, int RT, int DEPTH, bool HOT, bool CENSUS = false, bool REC = false, bool THR = false>
 __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(const StepParams p, int warps_per_cta, int slot_words) {
     constexpr int NBUF = DEPTH + 1;
     // HOT: the plain random-play step (shift + reposition + newton, discrete host ids, int32 action arrays,
@@ -159,7 +163,7 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
     const int OW = W + ((REC ? p.agent_obs : p.obs_coord != nullptr) ? D : 0);
     const bool inplace = (gout == gin) && !(kflags & HK_F_STORE_ALL);
     // the short path for ended games covers plain single steps only
-    const bool ended_fast_path = !REC &&
+    const bool ended_fast_path = !REC && !THR &&
         kT == 1 && !(OBS && p.obs) && !p.host_out && !(kops & ~(HK_OP_SHIFT | HK_OP_REPOSITION | HK_OP_NEWTON)) &&
         !(kflags & (HK_F_HOST_ALL_COORD | HK_F_HOST_ZEILLINGER | HK_F_AGENT_FIRST | HK_F_AGENT_LAST));
     const bool compact_path = !REC &&
@@ -327,6 +331,18 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
             cnt += __popc(__ballot_sync(0xffffffffu, lv));
             mylive |= lv ? (1u << r) : 0u;
         }
+        int32_t over = kT + 1;  // (THR) the crossing step, kT + 1 while the game stays below the threshold
+        if constexpr (THR) {
+            bool e = false;
+            _Pragma("unroll UNR")
+            for (int r = 0; r < R; ++r) {
+                const int i = lane + 32 * r;
+                if (i >= N || !((mylive >> r) & 1u)) continue;
+#pragma unroll
+                for (int k = 0; k < D; ++k) e = e || (Elem<T>::to_float(x[i * D + k]) >= p.threshold);
+            }
+            if (__any_sync(0xffffffffu, e)) over = 0;
+        }
         // ---- ended games, single step: a short path of their own ----
         // Most games of a long rollout have at most one live row; nothing of the machinery below
         // (ballot rounds, the step loop, the filter) applies to them.  The lone row's lane plays the
@@ -455,6 +471,17 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
             int32_t len = kT + 1;
             int npairs = (ccnt + 1) >> 1;
             for (int st = 0; st < kT; ++st) {
+                if constexpr (THR) {
+                    if (p.stop_at_threshold && over <= st) {  // stopped at the threshold: the game sits out the step
+                        const bool dn = cur < 2;
+                        if (lane == 0) {
+                            if (p.done) p.done[(long long)st * p.B + g] = dn ? 1 : 0;
+                            if (p.reward) p.reward[(long long)st * p.B + g] = (kflags & HK_F_ROLE_AGENT) ? -0.0f : 0.0f;
+                        }
+                        if (p.done_count && dn) count_done(st);
+                        continue;
+                    }
+                }
                 if (st > 0 && cur >= 2 && 2 * cur <= ccnt) {
                     // Half of the listed rows have died: rebuild the list from the survivors so that the
                     // filter's cost keeps following the live count.  Rows that died go back to their slots
@@ -563,6 +590,16 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
                 }
                 if (p.done_count && dn) count_done(st);
                 if (dn && !prev_done) len = st + 1;
+                if constexpr (THR) {
+                    if (over > kT) {
+                        bool e = false;
+                        if (alive) {
+#pragma unroll
+                            for (int k = 0; k < D; ++k) e = e || (Elem<T>::to_float(v[k]) >= p.threshold);
+                        }
+                        if (__any_sync(0xffffffffu, e)) over = st + 1;
+                    }
+                }
                 ha = ha_n;
                 ax = ax_n;
             }
@@ -617,6 +654,9 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
             if (lane == 0) {
                 if (p.num_points) p.num_points[g] = cur;
                 if (p.length) p.length[g] = len;
+                if constexpr (THR) {
+                    if (p.over_step) p.over_step[g] = over;
+                }
             }
             if (p.exceed_flag) {
                 if (__any_sync(0xffffffffu, exceed) && lane == 0) *p.exceed_flag = 1;
@@ -642,6 +682,26 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
                 if (p.obs_t) {
                     gobs_t = p.obs_t + ((long long)st * p.B + g) * OW;
                     generic_features<T, D, RT>(x, mylive, f, gobs_t, N, R, lane, kflags, p.pad);
+                }
+            }
+            if constexpr (THR) {
+                if (p.stop_at_threshold && over <= st) {  // stopped at the threshold: the game sits out the step
+                    const bool dn = cnt < 2;
+                    if (lane == 0) {
+                        if (p.done) p.done[(long long)st * p.B + g] = dn ? 1 : 0;
+                        if (p.reward) p.reward[(long long)st * p.B + g] = (kflags & HK_F_ROLE_AGENT) ? -0.0f : 0.0f;
+                        if constexpr (REC) {
+                            const long long o = (long long)st * p.B + g;
+                            if (p.host_mask_t) p.host_mask_t[o] = 0;
+                            if (p.axis_played_t) p.axis_played_t[o] = -1;
+                        }
+                    }
+                    if constexpr (REC) {
+                        if (gobs_t && p.agent_obs && lane < D) gobs_t[W + lane] = 0.0f;
+                    }
+                    if (p.done_count && dn) count_done(st);
+                    __syncwarp();
+                    continue;
                 }
             }
             int32_t ha_n = 3, ax_n = 0;
@@ -967,6 +1027,19 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
             }
             if (p.done_count && dn) count_done(st);
             if (dn && !prev_done) len = st + 1;
+            if constexpr (THR) {
+                if (over > kT) {
+                    bool e = false;
+                    _Pragma("unroll UNR")
+                    for (int r = 0; r < R; ++r) {
+                        const int i = lane + 32 * r;
+                        if (i >= N || !((mylive >> r) & 1u)) continue;
+#pragma unroll
+                        for (int k = 0; k < D; ++k) e = e || (Elem<T>::to_float(x[i * D + k]) >= p.threshold);
+                    }
+                    if (__any_sync(0xffffffffu, e)) over = st + 1;
+                }
+            }
             ha = ha_n;
             ax = ax_n;
             __syncwarp();
@@ -1016,6 +1089,9 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
         if (lane == 0) {
             if (p.num_points) p.num_points[g] = cnt;
             if (p.length) p.length[g] = len;
+            if constexpr (THR) {
+                if (p.over_step) p.over_step[g] = over;
+            }
         }
         if (p.exceed_flag) {
             if (__any_sync(0xffffffffu, exceed) && lane == 0) *p.exceed_flag = 1;

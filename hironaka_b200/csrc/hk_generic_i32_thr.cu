@@ -1,0 +1,5 @@
+// warp-per-game kernel, int32 state, rollouts with a value threshold (hk_rollout_threshold)
+#include "hk_generic_launch.inl"
+namespace hk {
+int launch_generic_i32_thr(const StepParams& p, bool rec, int dev, cudaStream_t stream) { return dispatch_generic_threshold<int32_t>(p, rec, dev, stream); }
+}  // namespace hk

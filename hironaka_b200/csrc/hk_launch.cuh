@@ -68,5 +68,10 @@ int launch_small_i32_rec(const StepParams& p, int dev, cudaStream_t stream);
 int launch_small_f32_rec(const StepParams& p, int dev, cudaStream_t stream);
 int launch_generic_i32_rec(const StepParams& p, int dev, cudaStream_t stream);
 int launch_generic_f32_rec(const StepParams& p, int dev, cudaStream_t stream);
+// rollouts with a value threshold (hk_rollout_threshold), recorded (`rec`) or not, instantiations of their own in both families
+int launch_small_i32_thr(const StepParams& p, bool rec, int dev, cudaStream_t stream);
+int launch_small_f32_thr(const StepParams& p, bool rec, int dev, cudaStream_t stream);
+int launch_generic_i32_thr(const StepParams& p, bool rec, int dev, cudaStream_t stream);
+int launch_generic_f32_thr(const StepParams& p, bool rec, int dev, cudaStream_t stream);
 
 }  // namespace hk

@@ -333,9 +333,15 @@ __device__ __forceinline__ uint32_t zeillinger_rows(const T (&y)[K * D], uint32_
 // POLICY: instantiation that can evaluate the fixed players (kept out of the ordinary step kernels)
 // REC: recorded rollouts; `played` receives the coordinate bitmask and the axis the shift used (a fixed host on a game
 // without live rows records 0, as hk_host_policy reports it)
-template <typename T, int N, int D, int RS = 0, bool POLICY = false, bool REC = false>
+// THR: rollouts with a value threshold; a game stopped there (`frozen`) takes part in the warp-wide votes of the step
+// with no live row and keeps its live mask and its live rows as they are (dead rows may change: they are padded on the
+// way out).  The Newton filter runs on its rows as they are (it only rewrites dead rows) and its result is dropped.
+template <typename T, int N, int D, int RS = 0, bool POLICY = false, bool REC = false, bool THR = false>
 __device__ __forceinline__ uint32_t game_step(T (&x)[N * D], uint32_t lm, uint32_t ops, uint32_t flags, int32_t ha,
-                                              int32_t ax_in, uint32_t* scratch = nullptr, uint32_t* played = nullptr) {
+                                              int32_t ax_in, uint32_t* scratch = nullptr, uint32_t* played = nullptr,
+                                              bool frozen = false) {
+    const uint32_t lm_in = lm;
+    if constexpr (THR) lm = frozen ? 0u : lm;
     if (ops & HK_OP_SHIFT) {
         uint32_t cm;
         int ax = ax_in;
@@ -362,15 +368,19 @@ __device__ __forceinline__ uint32_t game_step(T (&x)[N * D], uint32_t lm, uint32
     }
     if (ops & HK_OP_REPOSITION) op_reposition<T, N, D>(x, lm);
     if (ops & HK_OP_NEWTON) {
+        const uint32_t lm_f = THR ? (frozen ? lm_in : lm) : lm;
+        uint32_t nl;
         if constexpr (RS > 0) {
-            lm = op_newton_rolled<T, N, D, RS>(x, lm, scratch);
+            nl = op_newton_rolled<T, N, D, RS>(x, lm_f, scratch);
         } else {
-            lm = op_newton<T, N, D>(x, lm);
+            nl = op_newton<T, N, D>(x, lm_f);
         }
+        lm = (THR && frozen) ? 0u : nl;
     }
     if constexpr (Elem<T>::is_float) {
         if (ops & HK_OP_RESCALE) op_rescale<N, D>(x, lm, flags & HK_F_RESCALE_EPS);
     }
+    if constexpr (THR) lm = frozen ? lm_in : lm;
     return lm;
 }
 
@@ -398,6 +408,7 @@ struct LaneState {
     int32_t len;
     bool origin;  // census only: no live row, or the lone live row sits at the origin (a fixed point of every op)
     uint32_t played[2];  // recorded rollouts: the host's coordinate bitmask and the axis of the last step (0 without a shift)
+    int32_t over;        // value thresholds: the crossing step as p.over_step reports it (T + 1 while below)
 };
 
 __host__ __device__ constexpr int next_lower_tier(int K) {
@@ -407,7 +418,10 @@ __host__ __device__ constexpr int next_lower_tier(int K) {
 // Runs steps [st, T) of one tile on K compact rows; returns the step index at which it stopped
 // (T, or earlier when every game of the warp fits the next lower tier; REC: after one step).  The lane's game area in
 // shared memory (`row`) holds the current state on entry and on exit.
-template <typename T, int N, int D, int K, bool POLICY, bool REC = false>
+// THR (hk_rollout_threshold): after every step a game that has not crossed yet compares its live entries with the
+// threshold; with p.stop_at_threshold a game that has crossed sits out the later steps (game_step, `frozen`) and writes
+// its per-step outputs as an ended game that does not change: its done flag again, no reward, (REC) no action.
+template <typename T, int N, int D, int K, bool POLICY, bool REC = false, bool THR = false>
 __device__ __forceinline__ int tier_steps(const StepParams& p, LaneState& ls, uint32_t* row, uint32_t lm, int st,
                                           bool& exceed, bool& chg) {
     const long long B = p.B;
@@ -460,7 +474,17 @@ __device__ __forceinline__ int tier_steps(const StepParams& p, LaneState& ls, ui
         }
         const bool prev_done = ls.cnt < 2;
         if constexpr (REC) ls.played[0] = ls.played[1] = 0u;
-        clm = game_step<T, K, D, RS, POLICY, REC>(y, clm, p.ops, p.flags, ls.ha, ls.ax, row, ls.played);
+        const bool frozen = THR && p.stop_at_threshold && ls.over <= st;
+        clm = game_step<T, K, D, RS, POLICY, REC, THR>(y, clm, p.ops, p.flags, ls.ha, ls.ax, row, ls.played, frozen);
+        if constexpr (THR) {
+            if constexpr (REC) {
+                if (frozen) {
+                    ls.played[0] = 0u;
+                    ls.played[1] = 0xffffffffu;  // axis -1: no move
+                }
+            }
+            if (ls.over > p.T && exceeds<T, K, D>(y, clm, p.threshold)) ls.over = st + 1;
+        }
         if (K <= 4 && p.T == 1) {
             bool diff = (clm != clm_before) || (clm_before > 1u);  // compact rows fill from 0: > 1 means two or more rows
 #pragma unroll
@@ -1149,13 +1173,16 @@ struct NoRec {
     __device__ __forceinline__ void operator()(int, bool) const {}
 };
 
-template <typename T, int N, int D, bool POLICY, bool PACKED = true, typename Release = NoRelease, typename Rec = NoRec>
+// THR (hk_rollout_threshold): ls.over is set from the state on entry and kept by the tiers (tier_steps).
+template <typename T, int N, int D, bool POLICY, bool PACKED = true, typename Release = NoRelease, typename Rec = NoRec,
+          bool THR = false>
 __device__ __forceinline__ bool small_process_tile(const StepParams& p, LaneState& ls, uint32_t* row, bool& exceed,
                                                    bool& chg, uint32_t* gdst = nullptr, Release release = Release(),
                                                    Rec rec = Rec()) {
     constexpr int W = N * D;
     constexpr bool REC = !std::is_same<Rec, NoRec>::value;
     static_assert(!(REC && PACKED), "a recorded rollout steps on the exact tiers only");
+    static_assert(!(THR && PACKED), "a rollout with a value threshold steps on the exact tiers only");
     const T padv = Elem<T>::pad(p.pad);
     const bool mutate = p.ops != 0;
     bool normalised = false;
@@ -1198,6 +1225,9 @@ __device__ __forceinline__ bool small_process_tile(const StepParams& p, LaneStat
                 diff |= dr & sgn;
             }
             lm = ~dead & ((N == 32) ? 0xffffffffu : ((1u << N) - 1u));
+            if constexpr (THR) {
+                if (st == 0) ls.over = exceeds<T, N, D>(x, lm, p.threshold) ? 0 : p.T + 1;
+            }
             if (check) {
                 chg = chg || (diff != 0);
                 any_junk = __any_sync(0xffffffffu, diff != 0);
@@ -1274,23 +1304,23 @@ __device__ __forceinline__ bool small_process_tile(const StepParams& p, LaneStat
         }
         if (N > 2 && p.T == 1 && lmax <= 2) {  // the tail of a rollout driven step by step: ended games and two-point games only
             prestore();
-            st = tier_steps<T, N, D, (N > 2 ? 2 : N), POLICY, REC>(p, ls, row, lm, st, exceed, chg);
+            st = tier_steps<T, N, D, (N > 2 ? 2 : N), POLICY, REC, THR>(p, ls, row, lm, st, exceed, chg);
         } else if (N > 4 && lmax <= 4) {
             prestore();
-            st = tier_steps<T, N, D, (N > 4 ? 4 : N), POLICY, REC>(p, ls, row, lm, st, exceed, chg);
+            st = tier_steps<T, N, D, (N > 4 ? 4 : N), POLICY, REC, THR>(p, ls, row, lm, st, exceed, chg);
         } else if (N > 8 && lmax <= 8) {
             prestore();
-            st = tier_steps<T, N, D, (N > 8 ? 8 : N), POLICY, REC>(p, ls, row, lm, st, exceed, chg);
+            st = tier_steps<T, N, D, (N > 8 ? 8 : N), POLICY, REC, THR>(p, ls, row, lm, st, exceed, chg);
         } else if (N > 12 && lmax <= 12) {
             if (W % 4 != 0) prestore();
-            st = tier_steps<T, N, D, (N > 12 ? 12 : N), POLICY, REC>(p, ls, row, lm, st, exceed, chg);
+            st = tier_steps<T, N, D, (N > 12 ? 12 : N), POLICY, REC, THR>(p, ls, row, lm, st, exceed, chg);
             normalised = normalised || (W % 4 == 0);
         } else if (N > 16 && lmax <= 16) {
             if (W % 4 != 0) prestore();
-            st = tier_steps<T, N, D, (N > 16 ? 16 : N), POLICY, REC>(p, ls, row, lm, st, exceed, chg);
+            st = tier_steps<T, N, D, (N > 16 ? 16 : N), POLICY, REC, THR>(p, ls, row, lm, st, exceed, chg);
             normalised = normalised || (W % 4 == 0);
         } else {
-            st = tier_steps<T, N, D, N, POLICY, REC>(p, ls, row, lm, st, exceed, chg);
+            st = tier_steps<T, N, D, N, POLICY, REC, THR>(p, ls, row, lm, st, exceed, chg);
             normalised = true;
         }
         if constexpr (REC) rec(st0, true);
@@ -1307,7 +1337,8 @@ __device__ __forceinline__ void warp_copy_words(uint32_t* dst, const uint32_t* s
 // by instruction fetch: they do not carry that code.
 // REC: recorded rollouts (hk_small_record_kernel): before every step the features of the state go to the warp's obs
 // tile, after it the played actions are written and the tile leaves with one bulk store into row st of p.obs_t.
-template <typename T, int N, int D, bool OBS, bool POLICY, int WARPS, int STAGES, bool PACKED, bool REC>
+// THR: rollouts with a value threshold (hk_small_threshold_kernel), recorded (REC) or not; p.over_step leaves with length.
+template <typename T, int N, int D, bool OBS, bool POLICY, int WARPS, int STAGES, bool PACKED, bool REC, bool THR = false>
 __device__ __forceinline__ void small_kernel_body(const StepParams& p) {
     using L = SmallLayout<N, D, OBS || REC, WARPS, STAGES>;
     constexpr int SMALL_WARPS = WARPS;
@@ -1445,7 +1476,10 @@ __device__ __forceinline__ void small_kernel_body(const StepParams& p) {
                     __syncwarp();
                 }
             };
-            small_process_tile<T, N, D, POLICY, PACKED, NoRelease, decltype(rec)>(p, ls, row, exceed, chg, nullptr, NoRelease(), rec);
+            small_process_tile<T, N, D, POLICY, PACKED, NoRelease, decltype(rec), THR>(p, ls, row, exceed, chg, nullptr, NoRelease(),
+                                                                                   rec);
+        } else if constexpr (THR) {
+            small_process_tile<T, N, D, POLICY, PACKED, NoRelease, NoRec, THR>(p, ls, row, exceed, chg);
         } else if constexpr (HK_SMALL_DIRECT && PACKED && !OBS && !POLICY && SMALL_STAGES == 1 && !Elem<T>::is_float) {
             // packed tiers, direct route (tier_packed, DIRECT) of an in-place single step: the stage is refilled as soon as
             // the rows are gathered and the changed rows go straight to global memory
@@ -1467,6 +1501,9 @@ __device__ __forceinline__ void small_kernel_body(const StepParams& p) {
         if (ls.valid) {
             if (p.num_points) p.num_points[ls.g] = ls.cnt;
             if (p.length) p.length[ls.g] = ls.len;
+            if constexpr (THR) {
+                if (p.over_step) p.over_step[ls.g] = ls.over;
+            }
         }
         if (p.exceed_flag) {
             if (__any_sync(0xffffffffu, exceed && ls.valid) && lane == 0) *p.exceed_flag = 1;
@@ -1585,6 +1622,13 @@ __global__ void __launch_bounds__(WARPS * 32) hk_small_kernel(const StepParams p
 template <typename T, int N, int D, bool POLICY, int WARPS>
 __global__ void __launch_bounds__(WARPS * 32) hk_small_record_kernel(const StepParams p) {
     small_kernel_body<T, N, D, false, POLICY, WARPS, 1, false, true>(p);
+}
+
+// hk_rollout_threshold on the thread-per-game shapes: the rollout kernel's tile loop (REC: the recorded rollout's) with
+// the crossing step of every game and the stop, one stage per warp
+template <typename T, int N, int D, bool POLICY, int WARPS, bool REC>
+__global__ void __launch_bounds__(WARPS * 32) hk_small_threshold_kernel(const StepParams p) {
+    small_kernel_body<T, N, D, false, POLICY, WARPS, 1, false, REC, true>(p);
 }
 
 }  // namespace hk

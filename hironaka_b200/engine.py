@@ -55,6 +55,12 @@ class GameBatch:
                      (get_take_actions, hironaka/jax/util.py:117-123)
     semantics="torch": invalid actions and ended games are no-ops, order shift -> newton
                      (FusedGame.agent_move, hironaka/trainer/fused_game.py:150-162)
+
+    value_threshold: every step runs through hk_rollout_threshold, which follows each game against the threshold
+    (TensorPoints.value_threshold, hironaka/core/tensor_points.py:57-63): `crossed` (bool [B]) turns true once a
+    live entry of a game has reached it.  With stop_at_threshold a game that crosses is not stepped again (the gym
+    environments' stop_at_threshold); it enters every later call over the threshold, so it stays stopped.  For the
+    int32 state the threshold must be <= 2^30 / d.  `step` is then a one-step rollout without the census.
     """
 
     HOST_POLICIES = {None: 0, "stream": 0, "all_coord": C.HK_F_HOST_ALL_COORD, "zeillinger": C.HK_F_HOST_ZEILLINGER,
@@ -65,7 +71,7 @@ class GameBatch:
     def __init__(self, points: torch.Tensor, *, semantics: str = "jax", reposition: bool = True,
                  discrete_host_action: bool = True, role: str = "host", initial_filter: bool = False,
                  host_policy: Optional[str] = None, agent_policy: Optional[str] = None, census: bool = True,
-                 seed: int = 0):
+                 seed: int = 0, value_threshold: Optional[float] = None, stop_at_threshold: bool = False):
         if semantics not in ("jax", "torch"):
             raise ValueError("semantics must be 'jax' or 'torch'")
         if not points.is_cuda:
@@ -84,7 +90,12 @@ class GameBatch:
         # The census (one byte per game, hk_step_census) lets a step skip the games at rest and order the others
         # by live count.  It describes `self.points`: call reset_census() after writing into the tensor yourself.
         fixed = (self.HOST_POLICIES[host_policy] | self.AGENT_POLICIES[agent_policy]) & ~(C.HK_F_HOST_RANDOM | C.HK_F_AGENT_RANDOM)
-        self.census = _ops.new_census(self.points) if (census and not fixed) else None
+        self.value_threshold = None if value_threshold is None else float(value_threshold)
+        self.stop_at_threshold = bool(stop_at_threshold)
+        threshold = self.value_threshold is not None
+        self.census = _ops.new_census(self.points) if (census and not fixed and not threshold) else None
+        self.crossed = torch.zeros(self.B, dtype=torch.bool, device=self.device) if threshold else None
+        self._over_step = torch.empty(self.B, dtype=torch.int32, device=self.device) if threshold else None
         if initial_filter:  # generate_pts: newton -> (reposition) on the root states (util.py:385-392)
             _ops.step(self.points, ops=C.HK_OP_NEWTON | (C.HK_OP_REPOSITION if reposition else 0), inplace=True,
                       census=self.census)
@@ -96,9 +107,24 @@ class GameBatch:
     def step(self, host_action: Optional[torch.Tensor] = None, axis: Optional[torch.Tensor] = None,
              want_reward: bool = True):
         """One game-step in place; returns (done [B] bool, reward [B] f32 | None)."""
+        if self.value_threshold is not None:  # a one-step rollout that follows the threshold
+            ha = None if host_action is None else host_action.reshape(1, self.B)
+            ax = None if axis is None else axis.reshape(1, self.B)
+            done, reward, _, _ = self.rollout(ha, ax, want_done=True, want_reward=want_reward, want_length=False, steps=1)
+            return done[0], (None if reward is None else reward[0])
         r = _ops.step(self.points, host_action, axis, ops=self.ops, flags=self.flags, inplace=True, want_done=True,
                       want_reward=want_reward, census=self.census)
         return r.done, r.reward
+
+    def _threshold_args(self) -> dict:
+        if self.value_threshold is None:
+            return {}
+        return dict(value_threshold=self.value_threshold, stop_at_threshold=self.stop_at_threshold,
+                    over_step=self._over_step)
+
+    def _note_crossings(self, steps: int) -> None:
+        if self.value_threshold is not None:
+            self.crossed |= self._over_step <= steps
 
     def reset_census(self) -> None:
         """Forget what is known about the games (after `points` was written from outside)."""
@@ -115,12 +141,14 @@ class GameBatch:
             _, done, reward, dcount, length = _ops.rollout_random(
                 self.points, T, self.seed, ops=self.ops, flags=self.flags, host_actions=host_actions, axes=axes,
                 step_offset=self.steps_played, inplace=True, want_done=want_done, want_reward=want_reward,
-                want_length=want_length)
+                want_length=want_length, **self._threshold_args())
             self.steps_played += T
         else:
             _, done, reward, dcount, length = _ops.rollout(self.points, host_actions, axes, ops=self.ops, flags=self.flags,
                                                            inplace=True, want_done=want_done, want_reward=want_reward,
-                                                           want_done_count=True, want_length=want_length, steps=steps)
+                                                           want_done_count=True, want_length=want_length, steps=steps,
+                                                           **self._threshold_args())
+        self._note_crossings(dcount.shape[0])
         self.reset_census()  # the one-launch rollout does not keep it
         return done, reward, dcount, length
 
@@ -134,9 +162,11 @@ class GameBatch:
         obs_flags = (C.HK_F_OBS_RESCALE if scale_observation else 0) | \
             {"lex": C.HK_F_OBS_SORT_LEX, "coord0": C.HK_F_OBS_SORT_COORD0, "none": 0}[sort]
         traj = _ops.rollout_record(self.points, steps, host_actions, axes, ops=self.ops, flags=self.flags | obs_flags,
-                                   seed=self.seed, step_offset=self.steps_played, agent_obs=agent_obs, inplace=True)
+                                   seed=self.seed, step_offset=self.steps_played, agent_obs=agent_obs, inplace=True,
+                                   **self._threshold_args())
         if self.flags & (C.HK_F_HOST_RANDOM | C.HK_F_AGENT_RANDOM):
             self.steps_played += traj.done_count.shape[0]
+        self._note_crossings(traj.done_count.shape[0])
         self.reset_census()  # the one-launch rollout does not keep it
         return traj
 
@@ -151,7 +181,8 @@ class GameBatch:
         self._ha_dev[0].copy_(host_action_host, non_blocking=True)
         self._ax_dev[0].copy_(axis_host, non_blocking=True)
         _, _, _, dcount, _ = _ops.rollout(self.points, self._ha_dev, self._ax_dev, ops=self.ops, flags=self.flags,
-                                          inplace=True, want_done_count=True)
+                                          inplace=True, want_done_count=True, **self._threshold_args())
+        self._note_crossings(1)
         self.reset_census()
         return int(dcount.item())
 

@@ -178,10 +178,13 @@ def new_census(state: torch.Tensor) -> torch.Tensor:
 def rollout(state: torch.Tensor, host_actions: Optional[torch.Tensor], axes: Optional[torch.Tensor], *, ops: int,
             flags: int = 0, padding_value: float = -1.0, inplace: bool = True, want_done: bool = False,
             want_reward: bool = False, want_done_count: bool = True, want_length: bool = False,
-            steps: Optional[int] = None):
+            steps: Optional[int] = None, value_threshold: Optional[float] = None, stop_at_threshold: bool = False,
+            over_step: Optional[torch.Tensor] = None):
     """T fused steps in one launch (hk_rollout): host_actions / axes are int32 [T, B]; either may be
     None when the matching fixed-player flag (HK_F_HOST_* / HK_F_AGENT_*) is set, in which case
-    `steps` gives T if both are None."""
+    `steps` gives T if both are None.  With `value_threshold` the rollout runs through hk_rollout_threshold:
+    `over_step` (int32 [B], written when given) receives each game's crossing step, and `stop_at_threshold` stops
+    the games that cross."""
     dt = _require_state(state)
     B, N, d = state.shape
     dev = state.device
@@ -205,6 +208,10 @@ def rollout(state: torch.Tensor, host_actions: Optional[torch.Tensor], axes: Opt
     reward = torch.empty((T, B), dtype=torch.float32, device=dev) if want_reward else None
     dcount = torch.zeros(T, dtype=torch.int32, device=dev) if want_done_count else None
     length = torch.empty(B, dtype=torch.int32, device=dev) if want_length else None
+    if value_threshold is not None:
+        _rollout_threshold(state, dst, ha, ax, None, False, None, None, done, reward, dcount, length, T, dt, ops, flags,
+                           padding_value, 0, 0, value_threshold, stop_at_threshold, over_step)
+        return dst, (None if done is None else done.view(torch.bool)), reward, dcount, length
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream(dev).cuda_stream
         rc = lib().hk_rollout(_ptr(state), _ptr(dst), _ptr(ha), _ptr(ax), _ptr(done), _ptr(reward), _ptr(dcount),
@@ -215,10 +222,12 @@ def rollout(state: torch.Tensor, host_actions: Optional[torch.Tensor], axes: Opt
 
 def rollout_random(state: torch.Tensor, steps: int, seed: int, *, ops: int, flags: int = 0, host_actions=None, axes=None,
                    step_offset: int = 0, padding_value: float = -1.0, inplace: bool = True, want_done: bool = False,
-                   want_reward: bool = False, want_length: bool = False):
+                   want_reward: bool = False, want_length: bool = False, value_threshold: Optional[float] = None,
+                   stop_at_threshold: bool = False, over_step: Optional[torch.Tensor] = None):
     """`steps` fused steps with random players drawn INSIDE the kernel (hk_rollout_seeded): no [T, B] action streams.
     `flags` carries HK_F_HOST_RANDOM and / or HK_F_AGENT_RANDOM; the other player comes from its [T, B] stream or a
-    fixed-player flag.  Philox4x32-10 keyed by `seed`, counter (game, step_offset + t): see `random_actions`."""
+    fixed-player flag.  Philox4x32-10 keyed by `seed`, counter (game, step_offset + t): see `random_actions`.
+    `value_threshold`, `stop_at_threshold`, `over_step`: as in `rollout` (hk_rollout_threshold)."""
     dt = _require_state(state)
     B, N, d = state.shape
     dev = state.device
@@ -230,6 +239,12 @@ def rollout_random(state: torch.Tensor, steps: int, seed: int, *, ops: int, flag
     reward = torch.empty((T, B), dtype=torch.float32, device=dev) if want_reward else None
     dcount = torch.zeros(T, dtype=torch.int32, device=dev)
     length = torch.empty(B, dtype=torch.int32, device=dev) if want_length else None
+    if value_threshold is not None:
+        if not flags & (C.HK_F_HOST_RANDOM | C.HK_F_AGENT_RANDOM):
+            raise ValueError("rollout_random needs HK_F_HOST_RANDOM and / or HK_F_AGENT_RANDOM")
+        _rollout_threshold(state, dst, ha, ax, None, False, None, None, done, reward, dcount, length, T, dt, ops, flags,
+                           padding_value, seed, step_offset, value_threshold, stop_at_threshold, over_step)
+        return dst, (None if done is None else done.view(torch.bool)), reward, dcount, length
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream(dev).cuda_stream
         rc = lib().hk_rollout_seeded(_ptr(state), _ptr(dst), _ptr(ha), _ptr(ax), _ptr(done), _ptr(reward), _ptr(dcount),
@@ -237,6 +252,24 @@ def rollout_random(state: torch.Tensor, steps: int, seed: int, *, ops: int, flag
                                      int(step_offset), stream)
     check(rc, "hk_rollout_seeded")
     return dst, (None if done is None else done.view(torch.bool)), reward, dcount, length
+
+
+def _rollout_threshold(state, dst, ha, ax, obs, agent_obs, hmask, axis, done, reward, dcount, length, T, dt, ops, flags,
+                       padding_value, seed, step_offset, value_threshold, stop_at_threshold, over_step):
+    """hk_rollout_threshold on buffers the public entry points have prepared; `over_step` is the caller's int32 [B]."""
+    B, N, d = state.shape
+    dev = state.device
+    if over_step is not None and (over_step.dtype != torch.int32 or tuple(over_step.shape) != (B,) or
+                                  over_step.device != dev or not over_step.is_contiguous()):
+        raise ValueError("over_step must be a contiguous int32 [B] tensor on the state's device")
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        rc = lib().hk_rollout_threshold(_ptr(state), _ptr(dst), _ptr(ha), _ptr(ax), _ptr(obs), 1 if agent_obs else 0,
+                                        _ptr(hmask), _ptr(axis), _ptr(done), _ptr(reward), _ptr(dcount), _ptr(length), B, N,
+                                        d, T, dt, ops, flags, float(padding_value), int(seed) & (2 ** 64 - 1),
+                                        int(step_offset), float(value_threshold), 1 if stop_at_threshold else 0,
+                                        _ptr(over_step), stream)
+    check(rc, "hk_rollout_threshold")
 
 
 class Trajectory(NamedTuple):
@@ -254,14 +287,16 @@ def rollout_record(state: torch.Tensor, steps: Optional[int] = None, host_action
                    axes: Optional[torch.Tensor] = None, *, ops: int, flags: int = 0, seed: int = 0, step_offset: int = 0,
                    want_obs: bool = True, agent_obs: bool = False, want_actions: bool = True, want_done: bool = True,
                    want_reward: bool = True, want_length: bool = True, inplace: bool = True,
-                   padding_value: float = -1.0) -> Trajectory:
+                   padding_value: float = -1.0, value_threshold: Optional[float] = None, stop_at_threshold: bool = False,
+                   over_step: Optional[torch.Tensor] = None) -> Trajectory:
     """T fused steps in one launch that also record the trajectory (hk_rollout_record): obs[t] are the features of the
     state the players see at step t (the observation flags of `features`), host_mask / axis what step t played, as
     bitmasks and axes (replayed through `rollout` without HK_F_ACT_DISCRETE and the player flags they give the same
     rollout).  `agent_obs` appends step t's host coordinates to obs[t] as d floats 0/1.  The players are [T, B] int32
     streams, fixed-player flags, or the in-kernel random players (HK_F_HOST_RANDOM / HK_F_AGENT_RANDOM, keyed by `seed`
     and `step_offset`); `steps` gives T when no stream does.  The features after the last step are
-    features(trajectory.state)."""
+    features(trajectory.state).  `value_threshold`, `stop_at_threshold`, `over_step`: as in `rollout`
+    (hk_rollout_threshold); a stopped game records the features of its frozen state, host_mask 0 and axis -1."""
     dt = _require_state(state)
     B, N, d = state.shape
     dev = state.device
@@ -283,6 +318,10 @@ def rollout_record(state: torch.Tensor, steps: Optional[int] = None, host_action
     reward = torch.empty((T, B), dtype=torch.float32, device=dev) if want_reward else None
     dcount = torch.zeros(T, dtype=torch.int32, device=dev)
     length = torch.empty(B, dtype=torch.int32, device=dev) if want_length else None
+    if value_threshold is not None:
+        _rollout_threshold(state, dst, ha, ax, obs, agent_obs, hmask, axis, done, reward, dcount, length, T, dt, ops, flags,
+                           padding_value, seed, step_offset, value_threshold, stop_at_threshold, over_step)
+        return Trajectory(dst, obs, hmask, axis, None if done is None else done.view(torch.bool), reward, dcount, length)
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream(dev).cuda_stream
         rc = lib().hk_rollout_record(_ptr(state), _ptr(dst), _ptr(ha), _ptr(ax), _ptr(obs), 1 if agent_obs else 0, _ptr(hmask),

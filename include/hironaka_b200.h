@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define HK_VERSION 101 /* major*100 + minor */
+#define HK_VERSION 102 /* major*100 + minor */
 
 /* ---- status codes ---------------------------------------------------------------- */
 #define HK_OK 0
@@ -263,6 +263,33 @@ int hk_rollout_record(const void* state_in, void* state_out, const int32_t* host
                       float* reward_t, int32_t* done_count, int32_t* length, int64_t B, int32_t N, int32_t d, int32_t T,
                       int32_t dtype, uint32_t ops, uint32_t flags, float padding_value, uint64_t seed, int32_t step_offset,
                       void* stream);
+
+/* ---- rollout with a value threshold ---------------------------------------------------------
+ * hk_rollout_record that also follows every game against a value threshold (TensorPoints.value_threshold and
+ * exceed_threshold, the gym environments' stop_at_threshold), inside the one launch.  A game has crossed when a live
+ * entry is >= value_threshold (non-strict, compared as float32 like hk_overflow with strict = 0; for integer states a
+ * strict threshold v is v + 1).
+ *   over_step [B] int32, nullable, laid out like length: 0 if the input state has already crossed, t + 1 for the first
+ *             step t after which it has, T + 1 if it never does.
+ *   stop_at_threshold != 0: a game that has crossed (on entry or after step t) is not stepped again in this call.  Its
+ *             state stays as it was after the crossing step (on entry: as read, dead rows padded), done_t repeats its
+ *             done flag and done_count counts it by that flag, reward_t is 0.0 (-0.0 with HK_F_ROLE_AGENT), length
+ *             stays T + 1 unless it was already done; obs_t rows are the features of the frozen state, host_mask_t 0
+ *             and axis_played_t -1 for the steps it sits out.  The in-kernel random players stay keyed by
+ *             (game, step): every other game plays as without the stop.  Since a stopped game enters the next call
+ *             over the threshold, it stays stopped across calls.  Replayed as streams through this call with the same
+ *             threshold and stop flag, the recorded actions give the rollout back bit for bit.
+ *   Without the stop, games play on after they cross; over_step says from which step a game's int32 results can no
+ *   longer be trusted (int32 results are exact below 2^30).
+ * value_threshold: NaN is HK_ERR_BAD_ARG; with int32 state a finite threshold must be <= floor(2^30 / d)
+ * (HK_ERR_BAD_ARG otherwise): live inputs below it give shift sums below 2^30, so with the stop every state the kernel
+ * holds or writes is exact (1e8, the reference's default, passes for every d <= 10).  +inf never crosses; with +inf
+ * and over_step null the call is hk_rollout_record (same kernels, same results). */
+int hk_rollout_threshold(const void* state_in, void* state_out, const int32_t* host_action_t, const int32_t* axis_t,
+                         float* obs_t, int32_t agent_obs, int32_t* host_mask_t, int32_t* axis_played_t, uint8_t* done_t,
+                         float* reward_t, int32_t* done_count, int32_t* length, int64_t B, int32_t N, int32_t d, int32_t T,
+                         int32_t dtype, uint32_t ops, uint32_t flags, float padding_value, uint64_t seed, int32_t step_offset,
+                         float value_threshold, int32_t stop_at_threshold, int32_t* over_step, void* stream);
 
 /* ---- experience writer (SURVEY 8f rank 2) --------------------------------------------------------
  * Appends the rows with skip[b] == 0, IN BATCH ORDER, to circular replay buffers at
