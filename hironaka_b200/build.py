@@ -21,7 +21,7 @@ OUT_DIR = os.path.join(HERE, "_lib")
 OBJ_DIR = os.path.join(OUT_DIR, "obj")
 OUT = os.path.join(OUT_DIR, "libhironaka_b200.so")
 SOURCES = ["hk_capi.cu", "hk_small_i32_step.cu", "hk_small_i32_obs.cu", "hk_small_f32_step.cu", "hk_small_f32_obs.cu",
-           "hk_generic_i32.cu", "hk_generic_f32.cu", "hk_sched_i32.cu", "hk_sched_f32.cu", "hk_sched_i32_obs.cu", "hk_sched_f32_obs.cu", "hk_rows_i32.cu", "hk_rows_f32.cu",
+           "hk_generic_i32_plain_obs.cu", "hk_generic_f32_plain_obs.cu", "hk_sched_i32.cu", "hk_sched_f32.cu", "hk_sched_i32_obs.cu", "hk_sched_f32_obs.cu", "hk_rows_i32.cu", "hk_rows_f32.cu",
            "hk_small_i32_rec.cu", "hk_small_f32_rec.cu", "hk_generic_i32_rec.cu", "hk_generic_f32_rec.cu",
            "hk_small_i32_thr.cu", "hk_small_f32_thr.cu", "hk_generic_i32_thr.cu", "hk_generic_f32_thr.cu"]
 HEADERS = ["hk_common.cuh", "hk_small.cuh", "hk_generic.cuh", "hk_experience.cuh", "hk_value.cuh", "hk_launch.cuh",

@@ -15,21 +15,10 @@
 #include "hk_launch.cuh"
 #include "hk_value.cuh"
 
+using hk::GenericVariant;
+using hk::SmallVariant;
 using hk::StepParams;
 using hk::kMaxDevices;
-
-namespace hk {
-int launch_small_i32_noobs(const StepParams& p, int dev, cudaStream_t stream);
-int launch_small_i32_obs(const StepParams& p, int dev, cudaStream_t stream);
-int launch_small_f32_noobs(const StepParams& p, int dev, cudaStream_t stream);
-int launch_small_f32_obs(const StepParams& p, int dev, cudaStream_t stream);
-int launch_small_i32(const StepParams& p, bool obs, int dev, cudaStream_t stream) {
-    return obs ? launch_small_i32_obs(p, dev, stream) : launch_small_i32_noobs(p, dev, stream);
-}
-int launch_small_f32(const StepParams& p, bool obs, int dev, cudaStream_t stream) {
-    return obs ? launch_small_f32_obs(p, dev, stream) : launch_small_f32_noobs(p, dev, stream);
-}
-}  // namespace hk
 
 namespace {
 
@@ -58,6 +47,32 @@ int check_shape(long long B, int N, int d, int dtype) {
     if (dtype != HK_DTYPE_I32 && dtype != HK_DTYPE_F32) return HK_ERR_BAD_ARG;
     if (d > HK_MAX_DIM || N > HK_MAX_POINTS || (long long)N * d > HK_MAX_GAME_WORDS) return HK_ERR_UNSUPPORTED;
     return HK_OK;
+}
+
+// the variant of the one-launch kernels a call needs, from the outputs it asks for
+SmallVariant rollout_variant(const StepParams& p) {
+    const bool rec = p.obs_t || p.host_mask_t || p.axis_played_t;
+    if (p.over_step || p.stop_at_threshold) return rec ? SmallVariant::ThrRec : SmallVariant::Thr;
+    if (rec) return SmallVariant::Rec;
+    return p.obs ? SmallVariant::Obs : SmallVariant::Step;
+}
+
+// the thread-per-game family (`small`) or the warp-per-game family, in variant V
+template <typename T, SmallVariant V>
+int launch_variant(const StepParams& p, bool small, int dev, cudaStream_t stream) {
+    return small ? hk::dispatch_small<T, V>(p, dev, stream) : hk::dispatch_generic<T, hk::generic_variant(V)>(p, dev, stream);
+}
+
+template <typename T>
+int launch_family(const StepParams& p, bool small, int dev, cudaStream_t stream) {
+    switch (rollout_variant(p)) {
+        case SmallVariant::Step: return launch_variant<T, SmallVariant::Step>(p, small, dev, stream);
+        case SmallVariant::Obs: return launch_variant<T, SmallVariant::Obs>(p, small, dev, stream);
+        case SmallVariant::Rec: return launch_variant<T, SmallVariant::Rec>(p, small, dev, stream);
+        case SmallVariant::Thr: return launch_variant<T, SmallVariant::Thr>(p, small, dev, stream);
+        case SmallVariant::ThrRec: return launch_variant<T, SmallVariant::ThrRec>(p, small, dev, stream);
+    }
+    return HK_ERR_UNSUPPORTED;
 }
 
 int run(StepParams& p, int dtype, int force_generic, cudaStream_t stream) {
@@ -122,24 +137,12 @@ int run(StepParams& p, int dtype, int force_generic, cudaStream_t stream) {
             e = cudaMemsetAsync(p.done_bits, 0, (size_t)((p.B + 31) / 32) * 4, stream);
             if (e != cudaSuccess) return (int)e;
         }
-        return dtype == HK_DTYPE_I32 ? hk::launch_generic_i32(p, false, dev, stream) : hk::launch_generic_f32(p, false, dev, stream);
+        return dtype == HK_DTYPE_I32 ? hk::dispatch_generic<int32_t, GenericVariant::Plain>(p, dev, stream)
+                                     : hk::dispatch_generic<float, GenericVariant::Plain>(p, dev, stream);
     }
     // remove_repeated alone is not on the step path: it runs on the warp-per-game kernel for every shape
     const bool small = hk::is_small_shape(p.N, p.d) && !force_generic && !(p.ops & HK_OP_DEDUPE);
-    if (p.over_step || p.stop_at_threshold) {  // a rollout with a value threshold, recorded or not: instantiations of their own
-        const bool rec = p.obs_t || p.host_mask_t || p.axis_played_t;
-        if (dtype == HK_DTYPE_I32)
-            return small ? hk::launch_small_i32_thr(p, rec, dev, stream) : hk::launch_generic_i32_thr(p, rec, dev, stream);
-        return small ? hk::launch_small_f32_thr(p, rec, dev, stream) : hk::launch_generic_f32_thr(p, rec, dev, stream);
-    }
-    if (p.obs_t || p.host_mask_t || p.axis_played_t) {  // a recorded rollout: instantiations of its own
-        if (dtype == HK_DTYPE_I32)
-            return small ? hk::launch_small_i32_rec(p, dev, stream) : hk::launch_generic_i32_rec(p, dev, stream);
-        return small ? hk::launch_small_f32_rec(p, dev, stream) : hk::launch_generic_f32_rec(p, dev, stream);
-    }
-    if (dtype == HK_DTYPE_I32)
-        return small ? hk::launch_small_i32(p, obs, dev, stream) : hk::launch_generic_i32(p, obs, dev, stream);
-    return small ? hk::launch_small_f32(p, obs, dev, stream) : hk::launch_generic_f32(p, obs, dev, stream);
+    return dtype == HK_DTYPE_I32 ? launch_family<int32_t>(p, small, dev, stream) : launch_family<float>(p, small, dev, stream);
 }
 
 StepParams make_params(const void* in, void* out, long long B, int N, int d, float pad) {
@@ -156,11 +159,13 @@ StepParams make_params(const void* in, void* out, long long B, int N, int d, flo
     return p;
 }
 
-// the parameters of hk_rollout_record (and of hk_rollout_threshold before its threshold)
-StepParams record_params(const void* state_in, void* state_out, const int32_t* host_action_t, const int32_t* axis_t,
-                         float* obs_t, int32_t agent_obs, int32_t* host_mask_t, int32_t* axis_played_t, uint8_t* done_t,
-                         float* reward_t, int32_t* done_count, int32_t* length, long long B, int N, int d, int T,
-                         uint32_t ops, uint32_t flags, float padding_value, uint64_t seed, int32_t step_offset) {
+// the parameters of the one-launch rollouts (hk_rollout, hk_rollout_seeded, hk_rollout_record, and hk_rollout_threshold
+// before its threshold).  Without a random player the seed and step offset are 0; the streams of a random player are
+// dropped (run() drops them for every fixed or random player).
+StepParams rollout_params(const void* state_in, void* state_out, const int32_t* host_action_t, const int32_t* axis_t,
+                          float* obs_t, int32_t agent_obs, int32_t* host_mask_t, int32_t* axis_played_t, uint8_t* done_t,
+                          float* reward_t, int32_t* done_count, int32_t* length, long long B, int N, int d, int T,
+                          uint32_t ops, uint32_t flags, float padding_value, uint64_t seed, int32_t step_offset) {
     const bool random = flags & (HK_F_HOST_RANDOM | HK_F_AGENT_RANDOM);
     StepParams p = make_params(state_in, state_out, B, N, d, padding_value);
     p.host_action = (flags & HK_F_HOST_RANDOM) ? nullptr : host_action_t;
@@ -381,16 +386,8 @@ int hk_rollout(const void* state_in, void* state_out, const int32_t* host_action
                int32_t d, int32_t T, int32_t dtype, uint32_t ops, uint32_t flags, float padding_value,
                void* stream) {
     if (T < 1) return HK_ERR_BAD_ARG;
-    StepParams p = make_params(state_in, state_out, B, N, d, padding_value);
-    p.host_action = host_action_t;
-    p.axis = axis_t;
-    p.done = done_t;
-    p.reward = reward_t;
-    p.done_count = done_count;
-    p.length = length;
-    p.T = T;
-    p.ops = ops;
-    p.flags = flags;
+    StepParams p = rollout_params(state_in, state_out, host_action_t, axis_t, nullptr, 0, nullptr, nullptr, done_t, reward_t,
+                                  done_count, length, B, N, d, T, ops, flags, padding_value, 0, 0);
     return run(p, dtype, g_force_generic.load(), (cudaStream_t)stream);
 }
 
@@ -399,18 +396,8 @@ int hk_rollout_seeded(const void* state_in, void* state_out, const int32_t* host
                       int32_t d, int32_t T, int32_t dtype, uint32_t ops, uint32_t flags, float padding_value,
                       uint64_t seed, int32_t step_offset, void* stream) {
     if (T < 1 || !(flags & (HK_F_HOST_RANDOM | HK_F_AGENT_RANDOM))) return HK_ERR_BAD_ARG;
-    StepParams p = make_params(state_in, state_out, B, N, d, padding_value);
-    p.host_action = (flags & HK_F_HOST_RANDOM) ? nullptr : host_action_t;
-    p.axis = (flags & HK_F_AGENT_RANDOM) ? nullptr : axis_t;
-    p.done = done_t;
-    p.reward = reward_t;
-    p.done_count = done_count;
-    p.length = length;
-    p.T = T;
-    p.ops = ops;
-    p.flags = flags;
-    p.seed = seed;
-    p.step_offset = step_offset;
+    StepParams p = rollout_params(state_in, state_out, host_action_t, axis_t, nullptr, 0, nullptr, nullptr, done_t, reward_t,
+                                  done_count, length, B, N, d, T, ops, flags, padding_value, seed, step_offset);
     return run(p, dtype, g_force_generic.load(), (cudaStream_t)stream);
 }
 
@@ -420,9 +407,9 @@ int hk_rollout_record(const void* state_in, void* state_out, const int32_t* host
                       int32_t dtype, uint32_t ops, uint32_t flags, float padding_value, uint64_t seed, int32_t step_offset,
                       void* stream) {
     if (T < 1 || (agent_obs && !obs_t)) return HK_ERR_BAD_ARG;
-    StepParams p = record_params(state_in, state_out, host_action_t, axis_t, obs_t, agent_obs, host_mask_t, axis_played_t,
-                                 done_t, reward_t, done_count, length, B, N, d, T, ops, flags, padding_value, seed,
-                                 step_offset);
+    StepParams p = rollout_params(state_in, state_out, host_action_t, axis_t, obs_t, agent_obs, host_mask_t, axis_played_t,
+                                  done_t, reward_t, done_count, length, B, N, d, T, ops, flags, padding_value, seed,
+                                  step_offset);
     return run(p, dtype, g_force_generic.load(), (cudaStream_t)stream);
 }
 
@@ -435,9 +422,9 @@ int hk_rollout_threshold(const void* state_in, void* state_out, const int32_t* h
     const bool never = value_threshold == INFINITY;
     // int32 state: inputs below the threshold give shift sums below 2^30, the range in which the kernels are exact
     if (dtype == HK_DTYPE_I32 && !never && d >= 1 && (double)value_threshold > (double)((1 << 30) / d)) return HK_ERR_BAD_ARG;
-    StepParams p = record_params(state_in, state_out, host_action_t, axis_t, obs_t, agent_obs, host_mask_t, axis_played_t,
-                                 done_t, reward_t, done_count, length, B, N, d, T, ops, flags, padding_value, seed,
-                                 step_offset);
+    StepParams p = rollout_params(state_in, state_out, host_action_t, axis_t, obs_t, agent_obs, host_mask_t, axis_played_t,
+                                  done_t, reward_t, done_count, length, B, N, d, T, ops, flags, padding_value, seed,
+                                  step_offset);
     // without over_step and without a stop (+inf stops nothing) the call is the recorded rollout as it is
     p.threshold = value_threshold;
     p.over_step = over_step;

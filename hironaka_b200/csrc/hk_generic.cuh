@@ -119,24 +119,29 @@ __device__ __forceinline__ void generic_features(const T* x, uint32_t mylive, fl
     }
 }
 
-// smem per warp: DEPTH + 1 state buffers x[DEPTH + 1][Wpad] (the games up to DEPTH iterations ahead are in
-// flight while the current one is processed), then (OBS) f[Wpad] floats, then lmw[ceil(N/32)] (padded to
-// 4 words), then the compact list of live rows, (N + 1) * generic_compact_stride(D) words
+// smem per warp: two state buffers x[2][Wpad] (the next game is in flight while the current one is processed), then
+// (OBS) f[Wpad] floats, then lmw[ceil(N/32)] (padded to 4 words), then the compact list of live rows,
+// (N + 1) * generic_compact_stride(D) words
 // RT = rows per lane known at compile time (1: N <= 32, 2: N <= 64; the r-loops unroll and their
 // guards become predication) or 0 for any N (run-time loops).
-// CENSUS: the instantiation that serves hk_step_census (plain in-place single steps); it is separate so that
-// the census bookkeeping costs the other calls nothing (the kernel is bound by instruction issue).
-// REC: recorded rollouts (hk_rollout_record, with OBS for the feature buffer): every game takes the padded route,
-// whose step loop writes the features of the state before each step to row st of p.obs_t and the played actions after
-// the shift.
-// THR: rollouts with a value threshold (hk_rollout_threshold, recorded with REC): the crossing step of every game, from
+// V (GenericVariant):
+// CENSUS (Census, CensusHot): the instantiations that serve hk_step_census (plain in-place single steps); they are
+// separate so that the census bookkeeping costs the other calls nothing (the kernel is bound by instruction issue).
+// REC (Rec, ThrRec): recorded rollouts (hk_rollout_record, with OBS for the feature buffer): every game takes the padded
+// route, whose step loop writes the features of the state before each step to row st of p.obs_t and the played actions
+// after the shift.
+// THR (Thr, ThrRec): rollouts with a value threshold (hk_rollout_threshold): the crossing step of every game, from
 // its live entries on entry and after every step (one vote over the rows the warp holds), goes to p.over_step; with
 // p.stop_at_threshold a game that has crossed sits out the later steps of both routes and writes its per-step outputs
 // as an ended game that does not change: its done flag again, no reward, (REC) no action.
-template <typename T, int D, bool OBS, int RT, int DEPTH, bool HOT, bool CENSUS = false, bool REC = false, bool THR = false>
+template <typename T, int D, int RT, GenericVariant V>
 __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(const StepParams p, int warps_per_cta, int slot_words) {
-    constexpr int NBUF = DEPTH + 1;
-    // HOT: the plain random-play step (shift + reposition + newton, discrete host ids, int32 action arrays,
+    // (static: plain constexpr locals are captured by the [&] lambdas below, which changes the code the compiler emits)
+    static constexpr bool OBS = is_obs(V), HOT = is_hot(V), CENSUS = is_census(V), REC = is_rec(V), THR = is_thr(V);
+    // One game ahead in flight per warp.  Three ahead (four buffers) measured slower at C5 (0.232 vs 0.224 ms per step,
+    // tail 0.148 vs 0.138): the kernel is bound by instruction issue, not by the latency of its loads.
+    constexpr int NBUF = 2;
+    // HOT (Hot, CensusHot): the plain random-play step (shift + reposition + newton, discrete host ids, int32 action arrays,
     // one step, no observation) with its op and flag words known at compile time, so that the dozens of
     // run-time tests of them fold away; every other call takes the general instantiation.
     const uint32_t kops = HOT ? GENERIC_HOT_OPS : p.ops;
@@ -204,7 +209,6 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
     // The warp visits game gw + it * nw at iteration `it`.  Census bytes are held 32 iterations at a time (lane l:
     // iteration cbase + l; two batches, so the look-ahead never waits on a load); a ballot turns a batch into a
     // mask of the games to PLAY, and the loop jumps from one set bit to the next: a skipped game costs nothing.
-    static_assert(DEPTH == 1, "one game ahead");
     const bool use_census = CENSUS && (p.census != nullptr);
     const bool frozen_rest = (kflags & HK_F_FREEZE_ENDED) && !(kops & (HK_OP_REPOSITION | HK_OP_RESCALE));
     const uint32_t rows_k = CENSUS ? (uint32_t)p.rows_k : 0u;
@@ -302,7 +306,7 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
         if ((kops & HK_OP_SHIFT) && g_nx >= 0) {
             load_actions(p, kflags, g_nx, 0, ha_nx, ax_nx);
         }
-        cp_async_wait<DEPTH>();  // everything but the newest DEPTH groups has landed: game g is in buffer b
+        cp_async_wait<1>();  // everything but the newest group has landed: game g is in buffer b
         __syncwarp();
         T* x = reinterpret_cast<T*>(slot + b * Wpad);
 

@@ -1,5 +1,5 @@
-// warp-per-game kernel, float state, recorded rollouts (hk_rollout_record)
+// warp-per-game kernel, float state: recorded rollouts (hk_rollout_record)
 #include "hk_generic_launch.inl"
 namespace hk {
-int launch_generic_f32_rec(const StepParams& p, int dev, cudaStream_t stream) { return dispatch_generic_record<float>(p, dev, stream); }
+template int dispatch_generic<float, GenericVariant::Rec>(const StepParams&, int, cudaStream_t);
 }  // namespace hk

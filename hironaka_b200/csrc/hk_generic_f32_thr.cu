@@ -1,5 +1,6 @@
-// warp-per-game kernel, float state, rollouts with a value threshold (hk_rollout_threshold)
+// warp-per-game kernel, float state: rollouts with a value threshold, plain and recorded (hk_rollout_threshold)
 #include "hk_generic_launch.inl"
 namespace hk {
-int launch_generic_f32_thr(const StepParams& p, bool rec, int dev, cudaStream_t stream) { return dispatch_generic_threshold<float>(p, rec, dev, stream); }
+template int dispatch_generic<float, GenericVariant::Thr>(const StepParams&, int, cudaStream_t);
+template int dispatch_generic<float, GenericVariant::ThrRec>(const StepParams&, int, cudaStream_t);
 }  // namespace hk

@@ -1,7 +1,7 @@
 // hk_launch.cuh — launch helpers shared by the translation units of the library, and the
-// per-dtype launcher functions each unit defines.  The kernels are split over several .cu files
-// (hk_small_*.cu, hk_generic_*.cu) only so that they compile in parallel; hk_capi.cu holds the
-// extern "C" boundary and dispatches to these launchers.
+// launchers each unit defines.  The kernels are split over several .cu files (hk_small_*.cu,
+// hk_generic_*.cu) only so that they compile in parallel; hk_capi.cu holds the extern "C" boundary
+// and dispatches to these launchers.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -47,9 +47,32 @@ int kernel_ctas_per_sm(K kernel, KernelFacts& facts, int dev, int threads, size_
 
 inline bool is_small_shape(int N, int d) { return d == 3 && (N == 20 || N == 10 || N == 5); }
 
-// thread-per-game family (hk_small.cuh); `obs` selects the instantiation that builds features
-int launch_small_i32(const StepParams& p, bool obs, int dev, cudaStream_t stream);
-int launch_small_f32(const StepParams& p, bool obs, int dev, cudaStream_t stream);
+// one-launch paths of the two kernel families, one instantiation per (dtype, variant) in the hk_small_*.cu and
+// hk_generic_*.cu units (hk_small_launch.inl, hk_generic_launch.inl)
+template <typename T, SmallVariant V>
+int dispatch_small(const StepParams& p, int dev, cudaStream_t stream);  // thread-per-game (hk_small.cuh)
+template <typename T, GenericVariant V>
+int dispatch_generic(const StepParams& p, int dev, cudaStream_t stream);  // warp-per-game (hk_generic.cuh)
+extern template int dispatch_small<int32_t, SmallVariant::Step>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_small<int32_t, SmallVariant::Obs>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_small<int32_t, SmallVariant::Rec>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_small<int32_t, SmallVariant::Thr>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_small<int32_t, SmallVariant::ThrRec>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_small<float, SmallVariant::Step>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_small<float, SmallVariant::Obs>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_small<float, SmallVariant::Rec>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_small<float, SmallVariant::Thr>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_small<float, SmallVariant::ThrRec>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_generic<int32_t, GenericVariant::Plain>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_generic<int32_t, GenericVariant::Obs>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_generic<int32_t, GenericVariant::Rec>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_generic<int32_t, GenericVariant::Thr>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_generic<int32_t, GenericVariant::ThrRec>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_generic<float, GenericVariant::Plain>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_generic<float, GenericVariant::Obs>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_generic<float, GenericVariant::Rec>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_generic<float, GenericVariant::Thr>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_generic<float, GenericVariant::ThrRec>(const StepParams&, int, cudaStream_t);
 // census-scheduled thread-per-game kernel (hk_sched.cuh): in-place single steps with p.census
 int launch_sched_i32(const StepParams& p, int dev, cudaStream_t stream);
 int launch_sched_f32(const StepParams& p, int dev, cudaStream_t stream);
@@ -60,18 +83,5 @@ int launch_rows_i32(const StepParams& p, int dev, cudaStream_t stream);
 int launch_rows_f32(const StepParams& p, int dev, cudaStream_t stream);
 constexpr int ROWS_K = 8;  // = ROWS_MAX_K of hk_rows.cuh
 inline bool rows_shape(int N, int d) { return N <= 64 && d >= 2 && d <= 5; }
-// warp-per-game family (hk_generic.cuh)
-int launch_generic_i32(const StepParams& p, bool obs, int dev, cudaStream_t stream);
-int launch_generic_f32(const StepParams& p, bool obs, int dev, cudaStream_t stream);
-// recorded rollouts (hk_rollout_record), instantiations of their own in both families
-int launch_small_i32_rec(const StepParams& p, int dev, cudaStream_t stream);
-int launch_small_f32_rec(const StepParams& p, int dev, cudaStream_t stream);
-int launch_generic_i32_rec(const StepParams& p, int dev, cudaStream_t stream);
-int launch_generic_f32_rec(const StepParams& p, int dev, cudaStream_t stream);
-// rollouts with a value threshold (hk_rollout_threshold), recorded (`rec`) or not, instantiations of their own in both families
-int launch_small_i32_thr(const StepParams& p, bool rec, int dev, cudaStream_t stream);
-int launch_small_f32_thr(const StepParams& p, bool rec, int dev, cudaStream_t stream);
-int launch_generic_i32_thr(const StepParams& p, bool rec, int dev, cudaStream_t stream);
-int launch_generic_f32_thr(const StepParams& p, bool rec, int dev, cudaStream_t stream);
 
 }  // namespace hk

@@ -1333,13 +1333,17 @@ __device__ __forceinline__ void warp_copy_words(uint32_t* dst, const uint32_t* s
     for (int w = lane; w < words; w += 32) dst[w] = src[w];
 }
 
+// The thread-per-game kernel: warp-private rings of STAGES tiles of 32 games, WARPS warps per CTA, one persistent wave.
 // PACKED = false: the instantiation of the one-launch rollouts (p.T > 1), which never take the packed tiers and are bound
 // by instruction fetch: they do not carry that code.
-// REC: recorded rollouts (hk_small_record_kernel): before every step the features of the state go to the warp's obs
-// tile, after it the played actions are written and the tile leaves with one bulk store into row st of p.obs_t.
-// THR: rollouts with a value threshold (hk_small_threshold_kernel), recorded (REC) or not; p.over_step leaves with length.
-template <typename T, int N, int D, bool OBS, bool POLICY, int WARPS, int STAGES, bool PACKED, bool REC, bool THR = false>
+// V (SmallVariant): Obs builds the features of the final state into the warp's obs tile.  Rec (recorded rollouts):
+// before every step the features of the state go to the warp's obs tile, after it the played actions are written and
+// the tile leaves with one bulk store into row st of p.obs_t.  Thr, ThrRec: rollouts with a value threshold, recorded or
+// not; p.over_step leaves with length.
+template <typename T, int N, int D, bool POLICY, int WARPS, int STAGES, bool PACKED, SmallVariant V>
 __device__ __forceinline__ void small_kernel_body(const StepParams& p) {
+    // (static: plain constexpr locals are captured by the [&] lambdas below, which changes the code the compiler emits)
+    static constexpr bool OBS = is_obs(V), REC = is_rec(V), THR = is_thr(V);
     using L = SmallLayout<N, D, OBS || REC, WARPS, STAGES>;
     constexpr int SMALL_WARPS = WARPS;
     constexpr int SMALL_STAGES = STAGES;
@@ -1613,22 +1617,9 @@ __device__ __forceinline__ void small_kernel_body(const StepParams& p) {
     if (lane == 0) bulk_wait_all<0>();  // all bulk stores globally complete before the warp retires
 }
 
-template <typename T, int N, int D, bool OBS, bool POLICY, int WARPS, int STAGES, bool PACKED = true>
+template <typename T, int N, int D, bool POLICY, int WARPS, int STAGES, bool PACKED, SmallVariant V>
 __global__ void __launch_bounds__(WARPS * 32) hk_small_kernel(const StepParams p) {
-    small_kernel_body<T, N, D, OBS, POLICY, WARPS, STAGES, PACKED, false>(p);
-}
-
-// hk_rollout_record on the thread-per-game shapes: the rollout kernel's tile loop with the recorder, one stage per warp
-template <typename T, int N, int D, bool POLICY, int WARPS>
-__global__ void __launch_bounds__(WARPS * 32) hk_small_record_kernel(const StepParams p) {
-    small_kernel_body<T, N, D, false, POLICY, WARPS, 1, false, true>(p);
-}
-
-// hk_rollout_threshold on the thread-per-game shapes: the rollout kernel's tile loop (REC: the recorded rollout's) with
-// the crossing step of every game and the stop, one stage per warp
-template <typename T, int N, int D, bool POLICY, int WARPS, bool REC>
-__global__ void __launch_bounds__(WARPS * 32) hk_small_threshold_kernel(const StepParams p) {
-    small_kernel_body<T, N, D, false, POLICY, WARPS, 1, false, REC, true>(p);
+    small_kernel_body<T, N, D, POLICY, WARPS, STAGES, PACKED, V>(p);
 }
 
 }  // namespace hk

@@ -1,5 +1,5 @@
-// thread-per-game kernel, float state, instantiations WITH observation features
+// thread-per-game kernel, float state: steps with observation features
 #include "hk_small_launch.inl"
 namespace hk {
-int launch_small_f32_obs(const StepParams& p, int dev, cudaStream_t stream) { return dispatch_small<float, true>(p, dev, stream); }
+template int dispatch_small<float, SmallVariant::Obs>(const StepParams&, int, cudaStream_t);
 }  // namespace hk

@@ -1,5 +1,5 @@
-// thread-per-game kernel, float state, instantiations WITHOUT observation features
+// thread-per-game kernel, float state: steps and rollouts
 #include "hk_small_launch.inl"
 namespace hk {
-int launch_small_f32_noobs(const StepParams& p, int dev, cudaStream_t stream) { return dispatch_small<float, false>(p, dev, stream); }
+template int dispatch_small<float, SmallVariant::Step>(const StepParams&, int, cudaStream_t);
 }  // namespace hk

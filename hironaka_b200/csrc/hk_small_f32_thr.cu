@@ -1,5 +1,6 @@
-// thread-per-game kernel, float state, rollouts with a value threshold (hk_rollout_threshold)
+// thread-per-game kernel, float state: rollouts with a value threshold, plain and recorded (hk_rollout_threshold)
 #include "hk_small_launch.inl"
 namespace hk {
-int launch_small_f32_thr(const StepParams& p, bool rec, int dev, cudaStream_t stream) { return dispatch_small_threshold<float>(p, rec, dev, stream); }
+template int dispatch_small<float, SmallVariant::Thr>(const StepParams&, int, cudaStream_t);
+template int dispatch_small<float, SmallVariant::ThrRec>(const StepParams&, int, cudaStream_t);
 }  // namespace hk

@@ -1,5 +1,5 @@
-// thread-per-game kernel, int32 state, recorded rollouts (hk_rollout_record)
+// thread-per-game kernel, int32 state: recorded rollouts (hk_rollout_record)
 #include "hk_small_launch.inl"
 namespace hk {
-int launch_small_i32_rec(const StepParams& p, int dev, cudaStream_t stream) { return dispatch_small_record<int32_t>(p, dev, stream); }
+template int dispatch_small<int32_t, SmallVariant::Rec>(const StepParams&, int, cudaStream_t);
 }  // namespace hk

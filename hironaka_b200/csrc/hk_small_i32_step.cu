@@ -1,5 +1,5 @@
-// thread-per-game kernel, int32_t state, instantiations WITHOUT observation features
+// thread-per-game kernel, int32 state: steps and rollouts
 #include "hk_small_launch.inl"
 namespace hk {
-int launch_small_i32_noobs(const StepParams& p, int dev, cudaStream_t stream) { return dispatch_small<int32_t, false>(p, dev, stream); }
+template int dispatch_small<int32_t, SmallVariant::Step>(const StepParams&, int, cudaStream_t);
 }  // namespace hk

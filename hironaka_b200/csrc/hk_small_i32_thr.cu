@@ -1,5 +1,6 @@
-// thread-per-game kernel, int32 state, rollouts with a value threshold (hk_rollout_threshold)
+// thread-per-game kernel, int32 state: rollouts with a value threshold, plain and recorded (hk_rollout_threshold)
 #include "hk_small_launch.inl"
 namespace hk {
-int launch_small_i32_thr(const StepParams& p, bool rec, int dev, cudaStream_t stream) { return dispatch_small_threshold<int32_t>(p, rec, dev, stream); }
+template int dispatch_small<int32_t, SmallVariant::Thr>(const StepParams&, int, cudaStream_t);
+template int dispatch_small<int32_t, SmallVariant::ThrRec>(const StepParams&, int, cudaStream_t);
 }  // namespace hk

@@ -185,9 +185,8 @@ def rollout(state: torch.Tensor, host_actions: Optional[torch.Tensor], axes: Opt
     `steps` gives T if both are None.  With `value_threshold` the rollout runs through hk_rollout_threshold:
     `over_step` (int32 [B], written when given) receives each game's crossing step, and `stop_at_threshold` stops
     the games that cross."""
-    dt = _require_state(state)
-    B, N, d = state.shape
-    dev = state.device
+    _require_state(state)
+    B = state.shape[0]
     host_fixed = flags & (C.HK_F_HOST_ALL_COORD | C.HK_F_HOST_ZEILLINGER)
     agent_fixed = flags & (C.HK_F_AGENT_FIRST | C.HK_F_AGENT_LAST)
     if (host_actions is None and not host_fixed) or (axes is None and not agent_fixed):
@@ -201,23 +200,11 @@ def rollout(state: torch.Tensor, host_actions: Optional[torch.Tensor], axes: Opt
         if not steps:
             raise ValueError("steps is required when both players are fixed")
         T = int(steps)
-    ha = None if host_fixed else host_actions.to(device=dev, dtype=torch.int32).contiguous()
-    ax = None if agent_fixed else axes.to(device=dev, dtype=torch.int32).contiguous()
-    dst = state if inplace else torch.empty_like(state)
-    done = torch.empty((T, B), dtype=torch.uint8, device=dev) if want_done else None
-    reward = torch.empty((T, B), dtype=torch.float32, device=dev) if want_reward else None
-    dcount = torch.zeros(T, dtype=torch.int32, device=dev) if want_done_count else None
-    length = torch.empty(B, dtype=torch.int32, device=dev) if want_length else None
-    if value_threshold is not None:
-        _rollout_threshold(state, dst, ha, ax, None, False, None, None, done, reward, dcount, length, T, dt, ops, flags,
-                           padding_value, 0, 0, value_threshold, stop_at_threshold, over_step)
-        return dst, (None if done is None else done.view(torch.bool)), reward, dcount, length
-    with torch.cuda.device(dev):
-        stream = torch.cuda.current_stream(dev).cuda_stream
-        rc = lib().hk_rollout(_ptr(state), _ptr(dst), _ptr(ha), _ptr(ax), _ptr(done), _ptr(reward), _ptr(dcount),
-                              _ptr(length), B, N, d, T, dt, ops, flags, float(padding_value), stream)
-    check(rc, "hk_rollout")
-    return dst, (None if done is None else done.view(torch.bool)), reward, dcount, length
+    tr = _rollout(state, None if host_fixed else host_actions, None if agent_fixed else axes, T, "hk_rollout", ops=ops,
+                  flags=flags, padding_value=padding_value, inplace=inplace, want_done=want_done, want_reward=want_reward,
+                  want_done_count=want_done_count, want_length=want_length, value_threshold=value_threshold,
+                  stop_at_threshold=stop_at_threshold, over_step=over_step)
+    return tr.state, tr.done, tr.reward, tr.done_count, tr.length
 
 
 def rollout_random(state: torch.Tensor, steps: int, seed: int, *, ops: int, flags: int = 0, host_actions=None, axes=None,
@@ -228,48 +215,14 @@ def rollout_random(state: torch.Tensor, steps: int, seed: int, *, ops: int, flag
     `flags` carries HK_F_HOST_RANDOM and / or HK_F_AGENT_RANDOM; the other player comes from its [T, B] stream or a
     fixed-player flag.  Philox4x32-10 keyed by `seed`, counter (game, step_offset + t): see `random_actions`.
     `value_threshold`, `stop_at_threshold`, `over_step`: as in `rollout` (hk_rollout_threshold)."""
-    dt = _require_state(state)
-    B, N, d = state.shape
-    dev = state.device
-    T = int(steps)
-    ha = None if host_actions is None else host_actions.to(device=dev, dtype=torch.int32).contiguous()
-    ax = None if axes is None else axes.to(device=dev, dtype=torch.int32).contiguous()
-    dst = state if inplace else torch.empty_like(state)
-    done = torch.empty((T, B), dtype=torch.uint8, device=dev) if want_done else None
-    reward = torch.empty((T, B), dtype=torch.float32, device=dev) if want_reward else None
-    dcount = torch.zeros(T, dtype=torch.int32, device=dev)
-    length = torch.empty(B, dtype=torch.int32, device=dev) if want_length else None
-    if value_threshold is not None:
-        if not flags & (C.HK_F_HOST_RANDOM | C.HK_F_AGENT_RANDOM):
-            raise ValueError("rollout_random needs HK_F_HOST_RANDOM and / or HK_F_AGENT_RANDOM")
-        _rollout_threshold(state, dst, ha, ax, None, False, None, None, done, reward, dcount, length, T, dt, ops, flags,
-                           padding_value, seed, step_offset, value_threshold, stop_at_threshold, over_step)
-        return dst, (None if done is None else done.view(torch.bool)), reward, dcount, length
-    with torch.cuda.device(dev):
-        stream = torch.cuda.current_stream(dev).cuda_stream
-        rc = lib().hk_rollout_seeded(_ptr(state), _ptr(dst), _ptr(ha), _ptr(ax), _ptr(done), _ptr(reward), _ptr(dcount),
-                                     _ptr(length), B, N, d, T, dt, ops, flags, float(padding_value), int(seed) & (2 ** 64 - 1),
-                                     int(step_offset), stream)
-    check(rc, "hk_rollout_seeded")
-    return dst, (None if done is None else done.view(torch.bool)), reward, dcount, length
-
-
-def _rollout_threshold(state, dst, ha, ax, obs, agent_obs, hmask, axis, done, reward, dcount, length, T, dt, ops, flags,
-                       padding_value, seed, step_offset, value_threshold, stop_at_threshold, over_step):
-    """hk_rollout_threshold on buffers the public entry points have prepared; `over_step` is the caller's int32 [B]."""
-    B, N, d = state.shape
-    dev = state.device
-    if over_step is not None and (over_step.dtype != torch.int32 or tuple(over_step.shape) != (B,) or
-                                  over_step.device != dev or not over_step.is_contiguous()):
-        raise ValueError("over_step must be a contiguous int32 [B] tensor on the state's device")
-    with torch.cuda.device(dev):
-        stream = torch.cuda.current_stream(dev).cuda_stream
-        rc = lib().hk_rollout_threshold(_ptr(state), _ptr(dst), _ptr(ha), _ptr(ax), _ptr(obs), 1 if agent_obs else 0,
-                                        _ptr(hmask), _ptr(axis), _ptr(done), _ptr(reward), _ptr(dcount), _ptr(length), B, N,
-                                        d, T, dt, ops, flags, float(padding_value), int(seed) & (2 ** 64 - 1),
-                                        int(step_offset), float(value_threshold), 1 if stop_at_threshold else 0,
-                                        _ptr(over_step), stream)
-    check(rc, "hk_rollout_threshold")
+    _require_state(state)
+    if value_threshold is not None and not flags & (C.HK_F_HOST_RANDOM | C.HK_F_AGENT_RANDOM):
+        raise ValueError("rollout_random needs HK_F_HOST_RANDOM and / or HK_F_AGENT_RANDOM")
+    tr = _rollout(state, host_actions, axes, int(steps), "hk_rollout_seeded", ops=ops, flags=flags,
+                  padding_value=padding_value, inplace=inplace, want_done=want_done, want_reward=want_reward,
+                  want_length=want_length, seed=seed, step_offset=step_offset, value_threshold=value_threshold,
+                  stop_at_threshold=stop_at_threshold, over_step=over_step)
+    return tr.state, tr.done, tr.reward, tr.done_count, tr.length
 
 
 class Trajectory(NamedTuple):
@@ -297,9 +250,8 @@ def rollout_record(state: torch.Tensor, steps: Optional[int] = None, host_action
     and `step_offset`); `steps` gives T when no stream does.  The features after the last step are
     features(trajectory.state).  `value_threshold`, `stop_at_threshold`, `over_step`: as in `rollout`
     (hk_rollout_threshold); a stopped game records the features of its frozen state, host_mask 0 and axis -1."""
-    dt = _require_state(state)
-    B, N, d = state.shape
-    dev = state.device
+    _require_state(state)
+    B = state.shape[0]
     streams = [t for t in (host_actions, axes) if t is not None]
     if any(t.dim() != 2 or t.shape[1] != B for t in streams) or len({tuple(t.shape) for t in streams}) > 1:
         raise ValueError("host_actions and axes must be [T, B]")
@@ -308,6 +260,21 @@ def rollout_record(state: torch.Tensor, steps: Optional[int] = None, host_action
         raise ValueError("steps must be >= 1 and match the action streams")
     if agent_obs and not want_obs:
         raise ValueError("agent_obs needs want_obs")
+    return _rollout(state, host_actions, axes, T, "hk_rollout_record", ops=ops, flags=flags, padding_value=padding_value,
+                    inplace=inplace, want_done=want_done, want_reward=want_reward, want_length=want_length, seed=seed,
+                    step_offset=step_offset, want_obs=want_obs, agent_obs=agent_obs, want_actions=want_actions,
+                    value_threshold=value_threshold, stop_at_threshold=stop_at_threshold, over_step=over_step)
+
+
+def _rollout(state, host_actions, axes, T, entry, *, ops, flags, padding_value, inplace, want_done, want_reward,
+             want_length, want_done_count=True, seed=0, step_offset=0, want_obs=False, agent_obs=False,
+             want_actions=False, value_threshold=None, stop_at_threshold=False, over_step=None) -> Trajectory:
+    """A one-launch rollout of T steps on the players' [T, B] streams (None: no stream): allocates the outputs the
+    caller wants and launches `entry` (hk_rollout, hk_rollout_seeded or hk_rollout_record), or hk_rollout_threshold
+    when `value_threshold` is given; `over_step` is the caller's int32 [B]."""
+    dt = _DT[state.dtype]
+    B, N, d = state.shape
+    dev = state.device
     ha = None if host_actions is None else host_actions.to(device=dev, dtype=torch.int32).contiguous()
     ax = None if axes is None else axes.to(device=dev, dtype=torch.int32).contiguous()
     dst = state if inplace else torch.empty_like(state)
@@ -316,18 +283,33 @@ def rollout_record(state: torch.Tensor, steps: Optional[int] = None, host_action
     axis = torch.empty((T, B), dtype=torch.int32, device=dev) if want_actions else None
     done = torch.empty((T, B), dtype=torch.uint8, device=dev) if want_done else None
     reward = torch.empty((T, B), dtype=torch.float32, device=dev) if want_reward else None
-    dcount = torch.zeros(T, dtype=torch.int32, device=dev)
+    dcount = torch.zeros(T, dtype=torch.int32, device=dev) if want_done_count else None
     length = torch.empty(B, dtype=torch.int32, device=dev) if want_length else None
     if value_threshold is not None:
-        _rollout_threshold(state, dst, ha, ax, obs, agent_obs, hmask, axis, done, reward, dcount, length, T, dt, ops, flags,
-                           padding_value, seed, step_offset, value_threshold, stop_at_threshold, over_step)
-        return Trajectory(dst, obs, hmask, axis, None if done is None else done.view(torch.bool), reward, dcount, length)
+        entry = "hk_rollout_threshold"
+        if over_step is not None and (over_step.dtype != torch.int32 or tuple(over_step.shape) != (B,) or
+                                      over_step.device != dev or not over_step.is_contiguous()):
+            raise ValueError("over_step must be a contiguous int32 [B] tensor on the state's device")
+    seed = int(seed) & (2 ** 64 - 1)
+    pad = float(padding_value)
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream(dev).cuda_stream
-        rc = lib().hk_rollout_record(_ptr(state), _ptr(dst), _ptr(ha), _ptr(ax), _ptr(obs), 1 if agent_obs else 0, _ptr(hmask),
-                                     _ptr(axis), _ptr(done), _ptr(reward), _ptr(dcount), _ptr(length), B, N, d, T, dt, ops,
-                                     flags, float(padding_value), int(seed) & (2 ** 64 - 1), int(step_offset), stream)
-    check(rc, "hk_rollout_record")
+        if entry == "hk_rollout_threshold":
+            rc = lib().hk_rollout_threshold(_ptr(state), _ptr(dst), _ptr(ha), _ptr(ax), _ptr(obs), 1 if agent_obs else 0,
+                                            _ptr(hmask), _ptr(axis), _ptr(done), _ptr(reward), _ptr(dcount), _ptr(length), B,
+                                            N, d, T, dt, ops, flags, pad, seed, int(step_offset), float(value_threshold),
+                                            1 if stop_at_threshold else 0, _ptr(over_step), stream)
+        elif entry == "hk_rollout_record":
+            rc = lib().hk_rollout_record(_ptr(state), _ptr(dst), _ptr(ha), _ptr(ax), _ptr(obs), 1 if agent_obs else 0,
+                                         _ptr(hmask), _ptr(axis), _ptr(done), _ptr(reward), _ptr(dcount), _ptr(length), B, N,
+                                         d, T, dt, ops, flags, pad, seed, int(step_offset), stream)
+        elif entry == "hk_rollout_seeded":
+            rc = lib().hk_rollout_seeded(_ptr(state), _ptr(dst), _ptr(ha), _ptr(ax), _ptr(done), _ptr(reward), _ptr(dcount),
+                                         _ptr(length), B, N, d, T, dt, ops, flags, pad, seed, int(step_offset), stream)
+        else:
+            rc = lib().hk_rollout(_ptr(state), _ptr(dst), _ptr(ha), _ptr(ax), _ptr(done), _ptr(reward), _ptr(dcount),
+                                  _ptr(length), B, N, d, T, dt, ops, flags, pad, stream)
+    check(rc, entry)
     return Trajectory(dst, obs, hmask, axis, None if done is None else done.view(torch.bool), reward, dcount, length)
 
 

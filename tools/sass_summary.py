@@ -1,13 +1,36 @@
 """Per-kernel SASS extract of the built library: instruction count, code size and the mnemonics that show how data
 moves (UBLKCP = cp.async.bulk / TMA bulk copy, SYNCS = mbarrier, LDGSTS = cp.async, REDUX = warp reduce, ATOM/RED).
-    python tools/sass_summary.py [lib.so] > profiles/r2_sass_summary.txt"""
+    python tools/sass_summary.py [lib.so] > profiles/r2_sass_summary.txt
+    python tools/sass_summary.py --fingerprint [lib.so]
+--fingerprint prints one line per kernel: a hash of its instructions (without the function name and the addresses),
+the instruction count and the demangled name.  Two builds whose sorted hash lists are equal run the same machine code,
+whatever the kernels are called."""
 import collections
+import hashlib
 import re
 import subprocess
 import sys
 
-lib = sys.argv[1] if len(sys.argv) > 1 else "hironaka_b200/_lib/libhironaka_b200.so"
+args = [a for a in sys.argv[1:] if a != "--fingerprint"]
+lib = args[0] if args else "hironaka_b200/_lib/libhironaka_b200.so"
 out = subprocess.run(["cuobjdump", "-sass", lib], capture_output=True, text=True, check=True).stdout
+
+if "--fingerprint" in sys.argv:
+    code = []  # (mangled name, instructions) per kernel, in library order; a name that appears twice is kept twice
+    for line in out.splitlines():
+        m = re.search(r"Function : (\S+)", line)
+        if m:
+            code.append((m.group(1), []))
+            continue
+        m = re.match(r"\s+/\*[0-9a-f]{4,6}\*/\s+(.*?)\s*;", line)
+        if m and code:
+            code[-1][1].append(m.group(1))
+    demangled = subprocess.run(["c++filt"], input="\n".join(n for n, _ in code), capture_output=True,
+                               text=True).stdout.splitlines()
+    for (mangled, ins), nice in zip(code, demangled):
+        print(f"{hashlib.sha256(chr(10).join(ins).encode()).hexdigest()[:16]} {len(ins):6d} {nice}")
+    sys.exit(0)
+
 WATCH = ["UBLKCP", "SYNCS", "LDGSTS", "REDUX", "UTMALDG", "UTMASTG", "ATOMG", "RED.", "LDS", "STS", "LDG", "STG", "SHFL", "VOTE",
          "LOP3", "IADD3", "IMAD", "ISETP", "VIMNMX", "POPC", "FLO", "BAR", "MUFU"]
 kernels = collections.OrderedDict()

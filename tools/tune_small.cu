@@ -19,7 +19,7 @@ constexpr int N = 20, D = 3, T = 20;
 template <int WARPS, int STAGES, bool OBS = false>
 float launch(const hk::StepParams& p, cudaStream_t st, int sms, bool time_it, cudaEvent_t e0, cudaEvent_t e1) {
     using L = hk::SmallLayout<N, D, OBS, WARPS, STAGES>;
-    auto k = hk::hk_small_kernel<int32_t, N, D, OBS, false, WARPS, STAGES>;
+    auto k = hk::hk_small_kernel<int32_t, N, D, false, WARPS, STAGES, true, OBS ? hk::SmallVariant::Obs : hk::SmallVariant::Step>;
     static int per_sm = 0;
     if (!per_sm) {
         CK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L::SMEM_BYTES));
