@@ -28,19 +28,16 @@ constexpr int SCHED_ROUND_TILES = 32;  // tiles (of 32 games) a warp schedules t
 #define SCHED_PASS_UNROLL 2
 #endif
 constexpr int kSchedPassUnroll = SCHED_PASS_UNROLL;
-#ifndef SCHED_TILE_GROUP
-#define SCHED_TILE_GROUP 0  // 0: a warp owns one contiguous run of tiles; G > 0: runs of G tiles, dealt round-robin to the warps
-#endif
 #ifndef SCHED_DIRECT
 #define SCHED_DIRECT 1  // packed tiers release the stage after the gather and store changed rows straight to global memory
-#endif
-#ifndef SCHED_SPECULATE
-#define SCHED_SPECULATE 0  // (measured, not kept: no gain on the first steps, 3-5 % slower in the middle of a rollout) the first tile of a round is requested before the census pass has finished (see pass 1)
 #endif
 #ifndef SCHED_NATURAL_NUM
 #define SCHED_NATURAL_NUM 1  // a round is stepped tile by tile in natural order while at least NUM / DEN of
 #define SCHED_NATURAL_DEN 2  // its games are in play (tools/time_census.py)
 #endif
+// the class sort packs its counts in 10-bit fields: a sorted round has fewer games in play than games (< 1024) only
+// while the ratio is at most one (above one, rounds wholly in play would be sorted too)
+static_assert(SCHED_NATURAL_NUM <= SCHED_NATURAL_DEN, "a sorted round must have fewer than 1024 games in play");
 
 template <int N, int D, int WARPS, int STAGES, bool OBS = false>
 struct SchedLayout {
@@ -56,10 +53,43 @@ struct SchedLayout {
     static constexpr size_t SMEM_BYTES = BAR_BYTES + (size_t)WARPS * WARP_WORDS * 4;
 };
 
-__device__ __forceinline__ int census_class(uint32_t v) {
-    if (v == 0) return 6;          // unknown: counted after the load
-    if (v & 0x80u) return 1;       // ended, but not at rest under this launch's ops
-    return v <= 2 ? 1 : (v <= 4 ? 2 : (v <= 8 ? 3 : (v <= 12 ? 4 : (v <= 16 ? 5 : 6))));
+// Byte-SIMD helpers of the census pass: a 32-bit word holds the census bytes of four consecutive games.
+// bit 7 of each byte of the result: that byte of x (<= 0x7f) is >= t (t <= 0x7f; no borrow crosses a byte)
+__device__ __forceinline__ uint32_t bytes_ge7(uint32_t x7, uint32_t t) {
+    return ((x7 | 0x80808080u) - t * 0x01010101u) & 0x80808080u;
+}
+// bits 0..3: which bytes of x are non-zero
+__device__ __forceinline__ uint32_t nonzero_bytes4(uint32_t x) {
+    const uint32_t hi = (((x & 0x7f7f7f7fu) + 0x7f7f7f7fu) | x) & 0x80808080u;
+    return ((hi >> 7) * 0x01020408u) >> 24;  // bits 0, 8, 16, 24 -> 24, 25, 26, 27 (no two partial products collide)
+}
+
+// Class codes of four census bytes (the class array's format): class 0 = at rest or no such game; 1..6 = the tier
+// class of a game in play (6 for an unknown byte, 1 for "ended, not at rest under this launch's ops" and for 1-2
+// live rows, else 1 + [v > 2] + [v > 4] + [v > 8] + [v > 12] + [v > 16]); 0x80 = at rest; 0x40 = its live count.
+// vmask keeps the bytes of games that exist; rest7 returns the at-rest flags (bit 7 of each byte).
+__device__ __forceinline__ uint32_t census_codes4(uint32_t w, uint32_t vmask, bool frozen_rest, uint32_t& rest7) {
+    w &= vmask;
+    const uint32_t ended = w & 0x80808080u;
+    rest7 = ended & ((w << 6) | (frozen_rest ? 0x80808080u : 0u)) & vmask;  // ended and (bit 1 or frozen)
+    const uint32_t x7 = w & 0x7f7f7f7fu;
+    uint32_t c = 0x01010101u + (bytes_ge7(x7, 3) >> 7) + (bytes_ge7(x7, 5) >> 7) + (bytes_ge7(x7, 9) >> 7) +
+                 (bytes_ge7(x7, 13) >> 7) + (bytes_ge7(x7, 17) >> 7);
+    const uint32_t unknown = ~(bytes_ge7(x7, 1) | ended) & 0x80808080u;  // a zero byte
+    c += (unknown >> 7) * 5u;
+    const uint32_t endedff = (ended >> 7) * 0xffu;
+    c = (c & ~endedff) | (ended >> 7);
+    c &= vmask & ~((rest7 >> 7) * 0xffu);
+    return c | rest7 | ((w & 0x01010101u) << 6);
+}
+
+// Per-lane counts of the classes 1..6 of four class codes, packed in 10-bit fields: classes 1-3 in lo, 4-6 in hi.
+__device__ __forceinline__ void class_counts4(uint32_t code, uint32_t& lo, uint32_t& hi) {
+    const uint32_t x7 = code & 0x07070707u;
+    const int g1 = __popc(bytes_ge7(x7, 1)), g2 = __popc(bytes_ge7(x7, 2)), g3 = __popc(bytes_ge7(x7, 3));
+    const int g4 = __popc(bytes_ge7(x7, 4)), g5 = __popc(bytes_ge7(x7, 5)), g6 = __popc(bytes_ge7(x7, 6));
+    lo = (uint32_t)(g1 - g2) | ((uint32_t)(g2 - g3) << 10) | ((uint32_t)(g3 - g4) << 20);
+    hi = (uint32_t)(g4 - g5) | ((uint32_t)(g5 - g6) << 10) | ((uint32_t)g6 << 20);
 }
 
 // OBS: the instantiation that also builds the observation features of the new state (p.obs, sorted modes only):
@@ -107,108 +137,95 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) hk_sched_kernel(const StepPa
     const float rest_reward = (p.flags & HK_F_ROLE_AGENT) ? -0.0f : 0.0f;
     // piece lane -> (game slot within the instruction, piece within the game)
     const int sub = lane / LPG, piece = lane - sub * LPG;
-    int settled_total = 0;
+    int settled_total = 0;  // per lane: games at rest
+    // outputs of the games at rest as one vector store per lane (four games) where the pointer allows it
+    const bool done4 = p.done && ((reinterpret_cast<uintptr_t>(p.done) & 3u) == 0);
+    const bool reward16 = p.reward && aligned16(p.reward);
+    const bool npoints16 = p.num_points && aligned16(p.num_points);
 
     // A warp owns a CONTIGUOUS run of tiles (its games share DRAM pages when they are gathered one by one),
     // scheduled in rounds of SCHED_ROUND_TILES.
-#if SCHED_TILE_GROUP == 0
     const long long tpw = (ntiles + nw - 1) / nw;
     const long long t_begin = gw * tpw;
     const long long t_end = (t_begin + tpw < ntiles) ? (t_begin + tpw) : ntiles;
     auto tile_of = [&](long long j) -> long long { return t_begin + j; };  // the warp's j-th tile
-#else
-    constexpr int TG = SCHED_TILE_GROUP;
-    const long long t_end = ntiles;
-    auto tile_of = [&](long long j) -> long long { return ((j / TG) * nw + gw) * TG + (j % TG); };
-#endif
+    uint32_t* clsw = reinterpret_cast<uint32_t*>(clsb);
     for (long long j0 = 0; tile_of(j0) < t_end; j0 += SCHED_ROUND_TILES) {
         // ---- census of this round's tiles: outputs of the games at rest, class bytes of the others ----
-#if SCHED_TILE_GROUP == 0
         const int nk = (int)((t_end - t_begin - j0 < SCHED_ROUND_TILES) ? (t_end - t_begin - j0) : SCHED_ROUND_TILES);
-#else
-        int nk = 0;  // tiles of this round that exist: whole runs, then the part of the run that crosses the end
-#pragma unroll
-        for (int q = 0; q < SCHED_ROUND_TILES / TG; ++q) {
-            const long long left = t_end - tile_of(j0 + q * TG);
-            nk += (left >= TG) ? TG : (left > 0 ? (int)left : 0);
-        }
-#endif
-        uint32_t tilemask = 0, classes = 0;
-        int inplay = 0, ngames = 0;
-        bool spec = false;  // the round's first tile has been requested ahead of the schedule
-        // The round's census bytes are staged in shared memory (the class array doubles as the landing zone):
-        // cp.async in 4-byte pieces, 8 lanes per tile, all requests in flight at once, then ONE rolled loop
-        // over the tiles (an unrolled register version was 16 KB of straight-line code in a kernel whose hot
-        // loops compete for the instruction cache).
+        const int ngroups = (nk + 3) >> 2;  // groups of four tiles: lane l holds the census bytes of games 4l .. 4l+3
+        const long long first = tile_of(j0) << 5;  // the round's first game
+        const int cbytes = (int)((B - first < (long long)nk * 32) ? (B - first) : (long long)nk * 32);  // its games
+        // The round's census words are staged in the class array, one per lane and group, all requests in flight at
+        // once: cp.async where the census is 4-byte aligned, words assembled from byte loads otherwise (and for the
+        // word that crosses B).  Bytes past B read as 0.
         {
-            const uint8_t* cbase = p.census + (tile_of(j0) << 5);
-            const long long cbytes = ((B - (tile_of(j0) << 5)) < (long long)nk * 32) ? (B - (tile_of(j0) << 5)) : (long long)nk * 32;
-            if (SCHED_TILE_GROUP == 0 && ((reinterpret_cast<uintptr_t>(cbase) & 3u) == 0)) {
-                for (int o = lane * 4; o < nk * 32; o += 128) {
-                    if (o + 4 <= cbytes) cp_async_4(clsb + o, cbase + o);
-                    else {
-                        for (int q = 0; q < 4; ++q) clsb[o + q] = (o + q < cbytes) ? __ldg(cbase + o + q) : (uint8_t)0;
-                    }
-                }
-                cp_async_commit();
-                cp_async_wait<0>();
-            } else {
-                for (int k = 0; k < nk; ++k) {
-                    const long long g = (tile_of(j0 + k) << 5) + lane;
-                    clsb[k * 32 + lane] = (g < B) ? __ldg(p.census + g) : (uint8_t)0;
+            const uint8_t* cbase = p.census + first;
+            const bool caligned = (reinterpret_cast<uintptr_t>(cbase) & 3u) == 0;
+            for (int o = lane * 4; o < nk * 32; o += 128) {
+                if (caligned && o + 4 <= cbytes) {
+                    cp_async_4(clsb + o, cbase + o);
+                } else {
+                    uint32_t wv = 0;
+                    for (int q = 0; q < 4; ++q) wv |= (o + q < cbytes) ? (uint32_t)__ldg(cbase + o + q) << (8 * q) : 0u;
+                    clsw[o >> 2] = wv;
                 }
             }
+            cp_async_commit();
+            cp_async_wait<0>();
             __syncwarp();
         }
-        // pass 1: class of every game (0 = at rest or no such game), what is in play; without the fused observation
-        // also the outputs of the games at rest, from their census bytes (with it they are a second pass, below, that
-        // knows which tiles are about to be stepped whole).  Late in a rollout this loop IS the step (a warp walks its
-        // tiles, finds a handful of games in play): unrolled by two so that the tiles' dependency chains interleave.
-#pragma unroll kSchedPassUnroll
-        for (int k = 0; k < nk; ++k) {
-            const long long g = (tile_of(j0 + k) << 5) + lane;
-            const bool valid = g < B;
-            const uint32_t v = clsb[k * 32 + lane];
-            const bool rest = valid && (v & 0x80u) && ((v & 2u) || frozen_rest);
-            const int c = (!valid || rest) ? 0 : census_class(v);
-            clsb[k * 32 + lane] = (uint8_t)(c | (rest ? 0x80 : 0) | ((v & 1u) << 6));  // class | at rest | its live count
-            const uint32_t play = __ballot_sync(0xffffffffu, c != 0);
-            if (play) tilemask |= 1u << k;
-            inplay += __popc(play);
-            const uint32_t vbal = __ballot_sync(0xffffffffu, valid);
-            ngames += __popc(vbal);
-            classes |= 1u << c;
-            if constexpr (SCHED_SPECULATE) {
-                // The round's first tile predicts the round: when at least half of ITS games are in play the tile is
-                // requested now, as the natural order would, and the rest of this pass runs in the shadow of that
-                // load (early in a rollout the pass was a bubble of ~3 us in front of every warp's first tile).  A
-                // wrong guess (the round turns out to be sorted) costs one tile of traffic; its arrival is awaited
-                // below before the stage is used again.
-                if (k == 0 && bulk && play && __popc(play) * 2 >= __popc(vbal)) {
-                    spec = true;
-                    const long long first = g - lane;
-                    bulk_wait_read<0>();
-                    fence_async_smem();
-                    __syncwarp();
-                    if (lane == 0) {
-                        mbar_expect_tx(&bar[0], (uint32_t)__popc(vbal) * (uint32_t)(W * 4));
-                        bulk_load(stages, gst + first * W, (uint32_t)__popc(vbal) * (uint32_t)(W * 4), &bar[0]);
+        // pass 1, four games per lane: class codes of the round (one 32-bit word per lane and group, the byte order of
+        // the class array: byte k * 32 + i is game i of tile k), what is in play; without the fused observation also
+        // the outputs of the games at rest (with it they are a second pass, below, that knows which tiles are about to
+        // be stepped whole).  Late in a rollout this loop IS the step: a warp walks its tiles and finds a handful of
+        // games in play.  Kept rolled: the kernel's hot loops compete for the instruction cache.
+        uint32_t tilemask = 0;
+        int inplay = 0;
+        for (int G = 0; G < ngroups; ++G) {
+            const int o = G * 128 + lane * 4;  // the lane's first game, within the round
+            const int left = cbytes - o;
+            const uint32_t vmask = left >= 4 ? 0xffffffffu : (left > 0 ? (1u << (8 * left)) - 1u : 0u);
+            const uint32_t w = clsw[G * 32 + lane];
+            uint32_t rest7;
+            const uint32_t code = census_codes4(w, vmask, frozen_rest, rest7);
+            clsw[G * 32 + lane] = code;
+            const uint32_t cls = code & 0x07070707u;
+            // tile t of the group is lanes 8t .. 8t+7: byte t of the ballot
+            tilemask |= nonzero_bytes4(__ballot_sync(0xffffffffu, cls != 0)) << (4 * G);
+            inplay += __popc(bytes_ge7(cls, 1));
+            settled_total += __popc(rest7);
+            if constexpr (!OBS) {
+                if (rest7) {
+                    // Four games in one store, those in play included: the chunk loop writes their outputs later, from
+                    // this warp, after the __syncwarp that ends this pass (it orders these stores before those).
+                    const long long g0 = first + o;
+                    const bool whole = left >= 4;
+                    const uint32_t live = w & 0x01010101u;
+                    if (whole && done4) *reinterpret_cast<uint32_t*>(p.done + g0) = rest7 >> 7;
+                    if (whole && reward16) *reinterpret_cast<float4*>(p.reward + g0) = make_float4(rest_reward, rest_reward, rest_reward, rest_reward);
+                    if (whole && npoints16) *reinterpret_cast<int4*>(p.num_points + g0) = make_int4((int)(live & 1u), (int)((live >> 8) & 1u), (int)((live >> 16) & 1u), (int)(live >> 24));
+                    for (uint32_t m = rest7; m; m &= m - 1) {  // otherwise one store per game at rest
+                        const int b = (__ffs((int)m) - 1) >> 3;
+                        if (p.done && !(whole && done4)) p.done[g0 + b] = 1;
+                        if (p.reward && !(whole && reward16)) p.reward[g0 + b] = rest_reward;
+                        if (p.num_points && !(whole && npoints16)) p.num_points[g0 + b] = (int32_t)((live >> (8 * b)) & 1u);
                     }
                 }
-            }
-            if constexpr (!OBS) {
-                if (rest) {
-                    if (p.done) p.done[g] = 1;
-                    if (p.reward) p.reward[g] = rest_reward;
-                    if (p.num_points) p.num_points[g] = (int32_t)(v & 1u);
+                if (p.done_bits) {
+                    // the tile's word of the done mask: the games at rest now (the games that finish in this step are
+                    // ORed in by the chunk loop); eight lanes' nibbles, one lane per tile stores it
+                    uint32_t bits = nonzero_bytes4(rest7) << (4 * (lane & 7));
+                    bits |= __shfl_xor_sync(0xffffffffu, bits, 1);
+                    bits |= __shfl_xor_sync(0xffffffffu, bits, 2);
+                    bits |= __shfl_xor_sync(0xffffffffu, bits, 4);
+                    const int k = G * 4 + (lane >> 3);
+                    if ((lane & 7) == 0 && k < nk) p.done_bits[tile_of(j0 + k)] = bits;
                 }
-                const uint32_t restmask = __ballot_sync(0xffffffffu, rest);
-                settled_total += __popc(restmask);
-                // the tile's word of the done mask: the games at rest now, the games that finish in this step later
-                if (p.done_bits && lane == 0) p.done_bits[tile_of(j0 + k)] = restmask;
             }
         }
-        classes = __reduce_or_sync(0xffffffffu, classes) & ~1u;
+        inplay = __reduce_add_sync(0xffffffffu, inplay);
+        const int ngames = cbytes;
         // While most games are still in play the tiles are stepped whole, in natural order: one bulk copy per
         // tile and coalesced actions / outputs beat the per-game gather, and there is little to skip.  Later the
         // games in play are sorted by class and gathered one by one.
@@ -226,16 +243,52 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) hk_sched_kernel(const StepPa
                 if (m) order[total + __popc(bal & lt)] = (uint16_t)(k * 32 + lane);
                 total += __popc(bal);
             }
-        }
-        for (int q = 1; q <= 6 && !natural && inplay > 32; ++q) {
-            if (!((classes >> q) & 1u)) continue;
-            for (int k = 0; k < nk; ++k) {
-                if (!((tilemask >> k) & 1u)) continue;
-                const bool m = (clsb[k * 32 + lane] & 7u) == (uint32_t)q;
-                const uint32_t bal = __ballot_sync(0xffffffffu, m);
-                if (m) order[total + __popc(bal & lt)] = (uint16_t)(k * 32 + lane);
-                total += __popc(bal);
+        } else if (!natural) {
+            // One counting sort over the class words, in game order inside a class (group, lane, byte).  Counts are
+            // packed three classes to a word in 10-bit fields: a sorted round has fewer than 1024 games in play.
+            // First the round's count of each class, then its start in order[] ...
+            uint32_t tlo = 0, thi = 0;
+            for (int G = 0; G < ngroups; ++G) {
+                if (!((tilemask >> (4 * G)) & 0xfu)) continue;
+                uint32_t lo, hi;
+                class_counts4(clsw[G * 32 + lane], lo, hi);
+                tlo += lo;
+                thi += hi;
             }
+            tlo = __reduce_add_sync(0xffffffffu, tlo);
+            thi = __reduce_add_sync(0xffffffffu, thi);
+            const uint32_t s123 = ((tlo * 0x00100401u) >> 20) & 0x3ffu;  // games of classes 1..3
+            uint32_t plo = ((tlo << 10) + (tlo << 20)) & 0x3ffffc00u;    // starts of classes 1, 2, 3
+            uint32_t phi = s123 * 0x00100401u + (((thi << 10) + (thi << 20)) & 0x3ffffc00u);  // of 4, 5, 6
+            // ... then group by group: a warp scan of the lanes' packed counts gives each lane its place
+            for (int G = 0; G < ngroups; ++G) {
+                if (!((tilemask >> (4 * G)) & 0xfu)) continue;
+                const uint32_t code = clsw[G * 32 + lane];
+                uint32_t lo, hi;
+                class_counts4(code, lo, hi);
+                uint32_t ilo = lo, ihi = hi;  // inclusive scan over the lanes
+#pragma unroll
+                for (int s = 1; s < 32; s <<= 1) {
+                    const uint32_t a = __shfl_up_sync(0xffffffffu, ilo, s), b = __shfl_up_sync(0xffffffffu, ihi, s);
+                    if (lane >= s) {
+                        ilo += a;
+                        ihi += b;
+                    }
+                }
+                uint32_t qlo = plo + ilo - lo, qhi = phi + ihi - hi;  // this lane's next slot of each class
+                plo += __shfl_sync(0xffffffffu, ilo, 31);
+                phi += __shfl_sync(0xffffffffu, ihi, 31);
+#pragma unroll
+                for (int b = 0; b < 4; ++b) {
+                    const int c = (code >> (8 * b)) & 7;
+                    if (c == 0) continue;
+                    const int sh = 10 * (c > 3 ? c - 4 : c - 1);
+                    uint32_t& q = (c > 3) ? qhi : qlo;
+                    order[(q >> sh) & 0x3ffu] = (uint16_t)(G * 128 + lane * 4 + b);
+                    q += 1u << sh;
+                }
+            }
+            total = inplay;
         }
         __syncwarp();
         const int nchunks = natural ? __popc(tilemask) : ((total + 31) >> 5);
@@ -325,14 +378,9 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) hk_sched_kernel(const StepPa
         // that load's DRAM latency (late in a rollout a warp has one short chunk: the load was the longest wait of the step)
         long long g_cur = 0, g_nxt = 0;
         bool v_cur = false, v_nxt = false;
-        if (spec && !natural) {  // the guess was wrong: let the tile land, then forget it
-            mbar_wait(&bar[0], phase_bits & 1u);
-            phase_bits ^= 1u;
-            spec = false;
-        }
         if (inplay) {
             chunk_game(0, g_cur, v_cur);
-            if (!spec) gather(g_cur, v_cur, stages, 0);  // (natural order and a good guess: chunk 0 IS the tile in flight)
+            gather(g_cur, v_cur, stages, 0);
         }
         // pass 2 (fused observation only): the outputs of the games at rest, from their census bytes
         for (int k = 0; OBS && k < nk; ++k) {
@@ -346,7 +394,6 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) hk_sched_kernel(const StepPa
                 if (p.num_points) p.num_points[g] = (int32_t)v;
             }
             const uint32_t restmask = __ballot_sync(0xffffffffu, rest);
-            settled_total += __popc(restmask);
             if constexpr (OBS) {
                 // (warp-uniform) the constant observation of every game at rest of this tile — unless the tile is about to
                 // be stepped whole in natural order: its observation rows are then stored as one block, these included
@@ -585,7 +632,10 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) hk_sched_kernel(const StepPa
         }
     }
     if (bulk || obs_bulk) bulk_wait_all<0>();  // this lane's bulk stores are globally complete before the warp retires
-    if (p.done_count && settled_total && lane == 0) atomicAdd(p.done_count, settled_total);
+    if (p.done_count) {
+        settled_total = __reduce_add_sync(0xffffffffu, settled_total);
+        if (settled_total && lane == 0) atomicAdd(p.done_count, settled_total);
+    }
 }
 
 }  // namespace hk
