@@ -29,9 +29,7 @@ SIGNATURES = {
     "hk_step_census": (ctypes.c_int, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _i32, _i32, _i32, _u32, _u32, _f32, _f32, _p]),
     "hk_step_census_obs": (ctypes.c_int, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _i32, _i32, _i32, _u32, _u32, _f32,
                                           _f32, _p]),
-    "hk_debug_set_sched_geometry": (ctypes.c_int, [ctypes.c_int]),
     "hk_census_bytes": (_i64, [_i64, _i32, _i32]),
-    "hk_debug_set_rows_kernel": (ctypes.c_int, [ctypes.c_int]),
     "hk_debug_set_session_graphs": (ctypes.c_int, [ctypes.c_int]),
     "hk_shift": (ctypes.c_int, [_p, _p, _p, _p, _i64, _i32, _i32, _i32, _u32, _f32, _p]),
     "hk_reposition": (ctypes.c_int, [_p, _p, _i64, _i32, _i32, _i32, _f32, _p]),

@@ -22,8 +22,6 @@ using hk::kMaxDevices;
 
 namespace {
 
-std::atomic<int> g_no_rows_kernel{0};  // test / tuning hook (hk_debug_set_rows_kernel)
-std::atomic<int> g_sched_geometry{0};  // tuning hook (hk_debug_set_sched_geometry)
 std::atomic<int> g_use_pdl{0};  // programmatic dependent launch of the thread-per-game kernel (hk_debug_set_pdl)
 
 struct DevInfo {
@@ -122,15 +120,17 @@ int run(StepParams& p, int dtype, int force_generic, cudaStream_t stream) {
         if (obs && !(sched && (p.flags & (HK_F_OBS_SORT_COORD0 | HK_F_OBS_SORT_LEX | HK_F_OBS_SORT_LEX_FIRST))))
             return HK_ERR_UNSUPPORTED;
         if (sched && obs)
-            return dtype == HK_DTYPE_I32 ? hk::launch_sched_i32_obs(p, dev, stream) : hk::launch_sched_f32_obs(p, dev, stream);
+            return dtype == HK_DTYPE_I32 ? hk::dispatch_sched<int32_t, true>(p, dev, stream)
+                                         : hk::dispatch_sched<float, true>(p, dev, stream);
         if (sched)
-            return dtype == HK_DTYPE_I32 ? hk::launch_sched_i32(p, dev, stream) : hk::launch_sched_f32(p, dev, stream);
+            return dtype == HK_DTYPE_I32 ? hk::dispatch_sched<int32_t, false>(p, dev, stream)
+                                         : hk::dispatch_sched<float, false>(p, dev, stream);
         // Large padded shapes with at most 64 rows: the census carries a live mask per game after the bytes, and the
         // games with few live rows are stepped thread-per-game on their live rows alone (hk_rows_kernel) before
         // the warp-per-game kernel takes the rest.
-        if (hk::rows_shape(p.N, p.d) && !(p.ops & HK_OP_DEDUPE) && !g_no_rows_kernel.load()) {
+        if (hk::rows_shape(p.N, p.d) && !(p.ops & HK_OP_DEDUPE)) {
             p.live_mask = reinterpret_cast<uint64_t*>(p.census + ((p.B + 7) & ~7ll));
-            int rc2 = dtype == HK_DTYPE_I32 ? hk::launch_rows_i32(p, dev, stream) : hk::launch_rows_f32(p, dev, stream);
+            int rc2 = dtype == HK_DTYPE_I32 ? hk::dispatch_rows<int32_t>(p, dev, stream) : hk::dispatch_rows<float>(p, dev, stream);
             if (rc2 != HK_OK) return rc2;
             p.rows_k = hk::ROWS_K;
         } else if (p.done_bits) {  // the warp-per-game kernel ORs the bits in, one game at a time
@@ -194,7 +194,6 @@ std::atomic<int> g_no_session_graphs{0};  // test / tuning hook (hk_debug_set_se
 namespace hk {
 int device_sms(int dev) { return device_sms_impl(dev); }
 bool use_pdl() { return g_use_pdl.load(std::memory_order_relaxed) != 0; }
-int sched_geometry() { return g_sched_geometry.load(std::memory_order_relaxed); }
 }  // namespace hk
 
 extern "C" {
@@ -219,18 +218,6 @@ int hk_kernel_class(int N, int d) {
 // tuning hook: programmatic dependent launch on/off
 int hk_debug_set_pdl(int on) {
     g_use_pdl.store(on ? 1 : 0);
-    return HK_OK;
-}
-
-// tuning hook: geometry of the census-scheduled kernel (0 = 4 warps x 2 stages, 1 = 8 warps x 1 stage)
-int hk_debug_set_sched_geometry(int which) {
-    g_sched_geometry.store(which);
-    return HK_OK;
-}
-
-// test / tuning hook: the small-games kernel of large padded shapes (on by default)
-int hk_debug_set_rows_kernel(int on) {
-    g_no_rows_kernel.store(on ? 0 : 1);
     return HK_OK;
 }
 

@@ -1,7 +1,7 @@
 // hk_launch.cuh — launch helpers shared by the translation units of the library, and the
 // launchers each unit defines.  The kernels are split over several .cu files (hk_small_*.cu,
-// hk_generic_*.cu) only so that they compile in parallel; hk_capi.cu holds the extern "C" boundary
-// and dispatches to these launchers.
+// hk_generic_*.cu, hk_sched_*.cu, hk_rows_*.cu) only so that they compile in parallel; hk_capi.cu
+// holds the extern "C" boundary and dispatches to these launchers.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -16,7 +16,6 @@ constexpr int kMaxDevices = 64;
 
 int device_sms(int dev);  // hk_capi.cu
 bool use_pdl();           // hk_capi.cu (hk_debug_set_pdl)
-int sched_geometry();     // hk_capi.cu (hk_debug_set_sched_geometry)
 
 // per-kernel, per-device launch facts (dynamic smem opt-in + resident CTAs per SM), computed once
 struct KernelFacts {
@@ -73,14 +72,19 @@ extern template int dispatch_generic<float, GenericVariant::Obs>(const StepParam
 extern template int dispatch_generic<float, GenericVariant::Rec>(const StepParams&, int, cudaStream_t);
 extern template int dispatch_generic<float, GenericVariant::Thr>(const StepParams&, int, cudaStream_t);
 extern template int dispatch_generic<float, GenericVariant::ThrRec>(const StepParams&, int, cudaStream_t);
-// census-scheduled thread-per-game kernel (hk_sched.cuh): in-place single steps with p.census
-int launch_sched_i32(const StepParams& p, int dev, cudaStream_t stream);
-int launch_sched_f32(const StepParams& p, int dev, cudaStream_t stream);
-int launch_sched_i32_obs(const StepParams& p, int dev, cudaStream_t stream);  // + fused observation (sorted modes)
-int launch_sched_f32_obs(const StepParams& p, int dev, cudaStream_t stream);
-// small games of large padded shapes, thread-per-game on census masks (hk_rows.cuh)
-int launch_rows_i32(const StepParams& p, int dev, cudaStream_t stream);
-int launch_rows_f32(const StepParams& p, int dev, cudaStream_t stream);
+// census paths: the census-scheduled thread-per-game kernel (hk_sched.cuh), in-place single steps with p.census, OBS
+// with the fused observation (sorted modes); and the small games of large padded shapes, thread-per-game on census
+// masks (hk_rows.cuh).  One instantiation per unit (hk_sched_*.cu, hk_rows_*.cu)
+template <typename T, bool OBS>
+int dispatch_sched(const StepParams& p, int dev, cudaStream_t stream);
+template <typename T>
+int dispatch_rows(const StepParams& p, int dev, cudaStream_t stream);
+extern template int dispatch_sched<int32_t, false>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_sched<int32_t, true>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_sched<float, false>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_sched<float, true>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_rows<int32_t>(const StepParams&, int, cudaStream_t);
+extern template int dispatch_rows<float>(const StepParams&, int, cudaStream_t);
 constexpr int ROWS_K = 8;  // = ROWS_MAX_K of hk_rows.cuh
 inline bool rows_shape(int N, int d) { return N <= 64 && d >= 2 && d <= 5; }
 

@@ -1,5 +1,5 @@
 // small games of large padded shapes (hk_rows.cuh), float state
 #include "hk_rows_launch.inl"
 namespace hk {
-int launch_rows_f32(const StepParams& p, int dev, cudaStream_t stream) { return dispatch_rows<float>(p, dev, stream); }
+template int dispatch_rows<float>(const StepParams&, int, cudaStream_t);
 }  // namespace hk

@@ -1,5 +1,5 @@
 // small games of large padded shapes (hk_rows.cuh), int32_t state
 #include "hk_rows_launch.inl"
 namespace hk {
-int launch_rows_i32(const StepParams& p, int dev, cudaStream_t stream) { return dispatch_rows<int32_t>(p, dev, stream); }
+template int dispatch_rows<int32_t>(const StepParams&, int, cudaStream_t);
 }  // namespace hk

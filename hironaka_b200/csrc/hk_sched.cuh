@@ -28,9 +28,6 @@ constexpr int SCHED_ROUND_TILES = 32;  // tiles (of 32 games) a warp schedules t
 #define SCHED_PASS_UNROLL 2
 #endif
 constexpr int kSchedPassUnroll = SCHED_PASS_UNROLL;
-#ifndef SCHED_DIRECT
-#define SCHED_DIRECT 1  // packed tiers release the stage after the gather and store changed rows straight to global memory
-#endif
 #ifndef SCHED_NATURAL_NUM
 #define SCHED_NATURAL_NUM 1  // a round is stepped tile by tile in natural order while at least NUM / DEN of
 #define SCHED_NATURAL_DEN 2  // its games are in play (tools/time_census.py)
@@ -458,14 +455,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) hk_sched_kernel(const StepPa
             ls.ax = 0;
             ls.origin = false;
             if (ls.shift) load_actions(p, p.flags, ls.g, 0, ls.ha, ls.ax);
-            if constexpr (STAGES == 1 && HK_L2_PREFETCH) {
-                // one stage: the next tile cannot be requested before this one has been stored, but it can wait in L2
-                if (bulk && natural && tiles_left && lane == 0) {
-                    const long long tn = tile_of(j0 + (__ffs((int)tiles_left) - 1));
-                    const long long left = B - (tn << 5);
-                    bulk_prefetch_l2(gst + (tn << 5) * W, (uint32_t)(left < 32 ? left : 32) * (uint32_t)(W * 4));
-                }
-            }
+            // (measured and not kept: with one stage, a prefetch of the next tile into L2 here, as in hk_small.cuh)
             if (bulk) {  // this chunk's games have landed (they were requested one chunk ago)
                 mbar_wait(&bar[sidx], (phase_bits >> sidx) & 1u);
                 phase_bits ^= (1u << sidx);
@@ -488,7 +478,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) hk_sched_kernel(const StepPa
             bool exceed = false;
             bool chg = false;  // in place: only changed games go back
             bool released = false;  // the stage has been handed back (and refilled) in the middle of the step
-            if constexpr (SCHED_DIRECT && !OBS && STAGES == 1 && !Elem<T>::is_float) {
+            if constexpr (!OBS && STAGES == 1 && !Elem<T>::is_float) {
                 // packed tiers, direct route (hk_small.cuh): once the rows are gathered the stage is refilled — the next
                 // chunk's load runs behind this chunk's arithmetic — and the changed rows go straight to global memory
                 auto release = [&]() {

@@ -1,5 +1,5 @@
 // census-scheduled thread-per-game kernel, float state
 #include "hk_sched_launch.inl"
 namespace hk {
-int launch_sched_f32(const StepParams& p, int dev, cudaStream_t stream) { return dispatch_sched<float, false>(p, dev, stream); }
+template int dispatch_sched<float, false>(const StepParams&, int, cudaStream_t);
 }  // namespace hk

@@ -1,5 +1,5 @@
 // census-scheduled thread-per-game kernel with the fused observation, float state
 #include "hk_sched_launch.inl"
 namespace hk {
-int launch_sched_f32_obs(const StepParams& p, int dev, cudaStream_t stream) { return dispatch_sched<float, true>(p, dev, stream); }
+template int dispatch_sched<float, true>(const StepParams&, int, cudaStream_t);
 }  // namespace hk

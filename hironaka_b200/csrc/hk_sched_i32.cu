@@ -1,5 +1,5 @@
 // census-scheduled thread-per-game kernel, int32_t state
 #include "hk_sched_launch.inl"
 namespace hk {
-int launch_sched_i32(const StepParams& p, int dev, cudaStream_t stream) { return dispatch_sched<int32_t, false>(p, dev, stream); }
+template int dispatch_sched<int32_t, false>(const StepParams&, int, cudaStream_t);
 }  // namespace hk

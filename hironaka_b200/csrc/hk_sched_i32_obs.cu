@@ -1,5 +1,5 @@
 // census-scheduled thread-per-game kernel with the fused observation, int32_t state
 #include "hk_sched_launch.inl"
 namespace hk {
-int launch_sched_i32_obs(const StepParams& p, int dev, cudaStream_t stream) { return dispatch_sched<int32_t, true>(p, dev, stream); }
+template int dispatch_sched<int32_t, true>(const StepParams&, int, cudaStream_t);
 }  // namespace hk

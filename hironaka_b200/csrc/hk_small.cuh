@@ -1,8 +1,8 @@
 // hk_small.cuh — thread-per-game step kernel for small games (N <= 32, N*d words in registers).
 //
 // Mapping (DESIGN.md "K-small"): one lane owns one game; a warp owns tiles of 32 consecutive
-// games.  Each warp has a private shared-memory ring of STAGES tiles (one in the shipped geometry):
-// lane 0 issues one TMA bulk load per tile (32*N*d*4 contiguous bytes), all lanes wait on the stage's
+// games.  Each warp has a private shared-memory stage of one tile:
+// lane 0 issues one TMA bulk load per tile (32*N*d*4 contiguous bytes), all lanes wait on the warp's
 // mbarrier and read their own game with conflict-free vector LDS (game stride N*d words: 16-byte
 // reads are conflict-free when N*d/4 is odd, 8-byte when N*d/2 is odd, 4-byte when N*d is odd —
 // true for (20,3), (10,3), (5,3)).  The warp picks a tier from the largest live count among its 32
@@ -28,18 +28,15 @@ constexpr int SMALL_BAR_BYTES = 256;
 #define HK_SPARSE_STORE_MAX 16  // at most this many changed games of a tile are written one by one (tools/tune_small.cu: 4 -> 71.2, 8 -> 68.3, 16 -> 67.3, 32 -> 75.7 us/step at C2)
 #endif
 
-// WARPS warps per CTA, each with a private ring of STAGES tiles.  With STAGES >= 3 the refill of a
-// stage is issued one iteration after its store (cp.async.bulk.wait_group.read 1), so the issuing
-// lane never waits on the store it has just launched; with STAGES == 2 it has to wait for that
-// store to finish reading shared memory before the stage can be refilled.
-template <int N, int D, bool OBS, int WARPS, int STAGES>
+// WARPS warps per CTA, each with a private stage of one tile (and the obs tile with OBS).
+template <int N, int D, bool OBS, int WARPS>
 struct SmallLayout {
-    static_assert(WARPS * STAGES * 8 <= SMALL_BAR_BYTES, "mbarrier area too small");
+    static_assert(WARPS * 8 <= SMALL_BAR_BYTES, "mbarrier area too small");
     static constexpr int W = N * D;
     static constexpr int TILE_WORDS = 32 * W;
     static constexpr int OBS_W = W + D;
     static constexpr int OBS_WORDS = OBS ? 32 * OBS_W : 0;
-    static constexpr int WARP_WORDS = STAGES * TILE_WORDS + OBS_WORDS;
+    static constexpr int WARP_WORDS = TILE_WORDS + OBS_WORDS;
     static constexpr size_t SMEM_BYTES = SMALL_BAR_BYTES + (size_t)WARPS * WARP_WORDS * 4;
 };
 
@@ -582,24 +579,6 @@ __device__ __forceinline__ int tier_steps(const StepParams& p, LaneState& ls, ui
 // back to their slots from the index bits.  The vote is warp-uniform; a warp that fails it (large values,
 // negative entries in live rows) has touched nothing and takes the exact tiers.  Single steps of int32
 // state only.
-#ifndef HK_L2_PREFETCH
-#define HK_L2_PREFETCH 0  // (measured, not kept: +5 % on the first steps at 16 warps per SM, -8 % only at 8) one-stage geometries prefetch their next tile into L2 (cp.async.bulk.prefetch.L2)
-#endif
-#ifndef HK_PACKED_TIERS
-#define HK_PACKED_TIERS 1
-#endif
-#ifndef HK_DIRECT_PAIR_STORES
-#define HK_DIRECT_PAIR_STORES 1
-#endif
-#ifndef HK_SMALL_DIRECT
-#define HK_SMALL_DIRECT 0  // (measured, not kept: the tile-ring kernel with the direct route: C2 steps 2-4 94 92 79 -> 82 73 67 us, but every later step 68 us instead of 50-60: rollout mean 0.0658 -> 0.0672 ms)
-#endif
-#ifndef HK_DIRECT_MAX_ROWS
-#define HK_DIRECT_MAX_ROWS 8
-#endif
-#ifndef HK_PACKED_ROLLOUT
-#define HK_PACKED_ROLLOUT 0
-#endif
 #ifndef HK_PACKED_MIN
 #define HK_PACKED_MIN 2  // smallest warp maximum of live rows that takes a packed tier (2 against 3: C2 steps 4-6 77 61 50 -> 72 52 44 us, the direct route serves the two-row chunks of the sorted order)
 #endif
@@ -791,7 +770,7 @@ __device__ __forceinline__ bool tier_packed(const StepParams& p, LaneState& ls, 
                 const bool lv = (alive >> b) & 1u;
                 const int i = (int)(w[b] & 31u);
                 uint32_t* dst = DIRECT ? (gdst + i * D) : (row + i * D);
-                if constexpr (DIRECT && D == 3 && HK_DIRECT_PAIR_STORES) {
+                if constexpr (DIRECT && D == 3) {
                     // a 12-byte row is one 8-byte and one 4-byte store whatever its alignment (two requests instead of three)
                     uint32_t v[3];
 #pragma unroll
@@ -1260,28 +1239,24 @@ __device__ __forceinline__ bool small_process_tile(const StepParams& p, LaneStat
         // (Measured and not kept: dropping the exact 12- and 16-row tiers from the kernels that have packed ones — 3k
         // instructions less — sends warps whose values no longer pack, common from the fifth step on, to all N rows:
         // rollout mean 0.0449 -> 0.0470 ms per step.)
-        constexpr bool HAS_PACKED = HK_PACKED_TIERS && PACKED && !Elem<T>::is_float && !POLICY && D == 3;
+        constexpr bool HAS_PACKED = PACKED && !Elem<T>::is_float && !POLICY && D == 3;
         if constexpr (HAS_PACKED) {
             // (warp-uniform) single steps with the filter: packed rows while the values allow it.  (Measured and not kept
-            // for one-launch rollouts, HK_PACKED_ROLLOUT: the game would go back to the lane's game area after every
-            // packed step and be gathered again for the next one, 1.07 ms per 20-step C2 rollout against 0.64 ms with the
-            // exact tiers, which keep their rows in registers from step to step.)
-            if ((p.ops & HK_OP_NEWTON) && lmax <= 20 &&
-                ((p.T == 1 && lmax >= HK_PACKED_MIN) || (HK_PACKED_ROLLOUT && p.T > 1 && lmax >= 2))) {
+            // for one-launch rollouts: the game would go back to the lane's game area after every packed step and be
+            // gathered again for the next one, 1.07 ms per 20-step C2 rollout against 0.64 ms with the exact tiers, which
+            // keep their rows in registers from step to step.)
+            if ((p.ops & HK_OP_NEWTON) && lmax <= 20 && (p.T == 1 && lmax >= HK_PACKED_MIN)) {
                 prestore();
                 int32_t ha_n = 3, ax_n = 0;
                 if (ls.shift && st + 1 < p.T) load_actions(p, p.flags, ls.g, st + 1, ha_n, ax_n);  // the next step's actions
                 bool ok = false, tried = false;
                 if constexpr (!std::is_same<Release, NoRelease>::value) {
                     // (warp-uniform) direct route: in place, one step, no dead row had to be rewritten, nothing pending
-                    // (up to HK_DIRECT_MAX_ROWS rows: the 12-byte row stores of a lane are uncoalesced, three store
-                    // instructions per row slot — measured at C2: 18 % faster than the staged tile at 4 rows, 7 % at 8,
-                    // 25 % SLOWER at 12 and 2.5 times slower on the 20-row root filter)
-                    if (gdst != nullptr && p.T == 1 && lmax <= HK_DIRECT_MAX_ROWS && !any_junk && !__any_sync(0xffffffffu, chg)) {
+                    // (up to 8 rows: the 12-byte row stores of a lane are uncoalesced, three store instructions per row
+                    // slot — measured at C2: 18 % faster than the staged tile at 4 rows, 7 % at 8, 25 % SLOWER at 12 and
+                    // 2.5 times slower on the 20-row root filter)
+                    if (gdst != nullptr && p.T == 1 && lmax <= 8 && !any_junk && !__any_sync(0xffffffffu, chg)) {
                         if (lmax <= 4) ok = tier_packed<N, D, 4, true, Release>(p, ls, row, lm, lmax, st, exceed, chg, gdst, release);
-#if HK_DIRECT_MAX_ROWS > 8
-                        else if (lmax > 8) ok = tier_packed<N, D, 12, true, Release>(p, ls, row, lm, lmax, st, exceed, chg, gdst, release);
-#endif
                         else ok = tier_packed<N, D, 8, true, Release>(p, ls, row, lm, lmax, st, exceed, chg, gdst, release);
                         if (ok) return true;
                         tried = true;  // (the values do not pack: the exact tiers below)
@@ -1333,21 +1308,22 @@ __device__ __forceinline__ void warp_copy_words(uint32_t* dst, const uint32_t* s
     for (int w = lane; w < words; w += 32) dst[w] = src[w];
 }
 
-// The thread-per-game kernel: warp-private rings of STAGES tiles of 32 games, WARPS warps per CTA, one persistent wave.
+// The thread-per-game kernel: a warp-private stage of one tile of 32 games, WARPS warps per CTA, one persistent wave.
 // PACKED = false: the instantiation of the one-launch rollouts (p.T > 1), which never take the packed tiers and are bound
 // by instruction fetch: they do not carry that code.
 // V (SmallVariant): Obs builds the features of the final state into the warp's obs tile.  Rec (recorded rollouts):
 // before every step the features of the state go to the warp's obs tile, after it the played actions are written and
 // the tile leaves with one bulk store into row st of p.obs_t.  Thr, ThrRec: rollouts with a value threshold, recorded or
 // not; p.over_step leaves with length.
-template <typename T, int N, int D, bool POLICY, int WARPS, int STAGES, bool PACKED, SmallVariant V>
+template <typename T, int N, int D, bool POLICY, int WARPS, bool PACKED, SmallVariant V>
 __device__ __forceinline__ void small_kernel_body(const StepParams& p) {
     // (static: plain constexpr locals are captured by the [&] lambdas below, which changes the code the compiler emits)
     static constexpr bool OBS = is_obs(V), REC = is_rec(V), THR = is_thr(V);
-    using L = SmallLayout<N, D, OBS || REC, WARPS, STAGES>;
+    using L = SmallLayout<N, D, OBS || REC, WARPS>;
     constexpr int SMALL_WARPS = WARPS;
-    constexpr int SMALL_STAGES = STAGES;
-    constexpr bool DELAYED_REFILL = (STAGES >= 3) && !OBS;  // the single obs tile needs its store drained first
+    // One stage per warp.  The stage index `s` below is always 0, but it stays a loop variable: with the index folded by
+    // hand (one mbarrier, one phase bit, no rotation) ptxas emits different code for every variant.
+    constexpr int SMALL_STAGES = 1;
     constexpr int W = L::W;
     extern __shared__ __align__(128) uint8_t smem_raw[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -1366,7 +1342,6 @@ __device__ __forceinline__ void small_kernel_body(const StepParams& p) {
     const bool obs_tma = aligned16(p.obs);
     const T padv = Elem<T>::pad(p.pad);
     const bool write = (gout != nullptr);
-    const bool mutate = p.ops != 0;
     const bool inplace = (gout == gin) && !(p.flags & HK_F_STORE_ALL);
 
     pdl_launch_dependents();  // the next launch of the stream may begin its prologue as SMs free up
@@ -1414,11 +1389,8 @@ __device__ __forceinline__ void small_kernel_body(const StepParams& p) {
             load_actions(p, p.flags, ls.g, 0, ls.ha, ls.ax);
         }
 
-        if constexpr (SMALL_STAGES == 1 && HK_L2_PREFETCH) {
-            // one stage: this stage's next tile cannot be requested before this one has been stored, but it can wait in L2
-            if (lane == 0 && t + nw < ntiles && tile_tma(t + nw))
-                bulk_prefetch_l2(gin + (t + nw) * (long long)L::TILE_WORDS, (uint32_t)tile_words(t + nw) * 4u);
-        }
+        // (measured and not kept: a prefetch of the warp's next tile into L2 here, cp.async.bulk.prefetch.L2, +5 % on the
+        // first steps at 16 warps per SM, -8 % only at 8)
         if (tma) {
             mbar_wait(&bar[s], (phase_bits >> s) & 1u);
             phase_bits ^= (1u << s);
@@ -1431,7 +1403,6 @@ __device__ __forceinline__ void small_kernel_body(const StepParams& p) {
         // Did this lane's game change?  Unchanged games of an in-place call are not written back
         // (everything is when out != in).
         bool chg = !inplace;
-        bool released = false;  // the stage has been handed back (and refilled) in the middle of the step
         if constexpr (REC) {
             const int nrows = words / W;
             auto rec = [&](int st, bool after) {
@@ -1484,21 +1455,9 @@ __device__ __forceinline__ void small_kernel_body(const StepParams& p) {
                                                                                    rec);
         } else if constexpr (THR) {
             small_process_tile<T, N, D, POLICY, PACKED, NoRelease, NoRec, THR>(p, ls, row, exceed, chg);
-        } else if constexpr (HK_SMALL_DIRECT && PACKED && !OBS && !POLICY && SMALL_STAGES == 1 && !Elem<T>::is_float) {
-            // packed tiers, direct route (tier_packed, DIRECT) of an in-place single step: the stage is refilled as soon as
-            // the rows are gathered and the changed rows go straight to global memory
-            if (inplace && tma && p.T == 1) {  // (warp-uniform)
-                auto release = [&]() {
-                    released = true;
-                    fence_async_smem();
-                    __syncwarp();
-                    if (lane == 0) issue_load(t + nw, s);
-                };
-                small_process_tile<T, N, D, POLICY, PACKED, decltype(release)>(p, ls, row, exceed, chg, gout + ls.g * W, release);
-            } else {
-                small_process_tile<T, N, D, POLICY, PACKED>(p, ls, row, exceed, chg);
-            }
         } else {
+            // (measured and not kept: the direct route of the packed tiers here, as in the census kernel — C2 steps 2-4
+            // 94 92 79 -> 82 73 67 us, but every later step 68 us instead of 50-60: rollout mean 0.0658 -> 0.0672 ms)
             small_process_tile<T, N, D, POLICY, PACKED>(p, ls, row, exceed, chg);
         }
 
@@ -1597,19 +1556,11 @@ __device__ __forceinline__ void small_kernel_body(const StepParams& p) {
         fence_async_smem();
         __syncwarp();
         if (lane == 0) {
-            if constexpr (DELAYED_REFILL) {
-                // Every iteration commits a (possibly empty) bulk group, so "at most one group still
-                // reading" means the PREVIOUS iteration's store has drained its stage: refill that one.
+            if (stored) {
                 bulk_commit();
-                bulk_wait_read<1>();
-                if (t != gw) issue_load(t + (SMALL_STAGES - 1) * nw, s == 0 ? SMALL_STAGES - 1 : s - 1);
-            } else {
-                if (stored) {
-                    bulk_commit();
-                    bulk_wait_read<0>();  // the stage (and obs tile) may be overwritten from here on
-                }
-                if (!released) issue_load(t + SMALL_STAGES * nw, s);
+                bulk_wait_read<0>();  // the stage (and obs tile) may be overwritten from here on
             }
+            issue_load(t + SMALL_STAGES * nw, s);
         }
         __syncwarp();
         s = (s + 1 == SMALL_STAGES) ? 0 : s + 1;
@@ -1617,9 +1568,9 @@ __device__ __forceinline__ void small_kernel_body(const StepParams& p) {
     if (lane == 0) bulk_wait_all<0>();  // all bulk stores globally complete before the warp retires
 }
 
-template <typename T, int N, int D, bool POLICY, int WARPS, int STAGES, bool PACKED, SmallVariant V>
+template <typename T, int N, int D, bool POLICY, int WARPS, bool PACKED, SmallVariant V>
 __global__ void __launch_bounds__(WARPS * 32) hk_small_kernel(const StepParams p) {
-    small_kernel_body<T, N, D, POLICY, WARPS, STAGES, PACKED, V>(p);
+    small_kernel_body<T, N, D, POLICY, WARPS, PACKED, V>(p);
 }
 
 }  // namespace hk

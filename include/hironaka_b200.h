@@ -119,13 +119,6 @@ int hk_debug_force_generic(int on);
 /* Tuning hook: programmatic dependent launch (cudaLaunchAttributeProgrammaticStreamSerialization) of
  * the thread-per-game kernel, off by default (measured: no gain); results do not depend on it. */
 int hk_debug_set_pdl(int on);
-
-/* Tuning hook: geometry of the census-scheduled kernel (0 = the default: int32 state 4 warps x 1 stage held to 128 registers,
- * float32 state 4 warps x 2 stages; 1 = 8 warps x 1 stage). */
-int hk_debug_set_sched_geometry(int which);
-
-/* Test / tuning hook: the small-games kernel of large padded shapes (hk_rows_kernel); 0 turns it off. */
-int hk_debug_set_rows_kernel(int on);
 /* Test / tuning hook: hk_session_rollout_ex replays a repeated call (same arguments) as a CUDA graph; 0 turns that off. */
 int hk_debug_set_session_graphs(int on);
 

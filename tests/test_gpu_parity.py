@@ -708,22 +708,17 @@ def test_features_pack_borders(hb, family, N):
 # ---------------------------------------------------------------- the census step
 
 
-@pytest.mark.parametrize("shape", [(40003, 20, 3), (2500, 10, 3), (1111, 5, 3), (31, 20, 3), (3000, 64, 5), (700, 16, 4),
-                                   (5003, 33, 3), (900, 40, 2), (300, 100, 3)],
-                         ids=lambda s: "x".join(map(str, s)))
-@pytest.mark.parametrize("dtype", [np.int32, np.float32])
-@pytest.mark.parametrize("geometry", [0, 1])
-def test_census_step_equals_oracle(hb, shape, dtype, geometry):
-    """hk_step_census over whole rollouts: games at rest are answered from their census byte, games in play
-    are reordered by live count — state, done, reward, num_points and the finished count must equal the
-    oracle's after EVERY step, for both flavours, from starts with junk in dead rows, empty games and
-    lone points, with the caller rewriting games (and zeroing their census bytes) along the way."""
-    from hironaka_b200 import ops
-    from hironaka_b200._lib import lib
-    lib().hk_debug_set_sched_geometry(geometry)
-    B, N, d = shape
-    rng = np.random.default_rng(B + N + geometry)
-    T = 14
+CENSUS_FLAVOURS = {
+    "jax": (O.OP_SHIFT | O.OP_REPOSITION | O.OP_NEWTON, O.F_ACT_DISCRETE),
+    "torch-agent": (O.OP_SHIFT | O.OP_NEWTON, TORCH_FLAGS | O.F_ACT_DISCRETE | O.F_ROLE_AGENT),
+    "no-reposition": (O.OP_SHIFT | O.OP_NEWTON, O.F_ACT_DISCRETE),
+}
+
+
+def census_rollout_inputs(B, N, d, dtype, T=14):
+    """The start state and, per flavour of CENSUS_FLAVOURS (in that order), the T steps' actions and the games the
+    caller rewrites after steps 2, 6 and 10 (None elsewhere): all drawn from one generator seeded with B + N."""
+    rng = np.random.default_rng(B + N)
     x0 = random_state(rng, B, N, d, max_value=9, dead_frac=0.45, dup_frac=0.1).astype(dtype)
     junk = rng.random((B, N)) < 0.3
     x0[(x0[:, :, 0] < 0) & junk] = -7
@@ -731,43 +726,66 @@ def test_census_step_equals_oracle(hb, shape, dtype, geometry):
     x0[1::5, 1:] = -1
     x0[1::5, 0] = np.abs(x0[1::5, 0])
     ncls = 2 ** d - d - 1
-    for ops_bits, flags in ((O.OP_SHIFT | O.OP_REPOSITION | O.OP_NEWTON, O.F_ACT_DISCRETE),
-                            (O.OP_SHIFT | O.OP_NEWTON, TORCH_FLAGS | O.F_ACT_DISCRETE | O.F_ROLE_AGENT),
-                            (O.OP_SHIFT | O.OP_NEWTON, O.F_ACT_DISCRETE)):
-        o = x0.copy()
-        g = dev(x0)
-        census = ops.new_census(g)
+    steps = {}
+    for name in CENSUS_FLAVOURS:
+        steps[name] = []
         for t in range(T):
             ha = rng.integers(0, ncls, B).astype(np.int32)
             ax = rng.integers(0, d, B).astype(np.int32)
-            o, od, orw, onp = cport.step(o, ha, ax, ops_bits, flags)
-            dc = torch.zeros(1, dtype=torch.int32, device="cuda")
-            r = ops.step(g, dev(ha), dev(ax), ops=ops_bits, flags=flags, inplace=True, want_done=True, want_reward=True,
-                         want_num_points=True, census=census, done_count=dc)
-            assert np.array_equal(g.cpu().numpy(), o), (ops_bits, flags, t)
-            assert np.array_equal(r.done.cpu().numpy(), od.astype(bool)), (ops_bits, flags, t)
-            assert np.array_equal(r.reward.cpu().numpy().view(np.int32), orw.view(np.int32)), (ops_bits, flags, t)
-            assert np.array_equal(r.num_points.cpu().numpy(), onp), (ops_bits, flags, t)
-            assert int(dc.item()) == int(od.sum()), (ops_bits, flags, t)
-            if t % 4 == 2:  # the caller rewrites some games and zeroes their census bytes
+            rewrite = None
+            if t % 4 == 2:
                 idx = rng.permutation(B)[:max(1, B // 30)]
                 fresh = random_state(rng, len(idx), N, d, max_value=7, dead_frac=0.3).astype(dtype)
                 fresh[(fresh[:, :, 0] < 0) & (rng.random((len(idx), N)) < 0.5)] = -3
-                o[idx] = fresh
-                ti = torch.from_numpy(idx).cuda()
-                g[ti] = dev(fresh)
-                census[ti] = 0
-        c = census.cpu().numpy()[:B]
-        live = (o[:, :, 0] >= 0).sum(1)
-        known = c != 0
-        assert np.array_equal(np.where(c[known] & 0x80, c[known] & 1, c[known]), live[known]), "census counts"
-        if hb.ops.kernel_class(N, d) == 1:
-            assert known.all()
-        if census.numel() > B:  # large padded shape: the live masks of the known games name exactly the live rows
-            masks = census.cpu().numpy()[(B + 7) // 8 * 8:].view(np.uint64)
-            want = ((o[:, :, 0] >= 0).astype(np.uint64) << np.arange(N, dtype=np.uint64)[None, :]).sum(1, dtype=np.uint64)
-            assert np.array_equal(masks[known], want[known]), "census masks"
-    lib().hk_debug_set_sched_geometry(0)
+                rewrite = (idx, fresh)
+            steps[name].append((ha, ax, rewrite))
+    return x0, steps
+
+
+@pytest.mark.parametrize("shape", [(40003, 20, 3), (2500, 10, 3), (1111, 5, 3), (31, 20, 3), (3000, 64, 5), (700, 16, 4),
+                                   (5003, 33, 3), (900, 40, 2), (300, 100, 3)],
+                         ids=lambda s: "x".join(map(str, s)))
+@pytest.mark.parametrize("dtype", [np.int32, np.float32])
+@pytest.mark.parametrize("flavour", list(CENSUS_FLAVOURS))
+def test_census_step_equals_oracle(hb, shape, dtype, flavour):
+    """hk_step_census over whole rollouts: games at rest are answered from their census byte, games in play
+    are reordered by live count — state, done, reward, num_points and the finished count must equal the
+    oracle's after EVERY step, for both flavours, from starts with junk in dead rows, empty games and
+    lone points, with the caller rewriting games (and zeroing their census bytes) along the way.  The three
+    flavours of a shape and dtype share one input stream (census_rollout_inputs), each case plays its part."""
+    from hironaka_b200 import ops
+    B, N, d = shape
+    ops_bits, flags = CENSUS_FLAVOURS[flavour]
+    x0, steps = census_rollout_inputs(B, N, d, dtype)
+    o = x0.copy()
+    g = dev(x0)
+    census = ops.new_census(g)
+    for t, (ha, ax, rewrite) in enumerate(steps[flavour]):
+        o, od, orw, onp = cport.step(o, ha, ax, ops_bits, flags)
+        dc = torch.zeros(1, dtype=torch.int32, device="cuda")
+        r = ops.step(g, dev(ha), dev(ax), ops=ops_bits, flags=flags, inplace=True, want_done=True, want_reward=True,
+                     want_num_points=True, census=census, done_count=dc)
+        assert np.array_equal(g.cpu().numpy(), o), (ops_bits, flags, t)
+        assert np.array_equal(r.done.cpu().numpy(), od.astype(bool)), (ops_bits, flags, t)
+        assert np.array_equal(r.reward.cpu().numpy().view(np.int32), orw.view(np.int32)), (ops_bits, flags, t)
+        assert np.array_equal(r.num_points.cpu().numpy(), onp), (ops_bits, flags, t)
+        assert int(dc.item()) == int(od.sum()), (ops_bits, flags, t)
+        if rewrite is not None:  # the caller rewrites some games and zeroes their census bytes
+            idx, fresh = rewrite
+            o[idx] = fresh
+            ti = torch.from_numpy(idx).cuda()
+            g[ti] = dev(fresh)
+            census[ti] = 0
+    c = census.cpu().numpy()[:B]
+    live = (o[:, :, 0] >= 0).sum(1)
+    known = c != 0
+    assert np.array_equal(np.where(c[known] & 0x80, c[known] & 1, c[known]), live[known]), "census counts"
+    if hb.ops.kernel_class(N, d) == 1:
+        assert known.all()
+    if census.numel() > B:  # large padded shape: the live masks of the known games name exactly the live rows
+        masks = census.cpu().numpy()[(B + 7) // 8 * 8:].view(np.uint64)
+        want = ((o[:, :, 0] >= 0).astype(np.uint64) << np.arange(N, dtype=np.uint64)[None, :]).sum(1, dtype=np.uint64)
+        assert np.array_equal(masks[known], want[known]), "census masks"
 
 
 def test_census_step_baseline_size(hb):

@@ -16,8 +16,8 @@ full() {  # full <name> <kernel regex> <skip> <count> <command...>
 }
 $B > $OUT/plain_${TAG}.log 2>&1 || { echo "plain bench failed"; tail -5 $OUT/plain_${TAG}.log; exit 1; }
 ncu --metrics gpu__time_duration.sum --clock-control none -c 400 --csv --log-file $OUT/launches_${TAG}.csv $B > $OUT/ncu1_${TAG}.log 2>&1
-full step  hk_sched_kernel 21 21 python tools/time_census.py c2 2 census0
-full c5    "hk_(rows|generic)_kernel" 42 42 python tools/time_census.py c5 2 census0
+full step  hk_sched_kernel 21 21 python tools/time_census.py c2 2 census
+full c5    "hk_(rows|generic)_kernel" 42 42 python tools/time_census.py c5 2 census
 full obs   hk_small_kernel 41 20 python tools/profile_misc.py obs_c2
 full rollc2 hk_small_kernel 3 1 python tools/profile_misc.py rollout_c2
 full rollc5 hk_generic_kernel 3 1 python tools/profile_misc.py rollout_c5

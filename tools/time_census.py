@@ -1,5 +1,5 @@
 """Per-step device times of a C2 (or C5) random-play rollout: hk_step (tile ring) against hk_step_census
-(census-scheduled), both geometries.  python tools/time_census.py [c2|c5] [reps]"""
+(census-scheduled).  python tools/time_census.py [c2|c5] [reps] [census]"""
 import json
 import os
 import sys
@@ -30,9 +30,8 @@ ROOT = C.HK_OP_NEWTON | C.HK_OP_REPOSITION
 root_ms = []
 
 
-def run(census_mode, geometry=0):
+def run(census_mode):
     root_ms.clear()
-    L.hk_debug_set_sched_geometry(geometry)
     per = []
     final = None
     for rep in range(reps):
@@ -76,15 +75,13 @@ def run(census_mode, geometry=0):
 out = {}
 only = sys.argv[3] if len(sys.argv) > 3 else ""
 if only.startswith("census"):  # profiling runs: one mode only
-    per, _ = run(True, int(only[-1]))
+    per, _ = run(True)
     print(json.dumps({only: [round(float(v), 4) for v in per]}))
     sys.exit(0)
 base, xb = run(False)
 out["hk_step"] = {"mean_ms": float(base.mean()), "by_step": [round(float(v), 4) for v in base], "root_filter_ms": round(float(np.mean(root_ms)), 4)}
-for geo in [int(g) for g in os.environ.get('HK_GEOS', '0,1').split(',')]:
-    per, xc = run(True, geo)
-    assert os.environ.get("HK_NOASSERT") or torch.equal(xc, xb), "census rollout differs from hk_step rollout"
-    out[f"hk_step_census_geometry{geo}"] = {"mean_ms": float(per.mean()), "by_step": [round(float(v), 4) for v in per], "root_filter_ms": round(float(np.mean(root_ms)), 4)}
-L.hk_debug_set_sched_geometry(0)
+per, xc = run(True)
+assert os.environ.get("HK_NOASSERT") or torch.equal(xc, xb), "census rollout differs from hk_step rollout"
+out["hk_step_census"] = {"mean_ms": float(per.mean()), "by_step": [round(float(v), 4) for v in per], "root_filter_ms": round(float(np.mean(root_ms)), 4)}
 out["workload"] = f"{which}: B={B} N={N} d={d} T={T}"
 print(json.dumps(out))

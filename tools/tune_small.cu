@@ -1,6 +1,6 @@
 // tune_small.cu — standalone tuning harness for the thread-per-game kernel (not part of the product).
-// Plays R random-play rollouts of the C2 workload (N=20, d=3, 1 Mi games) with several ring
-// geometries and prints the mean launch time by rollout step for each, plus a state checksum.
+// Plays R random-play rollouts of the C2 workload (N=20, d=3, 1 Mi games) with several warps-per-CTA
+// counts and prints the mean launch time by rollout step for each, plus a state checksum.
 //   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -o tune_small tools/tune_small.cu
 #include <cstdio>
 #include <cstdlib>
@@ -16,15 +16,15 @@ constexpr int N = 20, D = 3, T = 20;
 #define TUNE_EXTRA_FLAGS 0u
 #endif
 
-template <int WARPS, int STAGES, bool OBS = false>
+template <int WARPS, bool OBS = false>
 float launch(const hk::StepParams& p, cudaStream_t st, int sms, bool time_it, cudaEvent_t e0, cudaEvent_t e1) {
-    using L = hk::SmallLayout<N, D, OBS, WARPS, STAGES>;
-    auto k = hk::hk_small_kernel<int32_t, N, D, false, WARPS, STAGES, true, OBS ? hk::SmallVariant::Obs : hk::SmallVariant::Step>;
+    using L = hk::SmallLayout<N, D, OBS, WARPS>;
+    auto k = hk::hk_small_kernel<int32_t, N, D, false, WARPS, true, OBS ? hk::SmallVariant::Obs : hk::SmallVariant::Step>;
     static int per_sm = 0;
     if (!per_sm) {
         CK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L::SMEM_BYTES));
         CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, WARPS * 32, L::SMEM_BYTES));
-        printf("  [W=%d S=%d OBS=%d] smem/CTA=%zu B, CTAs/SM=%d, warps/SM=%d\n", WARPS, STAGES, (int)OBS, L::SMEM_BYTES, per_sm, per_sm * WARPS);
+        printf("  [W=%d OBS=%d] smem/CTA=%zu B, CTAs/SM=%d, warps/SM=%d\n", WARPS, (int)OBS, L::SMEM_BYTES, per_sm, per_sm * WARPS);
     }
     long long ntiles = (p.B + 31) / 32;
     long long ctas = (ntiles + WARPS - 1) / WARPS;
@@ -37,7 +37,7 @@ float launch(const hk::StepParams& p, cudaStream_t st, int sms, bool time_it, cu
     return 0.f;
 }
 
-template <int WARPS, int STAGES, bool OBS = false>
+template <int WARPS, bool OBS = false>
 void run_variant(int B, int R, const std::vector<int32_t>& pts, const std::vector<int32_t>& ha, const std::vector<int32_t>& ax) {
     int sms = 148;
     CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, 0));
@@ -58,13 +58,13 @@ void run_variant(int B, int R, const std::vector<int32_t>& pts, const std::vecto
     for (int r = 0; r < R; ++r) {
         int32_t* s = d_state + (size_t)r * B * N * D;
         p.in = s; p.out = s; p.ops = HK_OP_NEWTON | HK_OP_REPOSITION; p.flags = 0; p.host_action = nullptr; p.axis = nullptr; p.done = nullptr; p.reward = nullptr;
-        launch<WARPS, STAGES, false>(p, st, sms, true, e0, e1);
+        launch<WARPS, false>(p, st, sms, true, e0, e1);
         CK(cudaEventSynchronize(e1)); float ms; CK(cudaEventElapsedTime(&ms, e0, e1)); init_ms += ms;
         p.ops = HK_OP_SHIFT | HK_OP_REPOSITION | HK_OP_NEWTON; p.flags = HK_F_ACT_DISCRETE | TUNE_EXTRA_FLAGS; p.done = d_done; p.reward = d_rew;
         if (OBS) { p.obs = d_obs; p.flags |= HK_F_OBS_SORT_LEX | HK_F_OBS_RESCALE; }
         for (int t = 0; t < T; ++t) {
             p.host_action = d_ha + ((size_t)r * T + t) * B; p.axis = d_ax + ((size_t)r * T + t) * B;
-            launch<WARPS, STAGES, OBS>(p, st, sms, true, e0, e1);
+            launch<WARPS, OBS>(p, st, sms, true, e0, e1);
             CK(cudaEventSynchronize(e1)); CK(cudaEventElapsedTime(&ms, e0, e1));
             if (r > 0) by_step[t] += ms;  // rollout 0 is warm-up
         }
@@ -74,7 +74,7 @@ void run_variant(int B, int R, const std::vector<int32_t>& pts, const std::vecto
         double cp = 0, mc = 0; float ms;
         for (int i = 0; i < 12; ++i) {
             int32_t* s = d_state + (size_t)(i % R) * B * N * D; p.in = s; p.out = s;
-            launch<WARPS, STAGES, false>(p, st, sms, true, e0, e1);
+            launch<WARPS, false>(p, st, sms, true, e0, e1);
             CK(cudaEventSynchronize(e1)); CK(cudaEventElapsedTime(&ms, e0, e1)); if (i >= 2) cp += ms;
         }
         for (int i = 0; i < 12; ++i) {
@@ -92,15 +92,15 @@ void run_variant(int B, int R, const std::vector<int32_t>& pts, const std::vecto
     unsigned long long cs = 1469598103934665603ull;
     for (size_t i = 0; i < out.size(); ++i) cs = (cs ^ (unsigned)out[i]) * 1099511628211ull;
     double tot = 0; for (int t = 0; t < T; ++t) { by_step[t] /= (R - 1); tot += by_step[t]; }
-    printf("W=%d S=%d OBS=%d: init %.1f us | mean/step %.2f us (%.3f of 6543.7 GB/s) | t0..t4: %.1f %.1f %.1f %.1f %.1f | t5..19 mean %.2f | checksum %016llx\n",
-           WARPS, STAGES, (int)OBS, 1e3 * init_ms / R, 1e3 * tot / T, (double)B * (OBS ? 733 : 493) / (tot / T * 1e-3) / 6543.7e9,
+    printf("W=%d OBS=%d: init %.1f us | mean/step %.2f us (%.3f of 6543.7 GB/s) | t0..t4: %.1f %.1f %.1f %.1f %.1f | t5..19 mean %.2f | checksum %016llx\n",
+           WARPS, (int)OBS, 1e3 * init_ms / R, 1e3 * tot / T, (double)B * (OBS ? 733 : 493) / (tot / T * 1e-3) / 6543.7e9,
            1e3 * by_step[0], 1e3 * by_step[1], 1e3 * by_step[2], 1e3 * by_step[3], 1e3 * by_step[4],
            1e3 * (tot - by_step[0] - by_step[1] - by_step[2] - by_step[3] - by_step[4]) / 15, cs);
     cudaFree(d_state); cudaFree(d_ha); cudaFree(d_ax); cudaFree(d_done); cudaFree(d_rew);
 }
 
 // one-launch T-step rollouts (hk_rollout): state read and written once per T steps
-template <int WARPS, int STAGES>
+template <int WARPS>
 void run_rollout(int B, int R, const std::vector<int32_t>& pts, const std::vector<int32_t>& ha, const std::vector<int32_t>& ax) {
     int sms = 148;
     CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, 0));
@@ -119,10 +119,10 @@ void run_rollout(int B, int R, const std::vector<int32_t>& pts, const std::vecto
     for (int r = 0; r < R; ++r) {
         int32_t* s = d_state + (size_t)r * B * N * D;
         p.in = s; p.out = s; p.T = 1; p.ops = HK_OP_NEWTON | HK_OP_REPOSITION; p.flags = 0; p.host_action = nullptr; p.axis = nullptr; p.done_count = nullptr;
-        launch<WARPS, STAGES>(p, st, sms, false, e0, e1);
+        launch<WARPS>(p, st, sms, false, e0, e1);
         p.T = T; p.ops = HK_OP_SHIFT | HK_OP_REPOSITION | HK_OP_NEWTON; p.flags = HK_F_ACT_DISCRETE; p.done_count = d_cnt;
         p.host_action = d_ha + (size_t)r * T * B; p.axis = d_ax + (size_t)r * T * B;
-        launch<WARPS, STAGES>(p, st, sms, true, e0, e1);
+        launch<WARPS>(p, st, sms, true, e0, e1);
         CK(cudaEventSynchronize(e1)); float ms; CK(cudaEventElapsedTime(&ms, e0, e1));
         if (r > 0) tot += ms;
     }
@@ -130,7 +130,7 @@ void run_rollout(int B, int R, const std::vector<int32_t>& pts, const std::vecto
     CK(cudaMemcpy(out.data(), d_state, sbytes, cudaMemcpyDeviceToHost));
     unsigned long long cs = 1469598103934665603ull;
     for (size_t i = 0; i < out.size(); ++i) cs = (cs ^ (unsigned)out[i]) * 1099511628211ull;
-    printf("ROLLOUT W=%d S=%d: %.3f ms per %d-step rollout = %.3e game-steps/s | checksum %016llx\n", WARPS, STAGES, tot / (R - 1), T,
+    printf("ROLLOUT W=%d: %.3f ms per %d-step rollout = %.3e game-steps/s | checksum %016llx\n", WARPS, tot / (R - 1), T,
            (double)B * T / (tot / (R - 1) * 1e-3), cs);
     cudaFree(d_state); cudaFree(d_ha); cudaFree(d_ax); cudaFree(d_cnt);
 }
