@@ -11,6 +11,7 @@
 #include <cstring>
 #include <new>
 
+#include "hk_census.cuh"
 #include "hk_experience.cuh"
 #include "hk_launch.cuh"
 #include "hk_value.cuh"
@@ -129,7 +130,7 @@ int run(StepParams& p, int dtype, int force_generic, cudaStream_t stream) {
         // games with few live rows are stepped thread-per-game on their live rows alone (hk_rows_kernel) before
         // the warp-per-game kernel takes the rest.
         if (hk::rows_shape(p.N, p.d) && !(p.ops & HK_OP_DEDUPE)) {
-            p.live_mask = reinterpret_cast<uint64_t*>(p.census + ((p.B + 7) & ~7ll));
+            p.live_mask = reinterpret_cast<uint64_t*>(p.census + hk::census_mask_offset(p.B));
             int rc2 = dtype == HK_DTYPE_I32 ? hk::dispatch_rows<int32_t>(p, dev, stream) : hk::dispatch_rows<float>(p, dev, stream);
             if (rc2 != HK_OK) return rc2;
             p.rows_k = hk::ROWS_K;
@@ -222,9 +223,7 @@ int hk_debug_set_pdl(int on) {
 }
 
 int64_t hk_census_bytes(int64_t B, int32_t N, int32_t d) {
-    if (B < 0) return 0;
-    if (hk::is_small_shape(N, d) || !hk::rows_shape(N, d)) return B;
-    return ((B + 7) & ~7ll) + 8 * B;  // census bytes, then one 64-bit live mask per game
+    return B < 0 ? 0 : hk::census_bytes(B, N, d);
 }
 
 // test / tuning hook: host-buffer rollouts replayed as CUDA graphs (on by default)
@@ -285,21 +284,8 @@ int hk_step_census(void* state, const int32_t* host_action, const int32_t* axis,
                    float* reward, int32_t* num_points, uint8_t* census, int32_t* done_count, int32_t* exceed_flag, int64_t B, int32_t N,
                    int32_t d, int32_t dtype, uint32_t ops, uint32_t flags, float padding_value, float value_threshold,
                    void* stream) {
-    if (census == nullptr || state == nullptr) return HK_ERR_BAD_ARG;
-    StepParams p = make_params(state, state, B, N, d, padding_value);
-    p.host_action = host_action;
-    p.axis = axis;
-    p.done = done;
-    p.done_bits = done_bits;
-    p.reward = reward;
-    p.num_points = num_points;
-    p.census = census;
-    p.done_count = done_count;
-    p.exceed_flag = exceed_flag;
-    p.ops = ops;
-    p.flags = flags;
-    p.threshold = value_threshold;
-    return run(p, dtype, g_force_generic.load(), (cudaStream_t)stream);
+    return hk_step_census_obs(state, host_action, axis, done, done_bits, reward, num_points, nullptr, nullptr, census,
+                              done_count, exceed_flag, B, N, d, dtype, ops, flags, padding_value, value_threshold, stream);
 }
 
 int hk_shift(const void* state_in, void* state_out, const int32_t* host_action, const int32_t* axis, int64_t B,

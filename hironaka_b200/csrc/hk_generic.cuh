@@ -11,7 +11,7 @@
 // owning rows l, l+32, ..., with the compact list of live rows feeding the dominator loop.  This is
 // the kernel for BASELINE config 5 (N=64, d=5).
 #pragma once
-#include "hk_common.cuh"
+#include "hk_census.cuh"
 
 #ifndef HK_GENERIC_MIN_CTAS
 #define HK_GENERIC_MIN_CTAS 4  // resident CTAs of 8 warps the register budget is sized for (tools/time_c5.py)
@@ -210,11 +210,10 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
     // iteration cbase + l; two batches, so the look-ahead never waits on a load); a ballot turns a batch into a
     // mask of the games to PLAY, and the loop jumps from one set bit to the next: a skipped game costs nothing.
     const bool use_census = CENSUS && (p.census != nullptr);
-    const bool frozen_rest = (kflags & HK_F_FREEZE_ENDED) && !(kops & (HK_OP_REPOSITION | HK_OP_RESCALE));
+    const bool frozen_rest = census_frozen_rest(kops, kflags);
     const uint32_t rows_k = CENSUS ? (uint32_t)p.rows_k : 0u;
-    auto at_rest = [&](uint32_t v) -> bool { return (v & 0x80u) && ((v & 2u) || frozen_rest); };
     auto skip_game = [&](uint32_t v) -> bool {
-        return at_rest(v) || (rows_k && v != 0 && (((v & 0x80u) ? (v & 1u) : v) <= rows_k));
+        return census_at_rest(v, frozen_rest) || (rows_k && v != 0 && census_live_count(v) <= rows_k);
     };
     // census mask of the game just stepped: bit i <=> row i alive (N <= 64)
     auto store_mask = [&](long long gg, uint32_t lo, uint32_t hi) {
@@ -237,11 +236,9 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
         const long long gg = gw + itl * nw;
         cv = (use_census && exists) ? (uint32_t)__ldg(p.census + gg) : 0u;
         if (use_census && !rows_k) {
-            const bool rest = exists && at_rest(cv);
+            const bool rest = exists && census_at_rest(cv, frozen_rest);
             if (rest) {
-                if (p.done) p.done[gg] = 1;
-                if (p.reward) p.reward[gg] = (kflags & HK_F_ROLE_AGENT) ? -0.0f : 0.0f;
-                if (p.num_points) p.num_points[gg] = (int32_t)(cv & 1u);
+                write_rest_outputs(p, gg, cv, rest_reward(kflags));
                 if (p.done_bits) atomicOr(p.done_bits + (gg >> 5), 1u << (gg & 31));
             }
             if (p.done_count) {
@@ -398,7 +395,7 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
             }
             if (lane == 0) {
                 if (p.done) p.done[g] = 1;
-                if (p.reward) p.reward[g] = (kflags & HK_F_ROLE_AGENT) ? -0.0f : 0.0f;
+                if (p.reward) p.reward[g] = rest_reward(kflags);
                 if (p.num_points) p.num_points[g] = cnt;
                 if (p.length) p.length[g] = 0;
                 if (CENSUS && p.done_bits) atomicOr(p.done_bits + (g >> 5), 1u << (g & 31));
@@ -415,7 +412,7 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
                     }
                 }
                 const bool org = !__any_sync(0xffffffffu, moving);
-                if (lane == 0) p.census[g] = (uint8_t)(0x80u | (org ? 2u : 0u) | (uint32_t)cnt);
+                if (lane == 0) p.census[g] = census_after_step(cnt, org);
                 if (p.live_mask)
                     store_mask(g, __ballot_sync(0xffffffffu, mylive & 1u), __ballot_sync(0xffffffffu, (mylive >> 1) & 1u));
             }
@@ -480,7 +477,7 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
                         const bool dn = cur < 2;
                         if (lane == 0) {
                             if (p.done) p.done[(long long)st * p.B + g] = dn ? 1 : 0;
-                            if (p.reward) p.reward[(long long)st * p.B + g] = (kflags & HK_F_ROLE_AGENT) ? -0.0f : 0.0f;
+                            if (p.reward) p.reward[(long long)st * p.B + g] = rest_reward(kflags);
                         }
                         if (p.done_count && dn) count_done(st);
                         continue;
@@ -587,10 +584,7 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
                 if (lane == 0) {
                     if (p.done) p.done[(long long)st * p.B + g] = dn ? 1 : 0;
                     if (CENSUS && p.done_bits && dn) atomicOr(p.done_bits + (g >> 5), 1u << (g & 31));
-                    if (p.reward) {
-                        const float rw = (dn && !prev_done) ? 1.0f : 0.0f;
-                        p.reward[(long long)st * p.B + g] = (kflags & HK_F_ROLE_AGENT) ? -rw : rw;
-                    }
+                    if (p.reward) p.reward[(long long)st * p.B + g] = step_reward(kflags, dn, prev_done);
                 }
                 if (p.done_count && dn) count_done(st);
                 if (dn && !prev_done) len = st + 1;
@@ -614,8 +608,7 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
                     for (int k = 0; k < D; ++k) moving = moving || (Elem<T>::bits(v[k]) != 0);
                 }
                 const bool org = !__any_sync(0xffffffffu, moving);
-                if (lane == 0)
-                    p.census[g] = (uint8_t)((cur <= 1) ? (0x80u | (org ? 2u : 0u) | (uint32_t)cur) : (uint32_t)(cur > 127 ? 127 : cur));
+                if (lane == 0) p.census[g] = census_after_step(cur, org);
                 if (p.live_mask) {
                     const bool al = (live >> lane) & 1u;
                     const uint32_t lo = __reduce_or_sync(0xffffffffu, (al && myslot < 32) ? (1u << myslot) : 0u);
@@ -693,7 +686,7 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
                     const bool dn = cnt < 2;
                     if (lane == 0) {
                         if (p.done) p.done[(long long)st * p.B + g] = dn ? 1 : 0;
-                        if (p.reward) p.reward[(long long)st * p.B + g] = (kflags & HK_F_ROLE_AGENT) ? -0.0f : 0.0f;
+                        if (p.reward) p.reward[(long long)st * p.B + g] = rest_reward(kflags);
                         if constexpr (REC) {
                             const long long o = (long long)st * p.B + g;
                             if (p.host_mask_t) p.host_mask_t[o] = 0;
@@ -1024,10 +1017,7 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
             if (lane == 0) {
                 if (p.done) p.done[(long long)st * p.B + g] = dn ? 1 : 0;
                 if (CENSUS && p.done_bits && dn) atomicOr(p.done_bits + (g >> 5), 1u << (g & 31));
-                if (p.reward) {
-                    float rw = (dn && !prev_done) ? 1.0f : 0.0f;
-                    p.reward[(long long)st * p.B + g] = (kflags & HK_F_ROLE_AGENT) ? -rw : rw;
-                }
+                if (p.reward) p.reward[(long long)st * p.B + g] = step_reward(kflags, dn, prev_done);
             }
             if (p.done_count && dn) count_done(st);
             if (dn && !prev_done) len = st + 1;
@@ -1061,8 +1051,7 @@ __global__ void __launch_bounds__(256, HK_GENERIC_MIN_CTAS) hk_generic_kernel(co
                 }
             }
             const bool org = !__any_sync(0xffffffffu, moving);
-            if (lane == 0)
-                p.census[g] = (uint8_t)((cnt <= 1) ? (0x80u | (org ? 2u : 0u) | (uint32_t)cnt) : (uint32_t)(cnt > 127 ? 127 : cnt));
+            if (lane == 0) p.census[g] = census_after_step(cnt, org);
             if (p.live_mask)
                 store_mask(g, __ballot_sync(0xffffffffu, mylive & 1u), __ballot_sync(0xffffffffu, (mylive >> 1) & 1u));
         }

@@ -44,7 +44,7 @@ int kernel_ctas_per_sm(K kernel, KernelFacts& facts, int dev, int threads, size_
     return v;
 }
 
-inline bool is_small_shape(int N, int d) { return d == 3 && (N == 20 || N == 10 || N == 5); }
+__host__ __device__ constexpr bool is_small_shape(int N, int d) { return d == 3 && (N == 20 || N == 10 || N == 5); }
 
 // one-launch paths of the two kernel families, one instantiation per (dtype, variant) in the hk_small_*.cu and
 // hk_generic_*.cu units (hk_small_launch.inl, hk_generic_launch.inl)
@@ -86,6 +86,6 @@ extern template int dispatch_sched<float, true>(const StepParams&, int, cudaStre
 extern template int dispatch_rows<int32_t>(const StepParams&, int, cudaStream_t);
 extern template int dispatch_rows<float>(const StepParams&, int, cudaStream_t);
 constexpr int ROWS_K = 8;  // = ROWS_MAX_K of hk_rows.cuh
-inline bool rows_shape(int N, int d) { return N <= 64 && d >= 2 && d <= 5; }
+__host__ __device__ constexpr bool rows_shape(int N, int d) { return N <= 64 && d >= 2 && d <= 5; }
 
 }  // namespace hk

@@ -15,7 +15,7 @@
 // live count is at most ROWS_MAX_K (and answers the games at rest from their census byte), the warp-per-game
 // kernel then takes the rest and skips what was done here.
 #pragma once
-#include "hk_launch.cuh"
+#include "hk_census.cuh"
 #include "hk_small.cuh"
 
 namespace hk {
@@ -32,9 +32,6 @@ struct RowsLayout {
     static constexpr int WARP_WORDS = STAGES * STAGE_WORDS + CLS_WORDS + ORDER_WORDS;
     static constexpr size_t SMEM_BYTES = (size_t)WARPS * WARP_WORDS * 4;
 };
-
-// live count a census byte stands for (valid for known bytes)
-__device__ __forceinline__ int census_count(uint32_t v) { return (v & 0x80u) ? (int)(v & 1u) : (int)v; }
 
 // K compact rows of one game per lane: gather order = slot order, so the lowest-slot-wins rule of the dedupe holds
 template <typename T, int D, int K>
@@ -99,8 +96,8 @@ __global__ void __launch_bounds__(WARPS * 32) hk_rows_kernel(const StepParams p)
     const long long nw = (long long)gridDim.x * WARPS;
     uint32_t* gst = reinterpret_cast<uint32_t*>(p.out);
     const uint32_t lt = (1u << lane) - 1u;
-    const bool frozen_rest = (p.flags & HK_F_FREEZE_ENDED) && !(p.ops & (HK_OP_REPOSITION | HK_OP_RESCALE));
-    const float rest_reward = (p.flags & HK_F_ROLE_AGENT) ? -0.0f : 0.0f;
+    const bool frozen_rest = census_frozen_rest(p.ops, p.flags);
+    const float rest_r = rest_reward(p.flags);
     int done_total = 0;
 
     // a warp owns a contiguous run of games, scheduled in rounds of RG games (a multiple of 32, at most
@@ -135,19 +132,15 @@ __global__ void __launch_bounds__(WARPS * 32) hk_rows_kernel(const StepParams p)
         for (int o = lane; o < ((ng + 31) & ~31); o += 32) {
             const bool valid = o < ng;
             const uint32_t v = valid ? (uint32_t)clsb[o] : 0u;
-            const bool rest = valid && (v & 0x80u) && ((v & 2u) || frozen_rest);
+            const bool rest = valid && census_at_rest(v, frozen_rest);
             const long long g = g0 + o;
-            if (rest) {
-                if (p.done) p.done[g] = 1;
-                if (p.reward) p.reward[g] = rest_reward;
-                if (p.num_points) p.num_points[g] = (int32_t)(v & 1u);
-            }
+            if (rest) write_rest_outputs(p, g, v, rest_r);
             const uint32_t restmask = __ballot_sync(0xffffffffu, rest);
             done_total += __popc(restmask);
             // the tile's word of the done mask: games at rest now; games that finish in this step are ORed in later
             // (by this kernel or by the warp-per-game launch that follows)
             if (p.done_bits && lane == 0) p.done_bits[g >> 5] = restmask;
-            const int cnt = census_count(v);
+            const int cnt = (int)census_live_count(v);
             const int c = (!valid || rest || v == 0 || cnt > ROWS_MAX_K) ? 0 : (cnt <= 2 ? 1 : (cnt <= 4 ? 2 : 3));
             if (valid) clsb[o] = (uint8_t)(c ? (c | (cnt << 2)) : 0);  // class in the low 2 bits, live count above
             classes |= 1u << c;
@@ -231,13 +224,10 @@ __global__ void __launch_bounds__(WARPS * 32) hk_rows_kernel(const StepParams p)
             const bool dn = ncnt < 2;
             if (cur.valid) {
                 if (p.done) p.done[cur.g] = dn ? 1 : 0;
-                if (p.reward) {
-                    const float r = (dn && !prev_done) ? 1.0f : 0.0f;
-                    p.reward[cur.g] = (p.flags & HK_F_ROLE_AGENT) ? -r : r;
-                }
+                if (p.reward) p.reward[cur.g] = step_reward(p.flags, dn, prev_done);
                 if (p.num_points) p.num_points[cur.g] = ncnt;
                 if (p.done_bits && dn) atomicOr(p.done_bits + (cur.g >> 5), 1u << (cur.g & 31));
-                p.census[cur.g] = (uint8_t)(dn ? (0x80u | (origin ? 2u : 0u) | (uint32_t)ncnt) : (uint32_t)ncnt);
+                p.census[cur.g] = census_after_step(ncnt, origin);
                 if (nmask != cur.mask) p.live_mask[cur.g] = nmask;
             }
             done_total += __popc(__ballot_sync(0xffffffffu, cur.valid && dn));

@@ -15,10 +15,9 @@
 //     processed by the same per-game code as the tile-ring kernel (small_process_tile).
 // Work and DRAM traffic follow the number of games still in play instead of the batch size.
 //
-// Census byte (HK census, include/hironaka_b200.h): 0 = unknown (the game is read and counted);
-// 1..127 = live rows of a game in play; 0x80 | c | (o ? 2 : 0) = ended game with c <= 1 live rows, dead rows
-// normalised, o = at rest for every op (no row, or the lone row at the origin).
+// The census byte is defined in hk_census.cuh.
 #pragma once
+#include "hk_census.cuh"
 #include "hk_small.cuh"
 
 namespace hk {
@@ -64,20 +63,25 @@ __device__ __forceinline__ uint32_t nonzero_bytes4(uint32_t x) {
 // Class codes of four census bytes (the class array's format): class 0 = at rest or no such game; 1..6 = the tier
 // class of a game in play (6 for an unknown byte, 1 for "ended, not at rest under this launch's ops" and for 1-2
 // live rows, else 1 + [v > 2] + [v > 4] + [v > 8] + [v > 12] + [v > 16]); 0x80 = at rest; 0x40 = its live count.
-// vmask keeps the bytes of games that exist; rest7 returns the at-rest flags (bit 7 of each byte).
+// vmask keeps the bytes of games that exist; rest7 returns the at-rest flags (bit 7 of each byte): census_at_rest of
+// each byte, four at a time.
 __device__ __forceinline__ uint32_t census_codes4(uint32_t w, uint32_t vmask, bool frozen_rest, uint32_t& rest7) {
+    constexpr uint32_t BYTES4 = 0x01010101u;                   // times a byte value: that value in each byte
+    constexpr uint32_t ENDED4 = CENSUS_ENDED * BYTES4;         // the ended bit of each byte
+    constexpr uint32_t LOW4 = (~CENSUS_ENDED & 0xffu) * BYTES4;  // the bits below it: a live count in play
+    static_assert(CENSUS_AT_ORIGIN << 6 == CENSUS_ENDED, "the at-origin bit is shifted onto the ended bit");
     w &= vmask;
-    const uint32_t ended = w & 0x80808080u;
-    rest7 = ended & ((w << 6) | (frozen_rest ? 0x80808080u : 0u)) & vmask;  // ended and (bit 1 or frozen)
-    const uint32_t x7 = w & 0x7f7f7f7fu;
+    const uint32_t ended = w & ENDED4;
+    rest7 = ended & ((w << 6) | (frozen_rest ? ENDED4 : 0u)) & vmask;  // ended and (at origin or frozen)
+    const uint32_t x7 = w & LOW4;
     uint32_t c = 0x01010101u + (bytes_ge7(x7, 3) >> 7) + (bytes_ge7(x7, 5) >> 7) + (bytes_ge7(x7, 9) >> 7) +
                  (bytes_ge7(x7, 13) >> 7) + (bytes_ge7(x7, 17) >> 7);
-    const uint32_t unknown = ~(bytes_ge7(x7, 1) | ended) & 0x80808080u;  // a zero byte
+    const uint32_t unknown = ~(bytes_ge7(x7, 1) | ended) & ENDED4;  // a zero byte
     c += (unknown >> 7) * 5u;
     const uint32_t endedff = (ended >> 7) * 0xffu;
     c = (c & ~endedff) | (ended >> 7);
     c &= vmask & ~((rest7 >> 7) * 0xffu);
-    return c | rest7 | ((w & 0x01010101u) << 6);
+    return c | rest7 | ((w & BYTES4) << 6);  // bit 0 of each byte (the live count of an ended game) at 0x40
 }
 
 // Per-lane counts of the classes 1..6 of four class codes, packed in 10-bit fields: classes 1-3 in lo, 4-6 in hi.
@@ -128,10 +132,8 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) hk_sched_kernel(const StepPa
     __syncwarp();
     uint32_t phase_bits = 0;  // bit s = parity to wait for on stage s
     const uint32_t lt = (1u << lane) - 1u;
-    // at rest under THIS launch: nothing to do for an origin / empty game; a frozen ended game also rests when
-    // neither reposition nor rescale would move its lone point
-    const bool frozen_rest = (p.flags & HK_F_FREEZE_ENDED) && !(p.ops & (HK_OP_REPOSITION | HK_OP_RESCALE));
-    const float rest_reward = (p.flags & HK_F_ROLE_AGENT) ? -0.0f : 0.0f;
+    const bool frozen_rest = census_frozen_rest(p.ops, p.flags);
+    const float rest_r = rest_reward(p.flags);
     // piece lane -> (game slot within the instruction, piece within the game)
     const int sub = lane / LPG, piece = lane - sub * LPG;
     int settled_total = 0;  // per lane: games at rest
@@ -200,12 +202,12 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) hk_sched_kernel(const StepPa
                     const bool whole = left >= 4;
                     const uint32_t live = w & 0x01010101u;
                     if (whole && done4) *reinterpret_cast<uint32_t*>(p.done + g0) = rest7 >> 7;
-                    if (whole && reward16) *reinterpret_cast<float4*>(p.reward + g0) = make_float4(rest_reward, rest_reward, rest_reward, rest_reward);
+                    if (whole && reward16) *reinterpret_cast<float4*>(p.reward + g0) = make_float4(rest_r, rest_r, rest_r, rest_r);
                     if (whole && npoints16) *reinterpret_cast<int4*>(p.num_points + g0) = make_int4((int)(live & 1u), (int)((live >> 8) & 1u), (int)((live >> 16) & 1u), (int)(live >> 24));
                     for (uint32_t m = rest7; m; m &= m - 1) {  // otherwise one store per game at rest
                         const int b = (__ffs((int)m) - 1) >> 3;
                         if (p.done && !(whole && done4)) p.done[g0 + b] = 1;
-                        if (p.reward && !(whole && reward16)) p.reward[g0 + b] = rest_reward;
+                        if (p.reward && !(whole && reward16)) p.reward[g0 + b] = rest_r;
                         if (p.num_points && !(whole && npoints16)) p.num_points[g0 + b] = (int32_t)((live >> (8 * b)) & 1u);
                     }
                 }
@@ -385,11 +387,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) hk_sched_kernel(const StepPa
             const uint32_t code = clsb[k * 32 + lane];
             const bool rest = code & 0x80u;
             const uint32_t v = (code >> 6) & 1u;  // live count of a game at rest
-            if (rest) {
-                if (p.done) p.done[g] = 1;
-                if (p.reward) p.reward[g] = rest_reward;
-                if (p.num_points) p.num_points[g] = (int32_t)v;
-            }
+            if (rest) write_rest_outputs(p, g, v, rest_r);
             const uint32_t restmask = __ballot_sync(0xffffffffu, rest);
             if constexpr (OBS) {
                 // (warp-uniform) the constant observation of every game at rest of this tile — unless the tile is about to
@@ -497,9 +495,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) hk_sched_kernel(const StepPa
             if (ls.valid) {
                 if (p.num_points) p.num_points[ls.g] = ls.cnt;
                 if (p.done_bits && ls.cnt < 2) atomicOr(p.done_bits + (ls.g >> 5), 1u << (ls.g & 31));
-                const uint32_t nv = (ls.cnt <= 1) ? (0x80u | (ls.origin ? 2u : 0u) | (uint32_t)ls.cnt)
-                                                  : (uint32_t)(ls.cnt > 127 ? 127 : ls.cnt);
-                p.census[ls.g] = (uint8_t)nv;
+                p.census[ls.g] = census_after_step(ls.cnt, ls.origin);
             }
             if (p.exceed_flag) {
                 if (__any_sync(0xffffffffu, exceed && ls.valid) && lane == 0) *p.exceed_flag = 1;
@@ -510,27 +506,8 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) hk_sched_kernel(const StepPa
                     float* orow = obs_tile + lane * OW;
                     bulk_wait_read<0>();  // the previous chunk's observation stores have read the tile
                     __syncwarp();
-                    {
-                        T z[W];
-                        load_game<T, W>(row, z);
-                        if constexpr (Elem<T>::is_float) {
-#pragma unroll
-                            for (int q = 0; q < W; ++q) z[q] = z[q] + 0.0f;
-                        }
-                        const uint32_t zl = live_mask<T, N, D>(z);
-                        const int zmax = __reduce_max_sync(0xffffffffu, ingrid ? __popc(zl) : 0);
-                        bool built = false;
-                        if constexpr (D <= 6) built = features_network<T, N, D>(z, zl, zmax, p.flags, p.pad, orow);
-                        if (!built) {
-                            const int gpow = (OW & -OW) > 32 ? 32 : (OW & -OW);
-                            features_rolled<T, N, D>(row, zl, zmax, p.flags, p.pad, orow, (lane * gpow) >> 5);
-                        }
-                    }
-                    if (p.obs_coord) {
-                        const uint32_t ocm = ingrid ? action_mask(load_action(p.obs_coord, ls.g, p.flags), p.flags) : 0u;
-#pragma unroll
-                        for (int k = 0; k < D; ++k) orow[W + k] = (float)((ocm >> k) & 1u);
-                    }
+                    lane_features<T, N, D>(p, row, orow, OW, lane, ingrid);
+                    append_obs_coord<D>(p, ls.g, ingrid, orow, W);
                     if (natural) {  // the tile's observations are contiguous
                         const long long first = ls.g - lane;
                         const int cnt = (int)((B - first < 32) ? (B - first) : 32);

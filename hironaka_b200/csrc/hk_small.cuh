@@ -492,10 +492,7 @@ __device__ __forceinline__ int tier_steps(const StepParams& p, LaneState& ls, ui
         const bool dn = ls.cnt < 2;
         if (ls.valid) {
             if (p.done) p.done[(long long)st * B + ls.g] = dn ? 1 : 0;
-            if (p.reward) {
-                float r = (dn && !prev_done) ? 1.0f : 0.0f;
-                p.reward[(long long)st * B + ls.g] = (p.flags & HK_F_ROLE_AGENT) ? -r : r;
-            }
+            if (p.reward) p.reward[(long long)st * B + ls.g] = step_reward(p.flags, dn, prev_done);
         }
         if (p.done_count) {
             const int c = __popc(__ballot_sync(0xffffffffu, ls.valid && dn));
@@ -739,10 +736,7 @@ __device__ __forceinline__ bool tier_packed(const StepParams& p, LaneState& ls, 
     const bool prev_done = cnt0 < 2, dn = cnt < 2;
     if (ls.valid) {
         if (p.done) p.done[(long long)st * p.B + ls.g] = dn ? 1 : 0;
-        if (p.reward) {
-            const float r = (dn && !prev_done) ? 1.0f : 0.0f;
-            p.reward[(long long)st * p.B + ls.g] = (p.flags & HK_F_ROLE_AGENT) ? -r : r;
-        }
+        if (p.reward) p.reward[(long long)st * p.B + ls.g] = step_reward(p.flags, dn, prev_done);
     }
     if (p.done_count) {
         const int c = __popc(__ballot_sync(0xffffffffu, ls.valid && dn));
@@ -1303,6 +1297,41 @@ __device__ __forceinline__ bool small_process_tile(const StepParams& p, LaneStat
     return false;
 }
 
+// ---- a lane's observation row ---------------------------------------------------------------------
+// Features of the game in the lane's row of the stage into orow (row stride OW words).  Every warp takes the same
+// route whatever its live counts (sorting network; the rolled routine only when values do not pack): per-tier variants
+// made the warps of an SM execute different code and the kernels instruction-fetch bound.  holds_game: the lane's row
+// is a game of the batch (the others do not count towards the warp's largest live count).
+template <typename T, int N, int D>
+__device__ __forceinline__ void lane_features(const StepParams& p, const uint32_t* row, float* orow, int OW, int lane,
+                                              const bool& holds_game) {
+    constexpr int W = N * D;
+    T z[W];
+    load_game<T, W>(row, z);
+    if constexpr (Elem<T>::is_float) {
+#pragma unroll
+        for (int q = 0; q < W; ++q) z[q] = z[q] + 0.0f;
+    }
+    const uint32_t zl = live_mask<T, N, D>(z);
+    const int zmax = __reduce_max_sync(0xffffffffu, holds_game ? __popc(zl) : 0);
+    bool built = false;
+    if constexpr (D <= 6) built = features_network<T, N, D>(z, zl, zmax, p.flags, p.pad, orow);
+    if (!built) {
+        // rows of stride OW words: lanes 32/g apart share a bank (g = largest power of two in OW)
+        const int gpow = (OW & -OW) > 32 ? 32 : (OW & -OW);
+        features_rolled<T, N, D>(row, zl, zmax, p.flags, p.pad, orow, (lane * gpow) >> 5);
+    }
+}
+
+// the coordinates p.obs_coord names for game g, as D floats 0/1 after the W feature words
+template <int D>
+__device__ __forceinline__ void append_obs_coord(const StepParams& p, long long g, const bool& holds_game, float* orow, int W) {
+    if (!p.obs_coord) return;
+    const uint32_t ocm = holds_game ? action_mask(load_action(p.obs_coord, g, p.flags), p.flags) : 0u;
+#pragma unroll
+    for (int k = 0; k < D; ++k) orow[W + k] = (float)((ocm >> k) & 1u);
+}
+
 // ---- tile movement -------------------------------------------------------------------------------
 __device__ __forceinline__ void warp_copy_words(uint32_t* dst, const uint32_t* src, int words, int lane) {
     for (int w = lane; w < words; w += 32) dst[w] = src[w];
@@ -1410,20 +1439,7 @@ __device__ __forceinline__ void small_kernel_body(const StepParams& p) {
                     if (p.obs_t == nullptr) return;
                     if (lane == 0) bulk_wait_read<0>();  // the previous row's store has read the obs tile
                     __syncwarp();
-                    T z[W];
-                    load_game<T, W>(row, z);
-                    if constexpr (Elem<T>::is_float) {
-#pragma unroll
-                        for (int q = 0; q < W; ++q) z[q] = z[q] + 0.0f;
-                    }
-                    const uint32_t zl = live_mask<T, N, D>(z);
-                    const int zmax = __reduce_max_sync(0xffffffffu, ls.valid ? __popc(zl) : 0);
-                    bool built = false;
-                    if constexpr (D <= 6) built = features_network<T, N, D>(z, zl, zmax, p.flags, p.pad, orow);
-                    if (!built) {
-                        const int gpow = (OW & -OW) > 32 ? 32 : (OW & -OW);
-                        features_rolled<T, N, D>(row, zl, zmax, p.flags, p.pad, orow, (lane * gpow) >> 5);
-                    }
+                    lane_features<T, N, D>(p, row, orow, OW, lane, ls.valid);
                     return;
                 }
                 if (ls.valid) {
@@ -1510,32 +1526,10 @@ __device__ __forceinline__ void small_kernel_body(const StepParams& p) {
         }
         if constexpr (OBS) {
             if (p.obs) {
-                {
-                    T z[W];
-                    load_game<T, W>(row, z);  // the new state, survivors scattered back to their slots
-                    if constexpr (Elem<T>::is_float) {
-#pragma unroll
-                        for (int q = 0; q < W; ++q) z[q] = z[q] + 0.0f;
-                    }
-                    const uint32_t zl = live_mask<T, N, D>(z);
-                    const int zmax = __reduce_max_sync(0xffffffffu, ls.valid ? __popc(zl) : 0);
-                    // Observation features of the FINAL state of the tile, as a phase of its own after the
-                    // steps.  Every warp takes the same route here whatever its live counts (sorting
-                    // network; the rolled routine only when values do not pack): per-tier variants made
-                    // the warps of an SM execute different code and the kernel instruction-fetch bound.
-                    bool built = false;
-                    if constexpr (D <= 6) built = features_network<T, N, D>(z, zl, zmax, p.flags, p.pad, orow);
-                    if (!built) {
-                        // rows of stride OW words: lanes 32/g apart share a bank (g = largest power of two in OW)
-                        const int gpow = (OW & -OW) > 32 ? 32 : (OW & -OW);
-                        features_rolled<T, N, D>(row, zl, zmax, p.flags, p.pad, orow, (lane * gpow) >> 5);
-                    }
-                }
-                if (p.obs_coord) {
-                    const uint32_t ocm = ls.valid ? action_mask(load_action(p.obs_coord, ls.g, p.flags), p.flags) : 0u;
-#pragma unroll
-                    for (int k = 0; k < D; ++k) orow[W + k] = (float)((ocm >> k) & 1u);
-                }
+                // Observation features of the FINAL state of the tile (survivors scattered back to their slots), as a
+                // phase of its own after the steps
+                lane_features<T, N, D>(p, row, orow, OW, lane, ls.valid);
+                append_obs_coord<D>(p, ls.g, ls.valid, orow, W);
                 const int owords = (words / W) * OW;
                 float* gobs = p.obs + t * 32ll * OW;
                 if (obs_tma && ((owords & 3) == 0)) {
