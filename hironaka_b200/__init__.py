@@ -10,6 +10,7 @@ Layers (bottom up):
   GameBatch        resident int32 batches, fused T-step rollouts, sharding + rollout all-gather
   HostSession      NumPy host-buffer sessions over hk_session_*
   VecHironaka*Env  batched forms of the gym environments (hironaka/gym_env)
+  search_depth     game-tree search of a fixed host against every agent reply (hironaka/util/search.py)
 """
 from . import constants
 from .constants import *  # noqa: F401,F403
@@ -40,10 +41,15 @@ def __getattr__(name):  # lazy: importing the package must not require torch or 
     if name in ("VecHironakaAgentEnv", "VecHironakaHostEnv"):
         from . import vec_env
         return getattr(vec_env, name)
+    if name in ("search_depth", "SearchResult", "STATUS_RESOLVED", "STATUS_MAX_DEPTH", "STATUS_MAX_NODES",
+                "STATUS_CAPACITY", "STATUS_INT32_BOUND"):
+        from . import search
+        return getattr(search, name)
     if name == "HostActionEncoder":
         from .host_action import HostActionEncoder
         return HostActionEncoder
-    if name in ("ops", "src", "functional", "engine", "session", "host_action", "build", "fused_game", "players", "replay_buffer", "vec_env"):
+    if name in ("ops", "src", "functional", "engine", "session", "host_action", "build", "fused_game", "players", "replay_buffer", "vec_env",
+                "search"):
         import importlib
         return importlib.import_module(f".{name}", __name__)
     raise AttributeError(f"module {__name__!r} has no attribute {name!r}")

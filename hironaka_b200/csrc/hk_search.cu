@@ -1,0 +1,154 @@
+// hk_search.cu — hk_search_workspace_bytes and hk_search_depth (include/hironaka_b200.h): the level loop of the game-tree
+// search.  Every level runs hk_host_policy on the frontier, the three bookkeeping kernels of hk_search.cuh, and hk_step
+// in place on the children, through the same C-ABI entry points a caller would use, so the children are bit for bit
+// what hk_step makes of them on either kernel family.
+#include <cuda_runtime.h>
+
+#include <cstring>
+
+#include "../../include/hironaka_b200.h"
+#include "hk_search.cuh"
+
+namespace {
+
+size_t align_up(size_t v) { return (v + 255) & ~(size_t)255; }
+
+// the caller's workspace, cut into 256-byte aligned pieces (the order of hk_search_workspace_bytes)
+struct SearchWorkspace {
+    int32_t* frontier[2];  // [capacity, N, d] each
+    int32_t* node_root[2]; // [capacity]
+    int32_t* child_mask;   // [capacity]
+    int32_t* child_axis;   // [capacity]
+    int32_t* policy;       // [max(B, capacity)]
+    uint8_t* count;        // [max(B, capacity)]
+    long long* tile_sum;   // [ceil(max(B, capacity) / SEARCH_THREADS)]
+    unsigned long long* root_children;  // [B]
+    int32_t* root_flag;    // [B]
+    long long* root_shift; // [B]
+    int32_t* active[2];    // [B] each
+    long long* counters;   // [2]
+};
+
+size_t carve(SearchWorkspace* w, char* base, long long B, int N, int d, long long capacity) {
+    const long long P = B > capacity ? B : capacity;
+    size_t off = 0;
+    auto take = [&](size_t bytes) {
+        char* ptr = base ? base + off : nullptr;
+        off += align_up(bytes);
+        return ptr;
+    };
+    for (int k = 0; k < 2; ++k) w->frontier[k] = (int32_t*)take((size_t)capacity * N * d * 4);
+    for (int k = 0; k < 2; ++k) w->node_root[k] = (int32_t*)take((size_t)capacity * 4);
+    w->child_mask = (int32_t*)take((size_t)capacity * 4);
+    w->child_axis = (int32_t*)take((size_t)capacity * 4);
+    w->policy = (int32_t*)take((size_t)P * 4);
+    w->count = (uint8_t*)take((size_t)P);
+    w->tile_sum = (long long*)take((size_t)((P + hk::SEARCH_THREADS - 1) / hk::SEARCH_THREADS) * 8);
+    w->root_children = (unsigned long long*)take((size_t)B * 8);
+    w->root_flag = (int32_t*)take((size_t)B * 4);
+    w->root_shift = (long long*)take((size_t)B * 8);
+    for (int k = 0; k < 2; ++k) w->active[k] = (int32_t*)take((size_t)B * 4);
+    w->counters = (long long*)take(16);
+    return off;
+}
+
+}  // namespace
+
+extern "C" {
+
+int64_t hk_search_workspace_bytes(int64_t B, int32_t N, int32_t d, int64_t capacity) {
+    if (B < 0 || N < 1 || d < 1 || capacity < 1) return 0;
+    SearchWorkspace w;
+    return (int64_t)(carve(&w, nullptr, B, N, d, capacity) + 256);  // + 256: room to align the caller's pointer
+}
+
+int hk_search_depth(const void* roots, int32_t* depth, int64_t* nodes, int8_t* status, int64_t B, int32_t N, int32_t d,
+                    int32_t dtype, uint32_t ops, uint32_t flags, int32_t max_depth, int64_t max_nodes, int64_t capacity,
+                    void* workspace, void* stream) {
+    if (B < 0 || N < 1 || d < 1 || (dtype != HK_DTYPE_I32 && dtype != HK_DTYPE_F32)) return HK_ERR_BAD_ARG;
+    if (hk_kernel_class(N, d) < 0) return HK_ERR_UNSUPPORTED;
+    if (dtype != HK_DTYPE_I32) return HK_ERR_UNSUPPORTED;  // float32 state is not searched
+    if (flags != HK_F_HOST_ZEILLINGER && flags != HK_F_HOST_ALL_COORD) return HK_ERR_BAD_ARG;
+    if ((ops & (HK_OP_SHIFT | HK_OP_NEWTON)) != (HK_OP_SHIFT | HK_OP_NEWTON) ||
+        (ops & ~(HK_OP_SHIFT | HK_OP_NEWTON | HK_OP_REPOSITION)))
+        return HK_ERR_BAD_ARG;
+    if (max_depth < 1 || max_nodes < 1 || capacity < 1) return HK_ERR_BAD_ARG;
+    if (B == 0) return HK_OK;
+    if (!roots || !depth || !nodes || !status || !workspace) return HK_ERR_BAD_ARG;
+    if (((uintptr_t)roots) & 3u) return HK_ERR_ALIGN;
+    cudaStream_t st = (cudaStream_t)stream;
+    SearchWorkspace w;
+    carve(&w, (char*)align_up((size_t)(uintptr_t)workspace), B, N, d, capacity);
+
+    cudaError_t e = cudaMemsetAsync(w.root_children, 0, (size_t)B * 8, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(w.root_flag, 0, (size_t)B * 4, st);
+    if (e != cudaSuccess) return (int)e;
+    {
+        const long long blocks = (B + 255) / 256;
+        hk::hk_search_init_kernel<<<(unsigned)(blocks > 4096 ? 4096 : blocks), 256, 0, st>>>(depth, (long long*)nodes, status,
+                                                                                            w.active[0], B);
+    }
+
+    hk::SearchParams p;
+    memset(&p, 0, sizeof(p));
+    p.N = N;
+    p.d = d;
+    p.bound = (int32_t)((1 << 30) / d);
+    p.max_nodes = max_nodes;
+    p.capacity = capacity;
+    p.policy = w.policy;
+    p.count = w.count;
+    p.tile_sum = w.tile_sum;
+    p.root_children = w.root_children;
+    p.root_flag = w.root_flag;
+    p.root_shift = w.root_shift;
+    p.counters = w.counters;
+    p.depth = depth;
+    p.nodes = (long long*)nodes;
+    p.status = status;
+    p.child_mask = w.child_mask;
+    p.child_axis = w.child_axis;
+
+    const int32_t* state = (const int32_t*)roots;
+    const int32_t* node_root = nullptr;  // level 0: node i is root i
+    long long M = B, n_active = B;
+    for (int level = 0;; ++level) {
+        const int next = level & 1;  // frontier, node-root list and root list the next level is written to
+        p.state = state;
+        p.node_root = node_root;
+        p.M = M;
+        p.level = level;
+        p.expand = level < max_depth;
+        p.active = w.active[level & 1];
+        p.active_next = w.active[(level + 1) & 1];
+        p.n_active = n_active;
+        p.child_state = w.frontier[next];
+        p.child_root = w.node_root[next];
+        if (p.expand) {
+            int rc = hk_host_policy(state, w.policy, M, N, d, HK_DTYPE_I32, flags, -1.0f, stream);
+            if (rc != HK_OK) return rc;
+        }
+        const unsigned tiles = (unsigned)((M + hk::SEARCH_THREADS - 1) / hk::SEARCH_THREADS);
+        hk::hk_search_count_kernel<<<tiles, hk::SEARCH_THREADS, 0, st>>>(p);
+        hk::hk_search_decide_kernel<<<1, hk::SEARCH_SCAN_THREADS, 0, st>>>(p);
+        long long counters[2];
+        e = cudaGetLastError();
+        if (e == cudaSuccess) e = cudaMemcpyAsync(counters, w.counters, sizeof(counters), cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+        if (e != cudaSuccess) return (int)e;
+        if (!p.expand || counters[0] == 0) break;
+        hk::hk_search_scatter_kernel<<<tiles, hk::SEARCH_THREADS, 0, st>>>(p);
+        e = cudaGetLastError();
+        if (e != cudaSuccess) return (int)e;
+        int rc = hk_step(w.frontier[next], w.frontier[next], w.child_mask, w.child_axis, nullptr, nullptr, nullptr, nullptr,
+                         nullptr, nullptr, counters[0], N, d, HK_DTYPE_I32, ops, 0, -1.0f, 1e8f, stream);
+        if (rc != HK_OK) return rc;
+        state = w.frontier[next];
+        node_root = w.node_root[next];
+        M = counters[0];
+        n_active = counters[1];
+    }
+    return (int)cudaGetLastError();
+}
+
+}  // extern "C"

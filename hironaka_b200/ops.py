@@ -380,6 +380,36 @@ def host_policy(state: torch.Tensor, host: str, padding_value: float = -1.0) -> 
     return mask
 
 
+def search_workspace_bytes(B: int, N: int, d: int, capacity: int) -> int:
+    """Bytes of device workspace `search_depth` needs (hk_search_workspace_bytes)."""
+    return int(lib().hk_search_workspace_bytes(B, N, d, capacity))
+
+
+def search_depth(roots: torch.Tensor, *, flags: int, ops: int, max_depth: int, max_nodes: int, capacity: int,
+                 workspace: Optional[torch.Tensor] = None):
+    """Game-tree search of a fixed host against every agent reply (hk_search_depth): (depth [B] int32, nodes [B]
+    int64, status [B] int8).  `flags` is HK_F_HOST_ZEILLINGER or HK_F_HOST_ALL_COORD, `ops` HK_OP_SHIFT | HK_OP_NEWTON
+    (| HK_OP_REPOSITION).  `workspace` is a uint8 tensor of at least search_workspace_bytes(B, N, d, capacity) bytes on
+    the roots' device (allocated here when None).  Synchronous: the call returns when the search is over."""
+    dt = _require_state(roots)
+    B, N, d = roots.shape
+    dev = roots.device
+    need = search_workspace_bytes(B, N, d, capacity)
+    if workspace is None:
+        workspace = torch.empty(max(need, 1), dtype=torch.uint8, device=dev)
+    elif workspace.dtype != torch.uint8 or workspace.numel() < need or workspace.device != dev:
+        raise ValueError(f"workspace must be a uint8 tensor of at least {need} bytes on the roots' device")
+    depth = torch.empty(B, dtype=torch.int32, device=dev)
+    nodes = torch.empty(B, dtype=torch.int64, device=dev)
+    status = torch.empty(B, dtype=torch.int8, device=dev)
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        rc = lib().hk_search_depth(_ptr(roots), _ptr(depth), _ptr(nodes), _ptr(status), B, N, d, dt, ops, flags,
+                                   int(max_depth), int(max_nodes), int(capacity), _ptr(workspace), stream)
+    check(rc, "hk_search_depth")
+    return depth, nodes, status
+
+
 def _single_op(fn_name: str, state: torch.Tensor, inplace: bool, padding_value: float) -> Optional[torch.Tensor]:
     dt = _require_state(state)
     B, N, d = state.shape

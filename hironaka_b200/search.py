@@ -1,0 +1,62 @@
+"""Game-tree search of a fixed host: how long can an adversarial agent make each game last?
+
+The batched form of search_depth (hironaka/util/search.py), which explores every agent reply to one host strategy
+recursively on one ListPoints game.  Here every root of a batch is searched at once, level by level on the GPU
+(hk_search_depth, include/hironaka_b200.h), with explicit limits: a depth limit, a node budget per root and a
+frontier capacity.  A root that hits a limit is a normal result, reported in `status`.
+"""
+from __future__ import annotations
+
+from typing import NamedTuple, Optional
+
+import torch
+
+from . import constants as C
+from . import ops as _ops
+
+STATUS_RESOLVED = C.HK_SEARCH_RESOLVED        # every line of play has ended
+STATUS_MAX_DEPTH = C.HK_SEARCH_MAX_DEPTH      # states at level max_depth have not ended
+STATUS_MAX_NODES = C.HK_SEARCH_MAX_NODES      # the next level would take the root past max_nodes
+STATUS_CAPACITY = C.HK_SEARCH_CAPACITY        # the next level of the batch did not fit in the frontier capacity
+STATUS_INT32_BOUND = C.HK_SEARCH_INT32_BOUND  # a state to expand has an entry >= 2^30 / d: its children would be inexact
+
+FRONTIER_BYTES = 1 << 28  # default capacity: one frontier fills 256 MiB
+
+
+class SearchResult(NamedTuple):
+    depth: torch.Tensor   # [B] int32 height of the explored tree (a lower bound unless status == STATUS_RESOLVED)
+    nodes: torch.Tensor   # [B] int64 states in the explored tree, root and ended leaves included
+    status: torch.Tensor  # [B] int8 STATUS_*
+
+
+def default_capacity(N: int, d: int) -> int:
+    """Frontier capacity used when none is given: FRONTIER_BYTES / (N * d * 4) nodes."""
+    return max(1, FRONTIER_BYTES // (N * d * 4))
+
+
+def search_depth(points: torch.Tensor, host: str = "zeillinger", *, reposition: bool = True, max_depth: int = 64,
+                 max_nodes: int = 1 << 16, capacity: Optional[int] = None) -> SearchResult:
+    """For each root of `points` (int32 [B, N, d] on a CUDA device, taken as given: pass
+    GameBatch(..., initial_filter=True).points for filtered roots), the longest game an agent can force against the
+    fixed `host` ("zeillinger" or "all_coord"), found by trying every agent reply.
+
+    A state with at most one live row has ended.  Any other state at level k is expanded: the host chooses its
+    coordinate set S, and each axis in S (in increasing order) gives one child at level k + 1, the state after the JAX
+    step (shift, reposition if `reposition`, Newton polytope).  Equal states are not merged.
+
+    Limits: `max_depth` levels below the root; `max_nodes` states per root (the level that would pass it is not
+    added); `capacity` states in one level of the whole batch (when the next level does not fit, roots are dropped from
+    the highest index down until it does).  The default capacity is default_capacity(N, d) = 2^28 / (N * d * 4)
+    states: the search keeps two frontiers of N * d * 4 bytes per state, so 512 MiB for both, plus a few words per state
+    and per root.  Only STATUS_CAPACITY depends on the capacity and on the other roots of the batch.
+
+    The call is synchronous (the number of states of each level is read back to size the next)."""
+    if host not in ("zeillinger", "all_coord"):
+        raise ValueError(f"host must be 'zeillinger' or 'all_coord'; got {host!r}")
+    B, N, d = points.shape
+    flags = C.HK_F_HOST_ZEILLINGER if host == "zeillinger" else C.HK_F_HOST_ALL_COORD
+    step_ops = C.HK_OP_SHIFT | C.HK_OP_NEWTON | (C.HK_OP_REPOSITION if reposition else 0)
+    cap = default_capacity(N, d) if capacity is None else int(capacity)
+    depth, nodes, status = _ops.search_depth(points, flags=flags, ops=step_ops, max_depth=max_depth,
+                                             max_nodes=max_nodes, capacity=cap)
+    return SearchResult(depth, nodes, status)

@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define HK_VERSION 102 /* major*100 + minor */
+#define HK_VERSION 103 /* major*100 + minor */
 
 /* ---- status codes ---------------------------------------------------------------- */
 #define HK_OK 0
@@ -212,6 +212,41 @@ int hk_dones(const void* state_in, uint8_t* done, int32_t* num_points, int64_t B
  * hironaka/gym_env/hironaka_host_env.py:62-66). */
 int hk_host_policy(const void* state_in, int32_t* coord_mask, int64_t B, int32_t N, int32_t d, int32_t dtype,
                    uint32_t flags, float padding_value, void* stream);
+
+/* ---- game-tree search of a fixed host ------------------------------------------------------
+ * How long can an adversarial agent make the game last against a fixed host?  The batched, level-by-level form of
+ * search_depth (hironaka/util/search.py): every agent reply is explored, every limit is explicit.
+ * For each root b of roots [B,N,d] (int32 state, taken as given: filter it first if you want filtered roots):
+ *   - a node is a state; it is ENDED when it has <= 1 live row (hk_step's done rule);
+ *   - a node at level k that has not ended is expanded: S = hk_host_policy(node) with flags (exactly one of
+ *     HK_F_HOST_ZEILLINGER, HK_F_HOST_ALL_COORD), and each axis a in S, in increasing order, gives one child at level
+ *     k + 1: hk_step of the node with coordinate bitmask S and axis a, ops (HK_OP_SHIFT | HK_OP_NEWTON, optionally
+ *     HK_OP_REPOSITION) and the JAX flags (0); padding -1;
+ *   - equal states are not merged and cycles are not detected: a state reached twice is counted twice.
+ * Outputs per root:
+ *   depth  [B] int32: height of the explored tree, 0 for an ended root; for a cut root a lower bound (its deepest level)
+ *   nodes  [B] int64: states in the explored tree, the root and the ended leaves included, cut levels not
+ *   status [B] int8 HK_SEARCH_*: RESOLVED; MAX_DEPTH (nodes at level max_depth have not ended); MAX_NODES (adding the
+ *          next level would take the root past max_nodes; the level is not added); CAPACITY (the next level of all
+ *          roots does not fit in `capacity` nodes: the roots are dropped from the highest index down until it fits);
+ *          INT32_BOUND (a node to expand has a live entry >= floor(2^30 / d): its children would not be exact).
+ *          At one level the checks apply in the order INT32_BOUND, MAX_NODES, CAPACITY.  A cut root has no later levels.
+ * The results do not depend on the launch geometry or on the other roots of the batch, except through CAPACITY.
+ * workspace: hk_search_workspace_bytes(B, N, d, capacity) bytes of device memory owned by the caller: two frontiers of
+ * `capacity` nodes (N*d*4 bytes each) and O(B + capacity) words of bookkeeping; the call allocates nothing.
+ * The call is SYNCHRONOUS: after every level it reads two counters back to the host (to size the next level's launches
+ * and to stop when no node is left), so it is not graph-capturable.
+ * Errors: float32 state HK_ERR_UNSUPPORTED; other flags, ops without HK_OP_SHIFT | HK_OP_NEWTON or with
+ * HK_OP_RESCALE / HK_OP_DEDUPE, max_depth < 1, max_nodes < 1, capacity < 1: HK_ERR_BAD_ARG. */
+#define HK_SEARCH_RESOLVED 0
+#define HK_SEARCH_MAX_DEPTH 1
+#define HK_SEARCH_MAX_NODES 2
+#define HK_SEARCH_CAPACITY 3
+#define HK_SEARCH_INT32_BOUND 4
+int64_t hk_search_workspace_bytes(int64_t B, int32_t N, int32_t d, int64_t capacity);
+int hk_search_depth(const void* roots, int32_t* depth, int64_t* nodes, int8_t* status, int64_t B, int32_t N, int32_t d,
+                    int32_t dtype, uint32_t ops, uint32_t flags, int32_t max_depth, int64_t max_nodes, int64_t capacity,
+                    void* workspace, void* stream);
 
 /* ---- multi-step rollout ------------------------------------------------------------------
  * T consecutive steps with the state held on chip between steps: one read and one write of
