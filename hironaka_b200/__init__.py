@@ -11,6 +11,7 @@ Layers (bottom up):
   HostSession      NumPy host-buffer sessions over hk_session_*
   VecHironaka*Env  batched forms of the gym environments (hironaka/gym_env)
   search_depth     game-tree search of a fixed host against every agent reply (hironaka/util/search.py)
+  search_value     game value: the shortest game the best host can force against every agent reply
 """
 from . import constants
 from .constants import *  # noqa: F401,F403
@@ -42,7 +43,7 @@ def __getattr__(name):  # lazy: importing the package must not require torch or 
         from . import vec_env
         return getattr(vec_env, name)
     if name in ("search_depth", "SearchResult", "STATUS_RESOLVED", "STATUS_MAX_DEPTH", "STATUS_MAX_NODES",
-                "STATUS_CAPACITY", "STATUS_INT32_BOUND"):
+                "STATUS_CAPACITY", "STATUS_INT32_BOUND", "search_value", "ValueResult", "STATUS_HISTORY"):
         from . import search
         return getattr(search, name)
     if name == "HostActionEncoder":

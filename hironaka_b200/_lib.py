@@ -48,6 +48,8 @@ SIGNATURES = {
                                             _u32, _u32, _f32, ctypes.c_uint64, _i32, _f32, _i32, _p, _p]),
     "hk_search_workspace_bytes": (_i64, [_i64, _i32, _i32, _i64]),
     "hk_search_depth": (ctypes.c_int, [_p, _p, _p, _p, _i64, _i32, _i32, _i32, _u32, _u32, _i32, _i64, _i64, _p, _p]),
+    "hk_search_value_workspace_bytes": (_i64, [_i64, _i32, _i32, _i64, _i64]),
+    "hk_search_value": (ctypes.c_int, [_p, _p, _p, _p, _p, _i64, _i32, _i32, _i32, _u32, _i32, _i64, _i64, _i64, _p, _p]),
     "hk_experience_scratch_words": (_i64, [_i64]),
     "hk_experience_append": (ctypes.c_int, [_p, _p, _p, _i32, _p, _p, _i32, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _p, _p,
                                             _p, _p, _i64, _p]),

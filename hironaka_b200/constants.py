@@ -1,7 +1,7 @@
 """Constants of the C-ABI (mirror of include/hironaka_b200.h; tests/test_capi_cpu.py checks
 that the two stay identical)."""
 
-HK_VERSION = 103
+HK_VERSION = 104
 
 HK_OK = 0
 HK_ERR_BAD_ARG = -1
@@ -41,12 +41,13 @@ HK_F_ACT_NIBBLE = 1 << 16
 HK_F_HOST_RANDOM = 1 << 17
 HK_F_AGENT_RANDOM = 1 << 18
 
-# status of a root after hk_search_depth
+# status of a root after hk_search_depth and hk_search_value (HISTORY: hk_search_value only)
 HK_SEARCH_RESOLVED = 0
 HK_SEARCH_MAX_DEPTH = 1
 HK_SEARCH_MAX_NODES = 2
 HK_SEARCH_CAPACITY = 3
 HK_SEARCH_INT32_BOUND = 4
+HK_SEARCH_HISTORY = 5
 
 # the two semantics of the reference
 TORCH_SEMANTICS = HK_F_NOOP_INVALID | HK_F_FREEZE_ENDED  # hironaka/src/_torch_ops.py:90-93

@@ -1,12 +1,14 @@
-// hk_search.cu — hk_search_workspace_bytes and hk_search_depth (include/hironaka_b200.h): the level loop of the game-tree
-// search.  Every level runs hk_host_policy on the frontier, the three bookkeeping kernels of hk_search.cuh, and hk_step
-// in place on the children, through the same C-ABI entry points a caller would use, so the children are bit for bit
-// what hk_step makes of them on either kernel family.
+// hk_search.cu — hk_search_workspace_bytes and hk_search_depth, hk_search_value_workspace_bytes and hk_search_value
+// (include/hironaka_b200.h): the level loops of the game-tree searches.  Every level of hk_search_depth runs
+// hk_host_policy on the frontier and the three bookkeeping kernels of hk_search.cuh; every level of hk_search_value runs
+// the four kernels of hk_minimax.cuh.  Both then run hk_step in place on the children, through the same C-ABI entry
+// point a caller would use, so the children are bit for bit what hk_step makes of them on either kernel family.
 #include <cuda_runtime.h>
 
 #include <cstring>
 
 #include "../../include/hironaka_b200.h"
+#include "hk_minimax.cuh"
 #include "hk_search.cuh"
 
 namespace {
@@ -50,6 +52,60 @@ size_t carve(SearchWorkspace* w, char* base, long long B, int N, int d, long lon
     for (int k = 0; k < 2; ++k) w->active[k] = (int32_t*)take((size_t)B * 4);
     w->counters = (long long*)take(16);
     return off;
+}
+
+// the workspace of hk_search_value (the order of hk_search_value_workspace_bytes)
+struct ValueWorkspace {
+    int32_t* frontier[2];  // [capacity, N, d] each
+    int32_t* node_root[2]; // [capacity]
+    int32_t* child_mask;   // [capacity]
+    int32_t* child_axis;   // [capacity]
+    uint8_t* kind;         // [max(B, capacity)]
+    uint8_t* count;        // [max(B, capacity)]
+    long long* tile_sum;   // [ceil(max(B, capacity) / SEARCH_THREADS)]
+    unsigned long long* root_children;  // [B]
+    int32_t* root_flag;    // [B]
+    long long* root_shift; // [B]
+    int32_t* active[2];    // [B] each
+    long long* counters;   // [2]
+    int32_t* h_parent;     // [history] each
+    int32_t* h_solved;
+    int32_t* h_rem;
+    uint8_t* h_mask;
+    uint8_t* h_rank;
+};
+
+size_t carve_value(ValueWorkspace* w, char* base, long long B, int N, int d, long long capacity, long long history) {
+    const long long P = B > capacity ? B : capacity;
+    size_t off = 0;
+    auto take = [&](size_t bytes) {
+        char* ptr = base ? base + off : nullptr;
+        off += align_up(bytes);
+        return ptr;
+    };
+    for (int k = 0; k < 2; ++k) w->frontier[k] = (int32_t*)take((size_t)capacity * N * d * 4);
+    for (int k = 0; k < 2; ++k) w->node_root[k] = (int32_t*)take((size_t)capacity * 4);
+    w->child_mask = (int32_t*)take((size_t)capacity * 4);
+    w->child_axis = (int32_t*)take((size_t)capacity * 4);
+    w->kind = (uint8_t*)take((size_t)P);
+    w->count = (uint8_t*)take((size_t)P);
+    w->tile_sum = (long long*)take((size_t)((P + hk::SEARCH_THREADS - 1) / hk::SEARCH_THREADS) * 8);
+    w->root_children = (unsigned long long*)take((size_t)B * 8);
+    w->root_flag = (int32_t*)take((size_t)B * 4);
+    w->root_shift = (long long*)take((size_t)B * 8);
+    for (int k = 0; k < 2; ++k) w->active[k] = (int32_t*)take((size_t)B * 4);
+    w->counters = (long long*)take(16);
+    w->h_parent = (int32_t*)take((size_t)history * 4);
+    w->h_solved = (int32_t*)take((size_t)history * 4);
+    w->h_rem = (int32_t*)take((size_t)history * 4);
+    w->h_mask = (uint8_t*)take((size_t)history);
+    w->h_rank = (uint8_t*)take((size_t)history);
+    return off;
+}
+
+bool value_args_ok(long long B, int N, int d, long long capacity, long long history) {
+    return B >= 0 && N >= 1 && d >= 2 && d <= 6 && capacity >= 1 && history >= 1 && history >= B &&
+           history <= 0x7fffffffll;
 }
 
 }  // namespace
@@ -149,6 +205,117 @@ int hk_search_depth(const void* roots, int32_t* depth, int64_t* nodes, int8_t* s
         n_active = counters[1];
     }
     return (int)cudaGetLastError();
+}
+
+int64_t hk_search_value_workspace_bytes(int64_t B, int32_t N, int32_t d, int64_t capacity, int64_t history) {
+    if (!value_args_ok(B, N, d, capacity, history)) return 0;
+    ValueWorkspace w;
+    return (int64_t)(carve_value(&w, nullptr, B, N, d, capacity, history) + 256);  // + 256: room to align the pointer
+}
+
+int hk_search_value(const void* roots, int32_t* value, int32_t* best_mask, int64_t* nodes, int8_t* status, int64_t B,
+                    int32_t N, int32_t d, int32_t dtype, uint32_t ops, int32_t max_depth, int64_t max_nodes,
+                    int64_t capacity, int64_t history, void* workspace, void* stream) {
+    if (B < 0 || N < 1 || d < 1 || (dtype != HK_DTYPE_I32 && dtype != HK_DTYPE_F32)) return HK_ERR_BAD_ARG;
+    if (hk_kernel_class(N, d) < 0 || d < 2 || d > 6) return HK_ERR_UNSUPPORTED;  // <= 186 children: a uint8 count
+    if (dtype != HK_DTYPE_I32) return HK_ERR_UNSUPPORTED;  // float32 state is not searched
+    if ((ops & (HK_OP_SHIFT | HK_OP_NEWTON)) != (HK_OP_SHIFT | HK_OP_NEWTON) ||
+        (ops & ~(HK_OP_SHIFT | HK_OP_NEWTON | HK_OP_REPOSITION)))
+        return HK_ERR_BAD_ARG;
+    if (max_depth < 1 || max_nodes < 1 || !value_args_ok(B, N, d, capacity, history)) return HK_ERR_BAD_ARG;
+    if (B == 0) return HK_OK;
+    if (!roots || !value || !best_mask || !nodes || !status || !workspace) return HK_ERR_BAD_ARG;
+    if (((uintptr_t)roots) & 3u) return HK_ERR_ALIGN;
+    cudaStream_t st = (cudaStream_t)stream;
+    ValueWorkspace w;
+    carve_value(&w, (char*)align_up((size_t)(uintptr_t)workspace), B, N, d, capacity, history);
+
+    static_assert(sizeof(hk::ValueParams) <= 4096, "ValueParams is passed by value to every kernel");
+    hk::ValueParams p;
+    memset(&p, 0, sizeof(p));
+    p.B = B;
+    p.N = N;
+    p.d = d;
+    p.bound = (int32_t)((1 << 30) / d);
+    p.max_nodes = max_nodes;
+    p.capacity = capacity;
+    p.history = history;
+    // the children of an expanded node: S over the sets with |S| >= 2 in increasing order, the axes of S in order
+    for (int S = 0; S < (1 << d); ++S) {
+        if (__builtin_popcount((unsigned)S) < 2) continue;
+        int rank = 0;
+        for (int a = 0; a < d; ++a)
+            if (S >> a & 1) p.pair[p.children++] = (uint16_t)(S | a << 6 | rank++ << 9);
+    }
+    p.kind = w.kind;
+    p.count = w.count;
+    p.tile_sum = w.tile_sum;
+    p.root_children = w.root_children;
+    p.root_flag = w.root_flag;
+    p.root_shift = w.root_shift;
+    p.counters = w.counters;
+    p.value = value;
+    p.best_mask = best_mask;
+    p.nodes = (long long*)nodes;
+    p.status = status;
+    p.h_parent = w.h_parent;
+    p.h_solved = w.h_solved;
+    p.h_rem = w.h_rem;
+    p.h_mask = w.h_mask;
+    p.h_rank = w.h_rank;
+    p.child_mask = w.child_mask;
+    p.child_axis = w.child_axis;
+
+    cudaError_t e = cudaMemsetAsync(w.root_children, 0, (size_t)B * 8, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(w.root_flag, 0, (size_t)B * 4, st);
+    if (e != cudaSuccess) return (int)e;
+    const long long root_blocks = (B + 255) / 256;
+    const unsigned root_grid = (unsigned)(root_blocks > 4096 ? 4096 : root_blocks);
+    hk::hk_value_init_kernel<<<root_grid, 256, 0, st>>>(p, w.active[0]);
+
+    const int32_t* state = (const int32_t*)roots;
+    const int32_t* node_root = nullptr;  // level 0: node i is root i
+    long long M = B, n_active = B, hist_base = 0;
+    for (int level = 0;; ++level) {
+        const int next = level & 1;  // frontier, node-root list and root list the next level is written to
+        p.state = state;
+        p.node_root = node_root;
+        p.M = M;
+        p.level = level;
+        p.expand = level < max_depth;
+        p.hist_base = hist_base;
+        p.hist_used = hist_base + M;
+        p.active = w.active[level & 1];
+        p.active_next = w.active[(level + 1) & 1];
+        p.n_active = n_active;
+        p.child_state = w.frontier[next];
+        p.child_root = w.node_root[next];
+        const unsigned tiles = (unsigned)((M + hk::SEARCH_THREADS - 1) / hk::SEARCH_THREADS);
+        hk::hk_value_solve_kernel<<<tiles, hk::SEARCH_THREADS, 0, st>>>(p);
+        hk::hk_value_count_kernel<<<tiles, hk::SEARCH_THREADS, 0, st>>>(p);
+        hk::hk_value_decide_kernel<<<1, hk::SEARCH_SCAN_THREADS, 0, st>>>(p);
+        long long counters[2];
+        e = cudaGetLastError();
+        if (e == cudaSuccess) e = cudaMemcpyAsync(counters, w.counters, sizeof(counters), cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+        if (e != cudaSuccess) return (int)e;
+        if (!p.expand || counters[0] == 0) break;
+        hk::hk_value_scatter_kernel<<<tiles, hk::SEARCH_THREADS, 0, st>>>(p);
+        e = cudaGetLastError();
+        if (e != cudaSuccess) return (int)e;
+        int rc = hk_step(w.frontier[next], w.frontier[next], w.child_mask, w.child_axis, nullptr, nullptr, nullptr, nullptr,
+                         nullptr, nullptr, counters[0], N, d, HK_DTYPE_I32, ops, 0, -1.0f, 1e8f, stream);
+        if (rc != HK_OK) return rc;
+        state = w.frontier[next];
+        node_root = w.node_root[next];
+        hist_base += M;
+        M = counters[0];
+        n_active = counters[1];
+    }
+    hk::hk_value_finish_kernel<<<root_grid, 256, 0, st>>>(p);
+    e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    return (int)e;
 }
 
 }  // extern "C"

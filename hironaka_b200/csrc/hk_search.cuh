@@ -144,21 +144,27 @@ __device__ __forceinline__ long long search_block_scan(long long v, long long* w
     return excl;
 }
 
+// exclusive scan in place of the tile sums of a frontier of M nodes: the raw position (before any cut) of each tile's
+// first child.  Every thread of a SEARCH_SCAN_THREADS block calls it.
+__device__ __forceinline__ void search_scan_tiles(long long* tile_sum, long long M, long long* ws) {
+    const long long tiles = (M + SEARCH_THREADS - 1) / SEARCH_THREADS;
+    long long carry = 0;
+    for (long long start = 0; start < tiles; start += SEARCH_SCAN_THREADS) {
+        const long long t = start + threadIdx.x;
+        const long long v = t < tiles ? tile_sum[t] : 0;
+        long long tot;
+        const long long ex = search_block_scan(v, ws, &tot);
+        if (t < tiles) tile_sum[t] = carry + ex;
+        carry += tot;
+    }
+}
+
 __global__ void __launch_bounds__(SEARCH_SCAN_THREADS) hk_search_decide_kernel(const SearchParams p) {
     __shared__ long long ws[32];
     __shared__ unsigned long long kept_total;
     if (threadIdx.x == 0) kept_total = 0;
-    // 1. exclusive scan of the tile sums: the raw position (before any cut) of each tile's first child
-    const long long tiles = (p.M + SEARCH_THREADS - 1) / SEARCH_THREADS;
-    long long carry = 0;
-    for (long long start = 0; start < tiles; start += SEARCH_SCAN_THREADS) {
-        const long long t = start + threadIdx.x;
-        const long long v = t < tiles ? p.tile_sum[t] : 0;
-        long long tot;
-        const long long ex = search_block_scan(v, ws, &tot);
-        if (t < tiles) p.tile_sum[t] = carry + ex;
-        carry += tot;
-    }
+    // 1. the raw position of each tile's first child
+    search_scan_tiles(p.tile_sum, p.M, ws);
     // 2. the roots in play, in increasing order: cuts int32 bound -> node budget -> capacity
     long long raw_carry = 0, kept_carry = 0, next_carry = 0;
     for (long long start = 0; start < p.n_active; start += SEARCH_SCAN_THREADS) {

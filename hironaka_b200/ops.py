@@ -410,6 +410,38 @@ def search_depth(roots: torch.Tensor, *, flags: int, ops: int, max_depth: int, m
     return depth, nodes, status
 
 
+def search_value_workspace_bytes(B: int, N: int, d: int, capacity: int, history: int) -> int:
+    """Bytes of device workspace `search_value` needs (hk_search_value_workspace_bytes; 0 for refused arguments)."""
+    return int(lib().hk_search_value_workspace_bytes(B, N, d, capacity, history))
+
+
+def search_value(roots: torch.Tensor, *, ops: int, max_depth: int, max_nodes: int, capacity: int, history: int,
+                 workspace: Optional[torch.Tensor] = None):
+    """Game value by minimax search over the host's choices (hk_search_value): (value [B] int32, best_mask [B] int32,
+    nodes [B] int64, status [B] int8).  `ops` is HK_OP_SHIFT | HK_OP_NEWTON (| HK_OP_REPOSITION).  `workspace` is a
+    uint8 tensor of at least search_value_workspace_bytes(B, N, d, capacity, history) bytes on the roots' device
+    (allocated here when None).  Synchronous: the call returns when the search is over."""
+    dt = _require_state(roots)
+    B, N, d = roots.shape
+    dev = roots.device
+    need = search_value_workspace_bytes(B, N, d, capacity, history)
+    if workspace is None:
+        workspace = torch.empty(max(need, 1), dtype=torch.uint8, device=dev)
+    elif workspace.dtype != torch.uint8 or workspace.numel() < need or workspace.device != dev:
+        raise ValueError(f"workspace must be a uint8 tensor of at least {need} bytes on the roots' device")
+    value = torch.empty(B, dtype=torch.int32, device=dev)
+    best_mask = torch.empty(B, dtype=torch.int32, device=dev)
+    nodes = torch.empty(B, dtype=torch.int64, device=dev)
+    status = torch.empty(B, dtype=torch.int8, device=dev)
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        rc = lib().hk_search_value(_ptr(roots), _ptr(value), _ptr(best_mask), _ptr(nodes), _ptr(status), B, N, d, dt,
+                                   ops, int(max_depth), int(max_nodes), int(capacity), int(history), _ptr(workspace),
+                                   stream)
+    check(rc, "hk_search_value")
+    return value, best_mask, nodes, status
+
+
 def _single_op(fn_name: str, state: torch.Tensor, inplace: bool, padding_value: float) -> Optional[torch.Tensor]:
     dt = _require_state(state)
     B, N, d = state.shape

@@ -4,6 +4,9 @@ The batched form of search_depth (hironaka/util/search.py), which explores every
 recursively on one ListPoints game.  Here every root of a batch is searched at once, level by level on the GPU
 (hk_search_depth, include/hironaka_b200.h), with explicit limits: a depth limit, a node budget per root and a
 frontier capacity.  A root that hits a limit is a normal result, reported in `status`.
+
+search_value (hk_search_value) answers the minimax question over the same tree with every host move: the fewest moves
+the best host needs to end the game, whatever the agent replies.
 """
 from __future__ import annotations
 
@@ -19,8 +22,11 @@ STATUS_MAX_DEPTH = C.HK_SEARCH_MAX_DEPTH      # states at level max_depth have n
 STATUS_MAX_NODES = C.HK_SEARCH_MAX_NODES      # the next level would take the root past max_nodes
 STATUS_CAPACITY = C.HK_SEARCH_CAPACITY        # the next level of the batch did not fit in the frontier capacity
 STATUS_INT32_BOUND = C.HK_SEARCH_INT32_BOUND  # a state to expand has an entry >= 2^30 / d: its children would be inexact
+STATUS_HISTORY = C.HK_SEARCH_HISTORY          # search_value: the next level did not fit in the batch's history
 
 FRONTIER_BYTES = 1 << 28  # default capacity: one frontier fills 256 MiB
+HISTORY_BYTES = 1 << 32   # search_value's default history: 4 GiB
+HISTORY_NODE_BYTES = 14   # parent, solved round and group count (int32 each), group set and rank (one byte each)
 
 
 class SearchResult(NamedTuple):
@@ -60,3 +66,45 @@ def search_depth(points: torch.Tensor, host: str = "zeillinger", *, reposition: 
     depth, nodes, status = _ops.search_depth(points, flags=flags, ops=step_ops, max_depth=max_depth,
                                              max_nodes=max_nodes, capacity=cap)
     return SearchResult(depth, nodes, status)
+
+
+class ValueResult(NamedTuple):
+    value: torch.Tensor      # [B] int32 game value (a strict lower bound minus one unless status == STATUS_RESOLVED)
+    best_mask: torch.Tensor  # [B] int32 the host's first move in an optimal line; 0 for an ended root, -1 unresolved
+    nodes: torch.Tensor      # [B] int64 states in the explored tree, root and ended leaves included
+    status: torch.Tensor     # [B] int8 STATUS_*
+
+
+def default_history() -> int:
+    """History used when none is given: HISTORY_BYTES / HISTORY_NODE_BYTES nodes."""
+    return HISTORY_BYTES // HISTORY_NODE_BYTES
+
+
+def search_value(points: torch.Tensor, *, reposition: bool = True, max_depth: int = 16, max_nodes: int = 1 << 22,
+                 capacity: Optional[int] = None, history: Optional[int] = None) -> ValueResult:
+    """For each root of `points` (int32 [B, N, d] on a CUDA device, 2 <= d <= 6, taken as given), the game value: the
+    fewest moves the best host needs to end the game, whatever the agent replies.
+
+    A state with at most one live row has ended (value 0).  Any other state is expanded into one child per host move
+    and agent reply: every coordinate set S with |S| >= 2 in increasing bitmask order, and each axis of S in
+    increasing order, the JAX step (shift, reposition if `reposition`, Newton polytope).  The children of one S form a
+    group.  After each level L is built, its ended states are solved; a group is won when all its children are solved
+    and a state is solved when its first group is won, up to the root.  A state at level l solved then has value L - l,
+    and `best_mask` of a root is the smallest S won in that round.  Only open states with no solved ancestor are
+    expanded.
+
+    Limits, as search_depth's: `max_depth` levels, `max_nodes` states per root, `capacity` states in one level of the
+    batch, the int32 bound; and `history`, the states of all levels of the batch, roots included, which the search keeps
+    to walk up from solved states (STATUS_HISTORY when the next level would not fit; roots are dropped from the highest
+    index down).  A root with another status has `value` = the last level checked, and its true value is larger.
+
+    Memory: the defaults are capacity = default_capacity(N, d) = 2^28 / (N * d * 4) states, two frontiers of 256 MiB,
+    and history = default_history() = 2^32 / 14 states at 14 bytes each, 4 GiB; plus a few words per frontier state
+    and per root.  The call is synchronous."""
+    B, N, d = points.shape
+    step_ops = C.HK_OP_SHIFT | C.HK_OP_NEWTON | (C.HK_OP_REPOSITION if reposition else 0)
+    cap = default_capacity(N, d) if capacity is None else int(capacity)
+    hist = default_history() if history is None else int(history)
+    value, best_mask, nodes, status = _ops.search_value(points, ops=step_ops, max_depth=max_depth, max_nodes=max_nodes,
+                                                        capacity=cap, history=hist)
+    return ValueResult(value, best_mask, nodes, status)

@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define HK_VERSION 103 /* major*100 + minor */
+#define HK_VERSION 104 /* major*100 + minor */
 
 /* ---- status codes ---------------------------------------------------------------- */
 #define HK_OK 0
@@ -247,6 +247,42 @@ int64_t hk_search_workspace_bytes(int64_t B, int32_t N, int32_t d, int64_t capac
 int hk_search_depth(const void* roots, int32_t* depth, int64_t* nodes, int8_t* status, int64_t B, int32_t N, int32_t d,
                     int32_t dtype, uint32_t ops, uint32_t flags, int32_t max_depth, int64_t max_nodes, int64_t capacity,
                     void* workspace, void* stream);
+
+/* ---- game value: minimax over the host's choices -----------------------------------------------
+ * How few moves does the best host need to end the game, whatever the agent replies?  For each root b of roots [B,N,d]
+ * (int32 state, taken as given, 2 <= d <= 6), level by level with the limits of hk_search_depth:
+ *   - a node with <= 1 live row has ENDED; its value is 0;
+ *   - an open node is expanded into one child per (S, axis): S over every coordinate set with |S| >= 2 in increasing
+ *     bitmask order, the axis over the members of S in increasing order; the child is hk_step of the node with bitmask S
+ *     and that axis, ops as for hk_search_depth, the JAX flags (0), padding -1.  The children of one S form a GROUP.
+ *     d*2^(d-1) - d children: 2, 9, 28, 75 or 186;
+ *   - after level L is built (round L): every ended node of level L is solved; a group is won when all its children
+ *     are solved; a node is solved when its first group is won, up to the root in the same round.  A node of level l
+ *     solved in round L has value L - l (the rounds go in level order, so this first value is the minimum);
+ *   - a node is expanded only if it is open, not solved and has no solved ancestor;
+ *   - limits: max_depth, max_nodes per root, `capacity` nodes per level of the whole batch, the int32 bound
+ *     (floor(2^30 / d)), and `history`: the nodes of every level of the whole batch, roots included, which the search
+ *     keeps to walk up from solved nodes.  At one level the cuts apply in the order INT32_BOUND, MAX_NODES, CAPACITY,
+ *     HISTORY; the last two drop roots from the highest index down.
+ * Outputs per root:
+ *   value     [B] int32: the game value when status is RESOLVED; otherwise the last level whose round was done for the
+ *             root, and the value is strictly larger
+ *   best_mask [B] int32: the smallest S among the root's groups won in the round that solved it, 0 for a root that has
+ *             ended, -1 when not RESOLVED
+ *   nodes     [B] int64: states in the explored tree, the root included (as hk_search_depth)
+ *   status    [B] int8 HK_SEARCH_*: RESOLVED, MAX_DEPTH, MAX_NODES, CAPACITY, INT32_BOUND as for hk_search_depth, or
+ *             HISTORY (the next level would take the batch's history past `history` nodes; it is not added).
+ * The results do not depend on the launch geometry or on the other roots of the batch, except through CAPACITY and
+ * HISTORY.  workspace: hk_search_value_workspace_bytes(B, N, d, capacity, history) bytes of device memory owned by
+ * the caller: two frontiers of `capacity` nodes (N*d*4 bytes each), 14 bytes per history node and O(B + capacity)
+ * words of bookkeeping; it returns 0 for arguments hk_search_value refuses.  SYNCHRONOUS, as hk_search_depth.
+ * Errors: float32 state, d outside 2..6: HK_ERR_UNSUPPORTED; ops as for hk_search_depth, max_depth < 1,
+ * max_nodes < 1, capacity < 1, history < max(B, 1) or history > 2^31 - 1: HK_ERR_BAD_ARG. */
+#define HK_SEARCH_HISTORY 5
+int64_t hk_search_value_workspace_bytes(int64_t B, int32_t N, int32_t d, int64_t capacity, int64_t history);
+int hk_search_value(const void* roots, int32_t* value, int32_t* best_mask, int64_t* nodes, int8_t* status, int64_t B,
+                    int32_t N, int32_t d, int32_t dtype, uint32_t ops, int32_t max_depth, int64_t max_nodes,
+                    int64_t capacity, int64_t history, void* workspace, void* stream);
 
 /* ---- multi-step rollout ------------------------------------------------------------------
  * T consecutive steps with the state held on chip between steps: one read and one write of
