@@ -1,13 +1,16 @@
-// hk_search.cu — hk_search_workspace_bytes and hk_search_depth, hk_search_value_workspace_bytes and hk_search_value
+// hk_search.cu — hk_search_workspace_bytes and hk_search_depth, hk_search_value_workspace_bytes and hk_search_value,
+// and their line forms hk_search_depth_line_workspace_bytes, hk_search_depth_line and hk_search_value_line
 // (include/hironaka_b200.h): the level loops of the game-tree searches.  Every level of hk_search_depth runs
 // hk_host_policy on the frontier and the three bookkeeping kernels of hk_search.cuh; every level of hk_search_value runs
 // the four kernels of hk_minimax.cuh.  Both then run hk_step in place on the children, through the same C-ABI entry
-// point a caller would use, so the children are bit for bit what hk_step makes of them on either kernel family.
+// point a caller would use, so the children are bit for bit what hk_step makes of them on either kernel family.  The
+// line forms run the same loops plus the kernels of hk_lines.cuh.
 #include <cuda_runtime.h>
 
 #include <cstring>
 
 #include "../../include/hironaka_b200.h"
+#include "hk_lines.cuh"
 #include "hk_minimax.cuh"
 #include "hk_search.cuh"
 
@@ -108,42 +111,56 @@ bool value_args_ok(long long B, int N, int d, long long capacity, long long hist
            history <= 0x7fffffffll;
 }
 
-}  // namespace
+// the workspace of hk_search_depth_line: hk_search_depth's, then the line history (the order of
+// hk_search_depth_line_workspace_bytes)
+struct DepthLineWorkspace {
+    SearchWorkspace s;
+    int32_t* h_parent;  // [history]
+    uint16_t* h_set;    // [history]
+    uint8_t* h_axis;    // [history]
+    int32_t* deep;      // [B]
+    long long* root_ch; // [B]
+};
 
-extern "C" {
-
-int64_t hk_search_workspace_bytes(int64_t B, int32_t N, int32_t d, int64_t capacity) {
-    if (B < 0 || N < 1 || d < 1 || capacity < 1) return 0;
-    SearchWorkspace w;
-    return (int64_t)(carve(&w, nullptr, B, N, d, capacity) + 256);  // + 256: room to align the caller's pointer
+size_t carve_depth_line(DepthLineWorkspace* w, char* base, long long B, int N, int d, long long capacity,
+                        long long history) {
+    size_t off = carve(&w->s, base, B, N, d, capacity);
+    auto take = [&](size_t bytes) {
+        char* ptr = base ? base + off : nullptr;
+        off += align_up(bytes);
+        return ptr;
+    };
+    w->h_parent = (int32_t*)take((size_t)history * 4);
+    w->h_set = (uint16_t*)take((size_t)history * 2);
+    w->h_axis = (uint8_t*)take((size_t)history);
+    w->deep = (int32_t*)take((size_t)B * 4);
+    w->root_ch = (long long*)take((size_t)B * 8);
+    return off;
 }
 
-int hk_search_depth(const void* roots, int32_t* depth, int64_t* nodes, int8_t* status, int64_t B, int32_t N, int32_t d,
-                    int32_t dtype, uint32_t ops, uint32_t flags, int32_t max_depth, int64_t max_nodes, int64_t capacity,
-                    void* workspace, void* stream) {
-    if (B < 0 || N < 1 || d < 1 || (dtype != HK_DTYPE_I32 && dtype != HK_DTYPE_F32)) return HK_ERR_BAD_ARG;
-    if (hk_kernel_class(N, d) < 0) return HK_ERR_UNSUPPORTED;
-    if (dtype != HK_DTYPE_I32) return HK_ERR_UNSUPPORTED;  // float32 state is not searched
-    if (flags != HK_F_HOST_ZEILLINGER && flags != HK_F_HOST_ALL_COORD) return HK_ERR_BAD_ARG;
-    if ((ops & (HK_OP_SHIFT | HK_OP_NEWTON)) != (HK_OP_SHIFT | HK_OP_NEWTON) ||
-        (ops & ~(HK_OP_SHIFT | HK_OP_NEWTON | HK_OP_REPOSITION)))
-        return HK_ERR_BAD_ARG;
-    if (max_depth < 1 || max_nodes < 1 || capacity < 1) return HK_ERR_BAD_ARG;
-    if (B == 0) return HK_OK;
-    if (!roots || !depth || !nodes || !status || !workspace) return HK_ERR_BAD_ARG;
-    if (((uintptr_t)roots) & 3u) return HK_ERR_ALIGN;
-    cudaStream_t st = (cudaStream_t)stream;
-    SearchWorkspace w;
-    carve(&w, (char*)align_up((size_t)(uintptr_t)workspace), B, N, d, capacity);
+bool depth_line_args_ok(long long B, int N, int d, long long capacity, long long history) {
+    return B >= 0 && N >= 1 && d >= 1 && capacity >= 1 && history >= 1 && history >= B && history <= 0x7fffffffll;
+}
 
+// what the depth line adds to hk_search_depth's level loop; nullptr for hk_search_depth itself
+struct DepthLine {
+    DepthLineWorkspace w;
+    long long history;
+    int32_t* line_mask;  // [B, max_depth]
+    int32_t* line_axis;  // [B, max_depth]
+};
+
+int run_search_depth(const void* roots, int32_t* depth, int64_t* nodes, int8_t* status, int64_t B, int32_t N,
+                     int32_t d, uint32_t ops, uint32_t flags, int32_t max_depth, int64_t max_nodes, int64_t capacity,
+                     const SearchWorkspace& w, DepthLine* line, void* stream) {
+    cudaStream_t st = (cudaStream_t)stream;
     cudaError_t e = cudaMemsetAsync(w.root_children, 0, (size_t)B * 8, st);
     if (e == cudaSuccess) e = cudaMemsetAsync(w.root_flag, 0, (size_t)B * 4, st);
+    if (e == cudaSuccess && line) e = cudaMemsetAsync(line->w.h_parent, 0xff, (size_t)B * 4, st);  // roots: parent -1
     if (e != cudaSuccess) return (int)e;
-    {
-        const long long blocks = (B + 255) / 256;
-        hk::hk_search_init_kernel<<<(unsigned)(blocks > 4096 ? 4096 : blocks), 256, 0, st>>>(depth, (long long*)nodes, status,
-                                                                                            w.active[0], B);
-    }
+    const long long root_blocks = (B + 255) / 256;
+    const unsigned root_grid = (unsigned)(root_blocks > 4096 ? 4096 : root_blocks);
+    hk::hk_search_init_kernel<<<root_grid, 256, 0, st>>>(depth, (long long*)nodes, status, w.active[0], B);
 
     hk::SearchParams p;
     memset(&p, 0, sizeof(p));
@@ -164,10 +181,20 @@ int hk_search_depth(const void* roots, int32_t* depth, int64_t* nodes, int8_t* s
     p.status = status;
     p.child_mask = w.child_mask;
     p.child_axis = w.child_axis;
+    hk::LineParams l;
+    memset(&l, 0, sizeof(l));
+    if (line) {
+        l.h_parent = line->w.h_parent;
+        l.h_set = line->w.h_set;
+        l.h_axis = line->w.h_axis;
+        l.deep = line->w.deep;
+        l.root_ch = line->w.root_ch;
+        l.capacity = capacity;
+    }
 
     const int32_t* state = (const int32_t*)roots;
     const int32_t* node_root = nullptr;  // level 0: node i is root i
-    long long M = B, n_active = B;
+    long long M = B, n_active = B, hist_base = 0;
     for (int level = 0;; ++level) {
         const int next = level & 1;  // frontier, node-root list and root list the next level is written to
         p.state = state;
@@ -185,8 +212,22 @@ int hk_search_depth(const void* roots, int32_t* depth, int64_t* nodes, int8_t* s
             if (rc != HK_OK) return rc;
         }
         const unsigned tiles = (unsigned)((M + hk::SEARCH_THREADS - 1) / hk::SEARCH_THREADS);
+        bool history_cut = false;  // the history room, not the capacity, bounds this level
+        if (line) {
+            l.hist_base = hist_base;
+            l.hist_used = hist_base + M;
+            const long long room = line->history - l.hist_used;
+            history_cut = p.expand && room < capacity;
+            p.capacity = history_cut ? room : capacity;
+            hk::hk_line_deep_kernel<<<tiles, hk::SEARCH_THREADS, 0, st>>>(p, l);
+        }
         hk::hk_search_count_kernel<<<tiles, hk::SEARCH_THREADS, 0, st>>>(p);
+        if (history_cut) {
+            const long long blocks = (n_active + 255) / 256;
+            hk::hk_line_save_kernel<<<(unsigned)(blocks > 4096 ? 4096 : blocks), 256, 0, st>>>(p, l);
+        }
         hk::hk_search_decide_kernel<<<1, hk::SEARCH_SCAN_THREADS, 0, st>>>(p);
+        if (history_cut) hk::hk_line_relabel_kernel<<<1, hk::SEARCH_SCAN_THREADS, 0, st>>>(p, l);
         long long counters[2];
         e = cudaGetLastError();
         if (e == cudaSuccess) e = cudaMemcpyAsync(counters, w.counters, sizeof(counters), cudaMemcpyDeviceToHost, st);
@@ -194,6 +235,7 @@ int hk_search_depth(const void* roots, int32_t* depth, int64_t* nodes, int8_t* s
         if (e != cudaSuccess) return (int)e;
         if (!p.expand || counters[0] == 0) break;
         hk::hk_search_scatter_kernel<<<tiles, hk::SEARCH_THREADS, 0, st>>>(p);
+        if (line) hk::hk_line_history_kernel<<<tiles, hk::SEARCH_THREADS, 0, st>>>(p, l);
         e = cudaGetLastError();
         if (e != cudaSuccess) return (int)e;
         int rc = hk_step(w.frontier[next], w.frontier[next], w.child_mask, w.child_axis, nullptr, nullptr, nullptr, nullptr,
@@ -201,10 +243,80 @@ int hk_search_depth(const void* roots, int32_t* depth, int64_t* nodes, int8_t* s
         if (rc != HK_OK) return rc;
         state = w.frontier[next];
         node_root = w.node_root[next];
+        hist_base += M;
         M = counters[0];
         n_active = counters[1];
     }
+    if (line) {
+        hk::hk_line_depth_walk_kernel<<<root_grid, 256, 0, st>>>(depth, l, line->line_mask, line->line_axis, B, max_depth);
+        e = cudaGetLastError();
+        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+        return (int)e;
+    }
     return (int)cudaGetLastError();
+}
+
+// the checks hk_search_depth and hk_search_depth_line share; HK_OK when the arguments pass
+int depth_args_error(int64_t B, int32_t N, int32_t d, int32_t dtype, uint32_t ops, uint32_t flags, int32_t max_depth,
+                     int64_t max_nodes, int64_t capacity) {
+    if (B < 0 || N < 1 || d < 1 || (dtype != HK_DTYPE_I32 && dtype != HK_DTYPE_F32)) return HK_ERR_BAD_ARG;
+    if (hk_kernel_class(N, d) < 0) return HK_ERR_UNSUPPORTED;
+    if (dtype != HK_DTYPE_I32) return HK_ERR_UNSUPPORTED;  // float32 state is not searched
+    if (flags != HK_F_HOST_ZEILLINGER && flags != HK_F_HOST_ALL_COORD) return HK_ERR_BAD_ARG;
+    if ((ops & (HK_OP_SHIFT | HK_OP_NEWTON)) != (HK_OP_SHIFT | HK_OP_NEWTON) ||
+        (ops & ~(HK_OP_SHIFT | HK_OP_NEWTON | HK_OP_REPOSITION)))
+        return HK_ERR_BAD_ARG;
+    if (max_depth < 1 || max_nodes < 1 || capacity < 1) return HK_ERR_BAD_ARG;
+    return HK_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int64_t hk_search_workspace_bytes(int64_t B, int32_t N, int32_t d, int64_t capacity) {
+    if (B < 0 || N < 1 || d < 1 || capacity < 1) return 0;
+    SearchWorkspace w;
+    return (int64_t)(carve(&w, nullptr, B, N, d, capacity) + 256);  // + 256: room to align the caller's pointer
+}
+
+int hk_search_depth(const void* roots, int32_t* depth, int64_t* nodes, int8_t* status, int64_t B, int32_t N, int32_t d,
+                    int32_t dtype, uint32_t ops, uint32_t flags, int32_t max_depth, int64_t max_nodes, int64_t capacity,
+                    void* workspace, void* stream) {
+    const int bad = depth_args_error(B, N, d, dtype, ops, flags, max_depth, max_nodes, capacity);
+    if (bad != HK_OK) return bad;
+    if (B == 0) return HK_OK;
+    if (!roots || !depth || !nodes || !status || !workspace) return HK_ERR_BAD_ARG;
+    if (((uintptr_t)roots) & 3u) return HK_ERR_ALIGN;
+    SearchWorkspace w;
+    carve(&w, (char*)align_up((size_t)(uintptr_t)workspace), B, N, d, capacity);
+    return run_search_depth(roots, depth, nodes, status, B, N, d, ops, flags, max_depth, max_nodes, capacity, w, nullptr,
+                            stream);
+}
+
+int64_t hk_search_depth_line_workspace_bytes(int64_t B, int32_t N, int32_t d, int64_t capacity, int64_t history) {
+    if (!depth_line_args_ok(B, N, d, capacity, history)) return 0;
+    DepthLineWorkspace w;
+    return (int64_t)(carve_depth_line(&w, nullptr, B, N, d, capacity, history) + 256);  // + 256: room to align
+}
+
+int hk_search_depth_line(const void* roots, int32_t* depth, int64_t* nodes, int8_t* status, int32_t* line_mask,
+                         int32_t* line_axis, int64_t B, int32_t N, int32_t d, int32_t dtype, uint32_t ops,
+                         uint32_t flags, int32_t max_depth, int64_t max_nodes, int64_t capacity, int64_t history,
+                         void* workspace, void* stream) {
+    const int bad = depth_args_error(B, N, d, dtype, ops, flags, max_depth, max_nodes, capacity);
+    if (bad != HK_OK) return bad;
+    if (!depth_line_args_ok(B, N, d, capacity, history)) return HK_ERR_BAD_ARG;
+    if (B == 0) return HK_OK;
+    if (!roots || !depth || !nodes || !status || !line_mask || !line_axis || !workspace) return HK_ERR_BAD_ARG;
+    if (((uintptr_t)roots) & 3u) return HK_ERR_ALIGN;
+    DepthLine line;
+    carve_depth_line(&line.w, (char*)align_up((size_t)(uintptr_t)workspace), B, N, d, capacity, history);
+    line.history = history;
+    line.line_mask = line_mask;
+    line.line_axis = line_axis;
+    return run_search_depth(roots, depth, nodes, status, B, N, d, ops, flags, max_depth, max_nodes, capacity, line.w.s,
+                            &line, stream);
 }
 
 int64_t hk_search_value_workspace_bytes(int64_t B, int32_t N, int32_t d, int64_t capacity, int64_t history) {
@@ -213,9 +325,11 @@ int64_t hk_search_value_workspace_bytes(int64_t B, int32_t N, int32_t d, int64_t
     return (int64_t)(carve_value(&w, nullptr, B, N, d, capacity, history) + 256);  // + 256: room to align the pointer
 }
 
-int hk_search_value(const void* roots, int32_t* value, int32_t* best_mask, int64_t* nodes, int8_t* status, int64_t B,
-                    int32_t N, int32_t d, int32_t dtype, uint32_t ops, int32_t max_depth, int64_t max_nodes,
-                    int64_t capacity, int64_t history, void* workspace, void* stream) {
+// hk_search_value, and hk_search_value_line when `line` is set (the line outputs are then required)
+static int run_search_value(const void* roots, int32_t* value, int32_t* best_mask, int64_t* nodes, int8_t* status,
+                            bool line, int32_t* line_mask, int32_t* line_axis, int64_t B, int32_t N, int32_t d,
+                            int32_t dtype, uint32_t ops, int32_t max_depth, int64_t max_nodes, int64_t capacity,
+                            int64_t history, void* workspace, void* stream) {
     if (B < 0 || N < 1 || d < 1 || (dtype != HK_DTYPE_I32 && dtype != HK_DTYPE_F32)) return HK_ERR_BAD_ARG;
     if (hk_kernel_class(N, d) < 0 || d < 2 || d > 6) return HK_ERR_UNSUPPORTED;  // <= 186 children: a uint8 count
     if (dtype != HK_DTYPE_I32) return HK_ERR_UNSUPPORTED;  // float32 state is not searched
@@ -225,6 +339,7 @@ int hk_search_value(const void* roots, int32_t* value, int32_t* best_mask, int64
     if (max_depth < 1 || max_nodes < 1 || !value_args_ok(B, N, d, capacity, history)) return HK_ERR_BAD_ARG;
     if (B == 0) return HK_OK;
     if (!roots || !value || !best_mask || !nodes || !status || !workspace) return HK_ERR_BAD_ARG;
+    if (line && (!line_mask || !line_axis)) return HK_ERR_BAD_ARG;
     if (((uintptr_t)roots) & 3u) return HK_ERR_ALIGN;
     cudaStream_t st = (cudaStream_t)stream;
     ValueWorkspace w;
@@ -313,9 +428,25 @@ int hk_search_value(const void* roots, int32_t* value, int32_t* best_mask, int64
         n_active = counters[1];
     }
     hk::hk_value_finish_kernel<<<root_grid, 256, 0, st>>>(p);
+    if (line) hk::hk_line_value_walk_kernel<<<root_grid, 256, 0, st>>>(p, p.hist_used, line_mask, line_axis, max_depth);
     e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     return (int)e;
+}
+
+int hk_search_value(const void* roots, int32_t* value, int32_t* best_mask, int64_t* nodes, int8_t* status, int64_t B,
+                    int32_t N, int32_t d, int32_t dtype, uint32_t ops, int32_t max_depth, int64_t max_nodes,
+                    int64_t capacity, int64_t history, void* workspace, void* stream) {
+    return run_search_value(roots, value, best_mask, nodes, status, false, nullptr, nullptr, B, N, d, dtype, ops,
+                            max_depth, max_nodes, capacity, history, workspace, stream);
+}
+
+int hk_search_value_line(const void* roots, int32_t* value, int32_t* best_mask, int64_t* nodes, int8_t* status,
+                         int32_t* line_mask, int32_t* line_axis, int64_t B, int32_t N, int32_t d, int32_t dtype,
+                         uint32_t ops, int32_t max_depth, int64_t max_nodes, int64_t capacity, int64_t history,
+                         void* workspace, void* stream) {
+    return run_search_value(roots, value, best_mask, nodes, status, true, line_mask, line_axis, B, N, d, dtype, ops,
+                            max_depth, max_nodes, capacity, history, workspace, stream);
 }
 
 }  // extern "C"

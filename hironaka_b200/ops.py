@@ -380,6 +380,14 @@ def host_policy(state: torch.Tensor, host: str, padding_value: float = -1.0) -> 
     return mask
 
 
+def _workspace(workspace: Optional[torch.Tensor], need: int, dev) -> torch.Tensor:
+    if workspace is None:
+        return torch.empty(max(need, 1), dtype=torch.uint8, device=dev)
+    if workspace.dtype != torch.uint8 or workspace.numel() < need or workspace.device != dev:
+        raise ValueError(f"workspace must be a uint8 tensor of at least {need} bytes on the roots' device")
+    return workspace
+
+
 def search_workspace_bytes(B: int, N: int, d: int, capacity: int) -> int:
     """Bytes of device workspace `search_depth` needs (hk_search_workspace_bytes)."""
     return int(lib().hk_search_workspace_bytes(B, N, d, capacity))
@@ -394,11 +402,7 @@ def search_depth(roots: torch.Tensor, *, flags: int, ops: int, max_depth: int, m
     dt = _require_state(roots)
     B, N, d = roots.shape
     dev = roots.device
-    need = search_workspace_bytes(B, N, d, capacity)
-    if workspace is None:
-        workspace = torch.empty(max(need, 1), dtype=torch.uint8, device=dev)
-    elif workspace.dtype != torch.uint8 or workspace.numel() < need or workspace.device != dev:
-        raise ValueError(f"workspace must be a uint8 tensor of at least {need} bytes on the roots' device")
+    workspace = _workspace(workspace, search_workspace_bytes(B, N, d, capacity), dev)
     depth = torch.empty(B, dtype=torch.int32, device=dev)
     nodes = torch.empty(B, dtype=torch.int64, device=dev)
     status = torch.empty(B, dtype=torch.int8, device=dev)
@@ -424,11 +428,7 @@ def search_value(roots: torch.Tensor, *, ops: int, max_depth: int, max_nodes: in
     dt = _require_state(roots)
     B, N, d = roots.shape
     dev = roots.device
-    need = search_value_workspace_bytes(B, N, d, capacity, history)
-    if workspace is None:
-        workspace = torch.empty(max(need, 1), dtype=torch.uint8, device=dev)
-    elif workspace.dtype != torch.uint8 or workspace.numel() < need or workspace.device != dev:
-        raise ValueError(f"workspace must be a uint8 tensor of at least {need} bytes on the roots' device")
+    workspace = _workspace(workspace, search_value_workspace_bytes(B, N, d, capacity, history), dev)
     value = torch.empty(B, dtype=torch.int32, device=dev)
     best_mask = torch.empty(B, dtype=torch.int32, device=dev)
     nodes = torch.empty(B, dtype=torch.int64, device=dev)
@@ -440,6 +440,60 @@ def search_value(roots: torch.Tensor, *, ops: int, max_depth: int, max_nodes: in
                                    stream)
     check(rc, "hk_search_value")
     return value, best_mask, nodes, status
+
+
+def search_depth_line_workspace_bytes(B: int, N: int, d: int, capacity: int, history: int) -> int:
+    """Bytes of device workspace `search_depth_line` needs (hk_search_depth_line_workspace_bytes; 0 for refused
+    arguments)."""
+    return int(lib().hk_search_depth_line_workspace_bytes(B, N, d, capacity, history))
+
+
+def search_depth_line(roots: torch.Tensor, *, flags: int, ops: int, max_depth: int, max_nodes: int, capacity: int,
+                      history: int, workspace: Optional[torch.Tensor] = None):
+    """search_depth with the worst line against the fixed host (hk_search_depth_line): (depth [B] int32, nodes [B]
+    int64, status [B] int8, line_mask [B, max_depth] int32, line_axis [B, max_depth] int32).  `workspace` is a uint8
+    tensor of at least search_depth_line_workspace_bytes(B, N, d, capacity, history) bytes on the roots' device
+    (allocated here when None).  Synchronous."""
+    dt = _require_state(roots)
+    B, N, d = roots.shape
+    dev = roots.device
+    workspace = _workspace(workspace, search_depth_line_workspace_bytes(B, N, d, capacity, history), dev)
+    depth = torch.empty(B, dtype=torch.int32, device=dev)
+    nodes = torch.empty(B, dtype=torch.int64, device=dev)
+    status = torch.empty(B, dtype=torch.int8, device=dev)
+    line_mask = torch.empty((B, max(int(max_depth), 0)), dtype=torch.int32, device=dev)
+    line_axis = torch.empty_like(line_mask)
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        rc = lib().hk_search_depth_line(_ptr(roots), _ptr(depth), _ptr(nodes), _ptr(status), _ptr(line_mask),
+                                        _ptr(line_axis), B, N, d, dt, ops, flags, int(max_depth), int(max_nodes),
+                                        int(capacity), int(history), _ptr(workspace), stream)
+    check(rc, "hk_search_depth_line")
+    return depth, nodes, status, line_mask, line_axis
+
+
+def search_value_line(roots: torch.Tensor, *, ops: int, max_depth: int, max_nodes: int, capacity: int, history: int,
+                      workspace: Optional[torch.Tensor] = None):
+    """search_value with an optimal line of every resolved root (hk_search_value_line): (value [B] int32, best_mask [B]
+    int32, nodes [B] int64, status [B] int8, line_mask [B, max_depth] int32, line_axis [B, max_depth] int32).  The
+    workspace is search_value's.  Synchronous."""
+    dt = _require_state(roots)
+    B, N, d = roots.shape
+    dev = roots.device
+    workspace = _workspace(workspace, search_value_workspace_bytes(B, N, d, capacity, history), dev)
+    value = torch.empty(B, dtype=torch.int32, device=dev)
+    best_mask = torch.empty(B, dtype=torch.int32, device=dev)
+    nodes = torch.empty(B, dtype=torch.int64, device=dev)
+    status = torch.empty(B, dtype=torch.int8, device=dev)
+    line_mask = torch.empty((B, max(int(max_depth), 0)), dtype=torch.int32, device=dev)
+    line_axis = torch.empty_like(line_mask)
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        rc = lib().hk_search_value_line(_ptr(roots), _ptr(value), _ptr(best_mask), _ptr(nodes), _ptr(status),
+                                        _ptr(line_mask), _ptr(line_axis), B, N, d, dt, ops, int(max_depth),
+                                        int(max_nodes), int(capacity), int(history), _ptr(workspace), stream)
+    check(rc, "hk_search_value_line")
+    return value, best_mask, nodes, status, line_mask, line_axis
 
 
 def _single_op(fn_name: str, state: torch.Tensor, inplace: bool, padding_value: float) -> Optional[torch.Tensor]:

@@ -7,6 +7,11 @@ frontier capacity.  A root that hits a limit is a normal result, reported in `st
 
 search_value (hk_search_value) answers the minimax question over the same tree with every host move: the fewest moves
 the best host needs to end the game, whatever the agent replies.
+
+search_depth_line and search_value_line return, with the same numbers, a line of play for each root: the agent's
+longest line against the fixed host, and an optimal line of the best host with the agent's best replies.  play_line
+replays lines into the states along them.  Along an optimal line the value drops by one per move, so its states with
+value - t at move t are exact value labels.
 """
 from __future__ import annotations
 
@@ -27,6 +32,8 @@ STATUS_HISTORY = C.HK_SEARCH_HISTORY          # search_value: the next level did
 FRONTIER_BYTES = 1 << 28  # default capacity: one frontier fills 256 MiB
 HISTORY_BYTES = 1 << 32   # search_value's default history: 4 GiB
 HISTORY_NODE_BYTES = 14   # parent, solved round and group count (int32 each), group set and rank (one byte each)
+DEPTH_LINE_NODE_BYTES = 7  # search_depth_line's history: parent (int32), set (16 bits, d <= 10), axis (one byte)
+MAX_HISTORY = (1 << 31) - 1  # parents are int32 entries
 
 
 class SearchResult(NamedTuple):
@@ -108,3 +115,89 @@ def search_value(points: torch.Tensor, *, reposition: bool = True, max_depth: in
     value, best_mask, nodes, status = _ops.search_value(points, ops=step_ops, max_depth=max_depth, max_nodes=max_nodes,
                                                         capacity=cap, history=hist)
     return ValueResult(value, best_mask, nodes, status)
+
+
+class DepthLine(NamedTuple):
+    depth: torch.Tensor   # [B] int32 as SearchResult.depth: the length of the line
+    nodes: torch.Tensor   # [B] int64 as SearchResult.nodes
+    status: torch.Tensor  # [B] int8 STATUS_*
+    mask: torch.Tensor    # [B, max_depth] int32 the host's set at each move; 0 past the line's end
+    axis: torch.Tensor    # [B, max_depth] int32 the agent's axis at each move; -1 past the line's end
+
+
+def default_depth_line_history() -> int:
+    """search_depth_line's history when none is given: HISTORY_BYTES / DEPTH_LINE_NODE_BYTES states, at most
+    MAX_HISTORY."""
+    return min(HISTORY_BYTES // DEPTH_LINE_NODE_BYTES, MAX_HISTORY)
+
+
+def search_depth_line(points: torch.Tensor, host: str = "zeillinger", *, reposition: bool = True, max_depth: int = 64,
+                      max_nodes: int = 1 << 16, capacity: Optional[int] = None,
+                      history: Optional[int] = None) -> DepthLine:
+    """search_depth, and for each root the agent's worst line against the fixed `host`: depth[b] moves (mask, axis),
+    each mask the host's choice on the state it is played on, the axes the lexicographically smallest sequence among
+    the lines that reach level depth[b] of the explored tree.  For a resolved root this is the smallest of the longest
+    games, and it ends at an ended state; for a cut root it is the smallest line to the deepest level explored, whose
+    end need not have ended.
+
+    The search keeps every state of every level in a history of DEPTH_LINE_NODE_BYTES = 7 bytes per state (parent
+    entry int32, set 16 bits, axis one byte), so `history` is one more limit: the states of all levels of the batch,
+    roots included, at most 2^31 - 1 because parents are int32 entries.  The default, default_depth_line_history(), is
+    2^32 / 7 states, 4 GiB.  A root cut by it gets STATUS_HISTORY; the cuts apply in the order of search_value (int32
+    bound, node budget, capacity, history, the last two from the highest root index down).  With a history large enough
+    for the whole search, depth, nodes and status equal search_depth's.  Synchronous."""
+    if host not in ("zeillinger", "all_coord"):
+        raise ValueError(f"host must be 'zeillinger' or 'all_coord'; got {host!r}")
+    B, N, d = points.shape
+    flags = C.HK_F_HOST_ZEILLINGER if host == "zeillinger" else C.HK_F_HOST_ALL_COORD
+    step_ops = C.HK_OP_SHIFT | C.HK_OP_NEWTON | (C.HK_OP_REPOSITION if reposition else 0)
+    cap = default_capacity(N, d) if capacity is None else int(capacity)
+    hist = default_depth_line_history() if history is None else int(history)
+    return DepthLine(*_ops.search_depth_line(points, flags=flags, ops=step_ops, max_depth=max_depth,
+                                             max_nodes=max_nodes, capacity=cap, history=hist))
+
+
+class ValueLine(NamedTuple):
+    value: torch.Tensor      # [B] int32 as ValueResult.value: the length of the line of a resolved root
+    best_mask: torch.Tensor  # [B] int32 as ValueResult.best_mask: the line's first mask
+    nodes: torch.Tensor      # [B] int64
+    status: torch.Tensor     # [B] int8 STATUS_*
+    mask: torch.Tensor       # [B, max_depth] int32 the host's set at each move; 0 past the line's end
+    axis: torch.Tensor       # [B, max_depth] int32 the agent's axis at each move; -1 past the line's end
+
+
+def search_value_line(points: torch.Tensor, *, reposition: bool = True, max_depth: int = 16, max_nodes: int = 1 << 22,
+                      capacity: Optional[int] = None, history: Optional[int] = None) -> ValueLine:
+    """search_value, and for each resolved root of value v > 0 an optimal line of v moves.  From a state of value
+    u > 0 the host plays the smallest S whose children all have value <= u - 1 (best_mask at the root), and the agent
+    the smallest axis of S whose child has value exactly u - 1; the line ends at an ended state.  Roots that had ended
+    and roots with another status than STATUS_RESOLVED get an empty line.  The line is read from the search's own
+    history: the memory and limits are search_value's.  Synchronous."""
+    B, N, d = points.shape
+    step_ops = C.HK_OP_SHIFT | C.HK_OP_NEWTON | (C.HK_OP_REPOSITION if reposition else 0)
+    cap = default_capacity(N, d) if capacity is None else int(capacity)
+    hist = default_history() if history is None else int(history)
+    return ValueLine(*_ops.search_value_line(points, ops=step_ops, max_depth=max_depth, max_nodes=max_nodes,
+                                             capacity=cap, history=hist))
+
+
+def play_line(points: torch.Tensor, mask: torch.Tensor, axis: torch.Tensor, *, reposition: bool = True) -> torch.Tensor:
+    """The states along lines: int32 [B, L + 1, N, d], state t after the first t moves of mask / axis ([B, L] each, as
+    search_depth_line and search_value_line return them), each move the searches' step (shift, reposition if
+    `reposition`, Newton polytope).  Past a line's end (axis -1) the state repeats: such a game is not stepped, since a
+    step with axis -1 would, under reposition, move a lone point to the origin.  One ops.step launch per move."""
+    B, N, d = points.shape
+    L = mask.shape[1]
+    if mask.shape != (B, L) or axis.shape != (B, L):
+        raise ValueError(f"mask and axis must both be [{B}, L]; got {tuple(mask.shape)} and {tuple(axis.shape)}")
+    step_ops = C.HK_OP_SHIFT | C.HK_OP_NEWTON | (C.HK_OP_REPOSITION if reposition else 0)
+    mask = mask.to(points.device, torch.int32)
+    axis = axis.to(points.device, torch.int32)
+    out = torch.empty((B, L + 1, N, d), dtype=points.dtype, device=points.device)
+    out[:, 0] = points
+    for t in range(L):
+        out[:, t + 1] = out[:, t]
+        idx = torch.nonzero(axis[:, t] >= 0).flatten()
+        if len(idx):
+            out[idx, t + 1] = _ops.step(out[idx, t].contiguous(), mask[idx, t], axis[idx, t], ops=step_ops).state
+    return out

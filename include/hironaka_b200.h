@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define HK_VERSION 104 /* major*100 + minor */
+#define HK_VERSION 105 /* major*100 + minor */
 
 /* ---- status codes ---------------------------------------------------------------- */
 #define HK_OK 0
@@ -283,6 +283,41 @@ int64_t hk_search_value_workspace_bytes(int64_t B, int32_t N, int32_t d, int64_t
 int hk_search_value(const void* roots, int32_t* value, int32_t* best_mask, int64_t* nodes, int8_t* status, int64_t B,
                     int32_t N, int32_t d, int32_t dtype, uint32_t ops, int32_t max_depth, int64_t max_nodes,
                     int64_t capacity, int64_t history, void* workspace, void* stream);
+
+/* ---- lines of play from the searches ---------------------------------------------------------
+ * A line is a sequence of moves (host coordinate bitmask S, agent axis), each the JAX step of the searches (shift,
+ * reposition if HK_OP_REPOSITION, Newton polytope, flags 0, padding -1).  line_mask and line_axis are [B, max_depth]
+ * int32; entries past a root's line length hold mask 0 and axis -1.
+ *
+ * hk_search_depth_line: hk_search_depth with the WORST LINE against the fixed host.  Its length is depth[b]; every mask
+ * is hk_host_policy (same flags) of the state it is played on; the axes are the lexicographically smallest sequence
+ * among the lines that reach level depth[b] of the explored tree.  For a RESOLVED root it is the smallest of the
+ * longest games and ends at an ended state; for a cut root it is the smallest line to its deepest explored level,
+ * which need not have ended.  The search keeps a history of every state of the batch (the parent's entry, int32, and
+ * the set, 16 bits, and the axis, one byte: 7 bytes per state), so `history` is one more limit: the states of all levels of the
+ * batch, roots included.  The cuts apply in the order INT32_BOUND, MAX_NODES, CAPACITY, HISTORY, the last two dropping
+ * roots from the highest index down, as in hk_search_value; a root cut by the history gets HK_SEARCH_HISTORY.  With a
+ * history large enough for the whole search, depth, nodes and status equal hk_search_depth's.
+ * workspace: hk_search_depth_line_workspace_bytes(B, N, d, capacity, history) bytes (hk_search_depth's, 7 bytes per
+ * history state and 12 per root); it returns 0 for arguments hk_search_depth_line refuses.
+ * Errors: those of hk_search_depth; history < max(B, 1) or > 2^31 - 1, null line outputs: HK_ERR_BAD_ARG.
+ *
+ * hk_search_value_line: hk_search_value with an OPTIMAL LINE for each RESOLVED root of value v > 0, of length v.  From a
+ * state of value u > 0 the host plays the smallest S whose children all have value <= u - 1 (at the root, best_mask),
+ * and the agent the smallest axis of S whose child has value exactly u - 1; the line ends at an ended state.  Roots
+ * that ended on entry and roots whose status is not RESOLVED get an empty line.  Every state of the line is solved in
+ * the root's round, so these are read from the search's own history: no extra memory, the workspace of
+ * hk_search_value.  value, best_mask, nodes and status equal hk_search_value's.
+ * Errors: those of hk_search_value; null line outputs: HK_ERR_BAD_ARG.  Both calls are SYNCHRONOUS. */
+int64_t hk_search_depth_line_workspace_bytes(int64_t B, int32_t N, int32_t d, int64_t capacity, int64_t history);
+int hk_search_depth_line(const void* roots, int32_t* depth, int64_t* nodes, int8_t* status, int32_t* line_mask,
+                         int32_t* line_axis, int64_t B, int32_t N, int32_t d, int32_t dtype, uint32_t ops,
+                         uint32_t flags, int32_t max_depth, int64_t max_nodes, int64_t capacity, int64_t history,
+                         void* workspace, void* stream);
+int hk_search_value_line(const void* roots, int32_t* value, int32_t* best_mask, int64_t* nodes, int8_t* status,
+                         int32_t* line_mask, int32_t* line_axis, int64_t B, int32_t N, int32_t d, int32_t dtype,
+                         uint32_t ops, int32_t max_depth, int64_t max_nodes, int64_t capacity, int64_t history,
+                         void* workspace, void* stream);
 
 /* ---- multi-step rollout ------------------------------------------------------------------
  * T consecutive steps with the state held on chip between steps: one read and one write of
