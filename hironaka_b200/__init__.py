@@ -13,6 +13,7 @@ Layers (bottom up):
   search_depth     game-tree search of a fixed host against every agent reply (hironaka/util/search.py)
   search_value     game value: the shortest game the best host can force against every agent reply
   search_*_line    the same searches with a line of play per root; play_line replays lines into states
+  search_value_labels  every state the value search solved: exact value, optimal host moves, path and rows
 """
 from . import constants
 from .constants import *  # noqa: F401,F403
@@ -45,7 +46,8 @@ def __getattr__(name):  # lazy: importing the package must not require torch or 
         return getattr(vec_env, name)
     if name in ("search_depth", "SearchResult", "STATUS_RESOLVED", "STATUS_MAX_DEPTH", "STATUS_MAX_NODES",
                 "STATUS_CAPACITY", "STATUS_INT32_BOUND", "search_value", "ValueResult", "STATUS_HISTORY",
-                "search_depth_line", "DepthLine", "search_value_line", "ValueLine", "play_line"):
+                "search_depth_line", "DepthLine", "search_value_line", "ValueLine", "play_line", "search_value_labels",
+                "ValueLabels"):
         from . import search
         return getattr(search, name)
     if name == "HostActionEncoder":

@@ -55,6 +55,9 @@ SIGNATURES = {
                                             _p, _p]),
     "hk_search_value_line": (ctypes.c_int, [_p, _p, _p, _p, _p, _p, _p, _i64, _i32, _i32, _i32, _u32, _i32, _i64, _i64, _i64,
                                             _p, _p]),
+    "hk_search_value_labels_workspace_bytes": (_i64, [_i64, _i32, _i32, _i64, _i64]),
+    "hk_search_value_labels": (ctypes.c_int, [_p, _p, _p, _p, _p, _i64, _p, _p, _p, _p, _p, _p, _p, _i64, _i32, _i32, _i32,
+                                              _u32, _i32, _i64, _i64, _i64, _p, _p]),
     "hk_experience_scratch_words": (_i64, [_i64]),
     "hk_experience_append": (ctypes.c_int, [_p, _p, _p, _i32, _p, _p, _i32, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _p, _p,
                                             _p, _p, _i64, _p]),

@@ -26,7 +26,7 @@ SOURCES = ["hk_capi.cu", "hk_small_i32_step.cu", "hk_small_i32_obs.cu", "hk_smal
            "hk_small_i32_thr.cu", "hk_small_f32_thr.cu", "hk_generic_i32_thr.cu", "hk_generic_f32_thr.cu",
            "hk_search.cu"]
 HEADERS = ["hk_common.cuh", "hk_census.cuh", "hk_small.cuh", "hk_generic.cuh", "hk_experience.cuh", "hk_value.cuh", "hk_launch.cuh",
-           "hk_small_launch.inl", "hk_generic_launch.inl", "hk_sched.cuh", "hk_sched_launch.inl", "hk_rows.cuh", "hk_rows_launch.inl", "hk_sortnet.inc", "hk_search.cuh", "hk_minimax.cuh", "hk_lines.cuh", os.path.join("..", "..", "include", "hironaka_b200.h")]
+           "hk_small_launch.inl", "hk_generic_launch.inl", "hk_sched.cuh", "hk_sched_launch.inl", "hk_rows.cuh", "hk_rows_launch.inl", "hk_sortnet.inc", "hk_search.cuh", "hk_minimax.cuh", "hk_lines.cuh", "hk_labels.cuh", os.path.join("..", "..", "include", "hironaka_b200.h")]
 
 ARCH_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMPILE_FLAGS = ARCH_FLAGS + ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "-c"]

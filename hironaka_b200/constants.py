@@ -1,7 +1,7 @@
 """Constants of the C-ABI (mirror of include/hironaka_b200.h; tests/test_capi_cpu.py checks
 that the two stay identical)."""
 
-HK_VERSION = 105
+HK_VERSION = 106
 
 HK_OK = 0
 HK_ERR_BAD_ARG = -1

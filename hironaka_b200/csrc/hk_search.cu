@@ -1,15 +1,17 @@
 // hk_search.cu — hk_search_workspace_bytes and hk_search_depth, hk_search_value_workspace_bytes and hk_search_value,
-// and their line forms hk_search_depth_line_workspace_bytes, hk_search_depth_line and hk_search_value_line
-// (include/hironaka_b200.h): the level loops of the game-tree searches.  Every level of hk_search_depth runs
-// hk_host_policy on the frontier and the three bookkeeping kernels of hk_search.cuh; every level of hk_search_value runs
-// the four kernels of hk_minimax.cuh.  Both then run hk_step in place on the children, through the same C-ABI entry
+// their line forms hk_search_depth_line_workspace_bytes, hk_search_depth_line and hk_search_value_line, and the value
+// labels hk_search_value_labels_workspace_bytes and hk_search_value_labels (include/hironaka_b200.h): the level loops
+// of the game-tree searches.  Every level of hk_search_depth runs hk_host_policy on the frontier and the three
+// bookkeeping kernels of hk_search.cuh; every level of hk_search_value runs the four kernels of hk_minimax.cuh.  Both then run hk_step in place on the children, through the same C-ABI entry
 // point a caller would use, so the children are bit for bit what hk_step makes of them on either kernel family.  The
-// line forms run the same loops plus the kernels of hk_lines.cuh.
+// line forms run the same loops plus the kernels of hk_lines.cuh, the value labels hk_search_value's loop plus the
+// kernels of hk_labels.cuh.
 #include <cuda_runtime.h>
 
 #include <cstring>
 
 #include "../../include/hironaka_b200.h"
+#include "hk_labels.cuh"
 #include "hk_lines.cuh"
 #include "hk_minimax.cuh"
 #include "hk_search.cuh"
@@ -105,6 +107,43 @@ size_t carve_value(ValueWorkspace* w, char* base, long long B, int N, int d, lon
     w->h_rank = (uint8_t*)take((size_t)history);
     return off;
 }
+
+// the workspace of hk_search_value_labels: hk_search_value's, then the label scan (the order of
+// hk_search_value_labels_workspace_bytes)
+struct LabelWorkspace {
+    ValueWorkspace v;
+    long long* tile_sum;   // [ceil(history / SEARCH_THREADS)]
+    long long* block_sum;  // [ceil(tiles / SEARCH_SCAN_THREADS)]
+    long long* total;      // [1]
+    int32_t* tile_level;   // [ceil(history / SEARCH_THREADS)]
+};
+
+size_t carve_labels(LabelWorkspace* w, char* base, long long B, int N, int d, long long capacity, long long history) {
+    size_t off = carve_value(&w->v, base, B, N, d, capacity, history);
+    auto take = [&](size_t bytes) {
+        char* ptr = base ? base + off : nullptr;
+        off += align_up(bytes);
+        return ptr;
+    };
+    const long long tiles = (history + hk::SEARCH_THREADS - 1) / hk::SEARCH_THREADS;
+    w->tile_sum = (long long*)take((size_t)tiles * 8);
+    w->block_sum = (long long*)take((size_t)((tiles + hk::SEARCH_SCAN_THREADS - 1) / hk::SEARCH_SCAN_THREADS) * 8);
+    w->total = (long long*)take(8);
+    w->tile_level = (int32_t*)take((size_t)tiles * 4);
+    return off;
+}
+
+// the outputs of hk_search_value_labels
+struct LabelOutputs {
+    long long max_labels;
+    int64_t* count;  // host
+    int32_t* root;
+    int32_t* level;
+    int32_t* value;
+    uint64_t* optimal;
+    int32_t* mask;
+    int32_t* axis;
+};
 
 bool value_args_ok(long long B, int N, int d, long long capacity, long long history) {
     return B >= 0 && N >= 1 && d >= 2 && d <= 6 && capacity >= 1 && history >= 1 && history >= B &&
@@ -325,11 +364,12 @@ int64_t hk_search_value_workspace_bytes(int64_t B, int32_t N, int32_t d, int64_t
     return (int64_t)(carve_value(&w, nullptr, B, N, d, capacity, history) + 256);  // + 256: room to align the pointer
 }
 
-// hk_search_value, and hk_search_value_line when `line` is set (the line outputs are then required)
+// hk_search_value, hk_search_value_line when `line` is set (the line outputs are then required), and
+// hk_search_value_labels when `labels` is set (the workspace is then hk_search_value_labels_workspace_bytes')
 static int run_search_value(const void* roots, int32_t* value, int32_t* best_mask, int64_t* nodes, int8_t* status,
-                            bool line, int32_t* line_mask, int32_t* line_axis, int64_t B, int32_t N, int32_t d,
-                            int32_t dtype, uint32_t ops, int32_t max_depth, int64_t max_nodes, int64_t capacity,
-                            int64_t history, void* workspace, void* stream) {
+                            bool line, int32_t* line_mask, int32_t* line_axis, const LabelOutputs* labels, int64_t B,
+                            int32_t N, int32_t d, int32_t dtype, uint32_t ops, int32_t max_depth, int64_t max_nodes,
+                            int64_t capacity, int64_t history, void* workspace, void* stream) {
     if (B < 0 || N < 1 || d < 1 || (dtype != HK_DTYPE_I32 && dtype != HK_DTYPE_F32)) return HK_ERR_BAD_ARG;
     if (hk_kernel_class(N, d) < 0 || d < 2 || d > 6) return HK_ERR_UNSUPPORTED;  // <= 186 children: a uint8 count
     if (dtype != HK_DTYPE_I32) return HK_ERR_UNSUPPORTED;  // float32 state is not searched
@@ -337,6 +377,13 @@ static int run_search_value(const void* roots, int32_t* value, int32_t* best_mas
         (ops & ~(HK_OP_SHIFT | HK_OP_NEWTON | HK_OP_REPOSITION)))
         return HK_ERR_BAD_ARG;
     if (max_depth < 1 || max_nodes < 1 || !value_args_ok(B, N, d, capacity, history)) return HK_ERR_BAD_ARG;
+    if (labels) {
+        if (labels->max_labels < 0 || !labels->count) return HK_ERR_BAD_ARG;
+        if (labels->max_labels > 0 && (!labels->root || !labels->level || !labels->value || !labels->optimal ||
+                                       !labels->mask || !labels->axis))
+            return HK_ERR_BAD_ARG;
+        *labels->count = 0;
+    }
     if (B == 0) return HK_OK;
     if (!roots || !value || !best_mask || !nodes || !status || !workspace) return HK_ERR_BAD_ARG;
     if (line && (!line_mask || !line_axis)) return HK_ERR_BAD_ARG;
@@ -429,6 +476,43 @@ static int run_search_value(const void* roots, int32_t* value, int32_t* best_mas
     }
     hk::hk_value_finish_kernel<<<root_grid, 256, 0, st>>>(p);
     if (line) hk::hk_line_value_walk_kernel<<<root_grid, 256, 0, st>>>(p, p.hist_used, line_mask, line_axis, max_depth);
+    if (labels) {
+        LabelWorkspace lw;
+        carve_labels(&lw, (char*)align_up((size_t)(uintptr_t)workspace), B, N, d, capacity, history);
+        hk::LabelParams q;
+        memset(&q, 0, sizeof(q));
+        q.used = p.hist_used;
+        q.tile_sum = lw.tile_sum;
+        q.block_sum = lw.block_sum;
+        q.total = lw.total;
+        q.tile_level = lw.tile_level;
+        q.max_labels = labels->max_labels;
+        q.max_depth = max_depth;
+        q.root = labels->root;
+        q.level = labels->level;
+        q.value = labels->value;
+        q.optimal = (unsigned long long*)labels->optimal;
+        q.mask = labels->mask;
+        q.axis = labels->axis;
+        const long long tiles = (q.used + hk::SEARCH_THREADS - 1) / hk::SEARCH_THREADS;
+        const long long blocks = (tiles + hk::SEARCH_SCAN_THREADS - 1) / hk::SEARCH_SCAN_THREADS;
+        const unsigned tile_grid = (unsigned)((tiles + 255) / 256);
+        hk::hk_label_level_kernel<<<tile_grid, 256, 0, st>>>(p, q, tiles);
+        hk::hk_label_count_kernel<<<(unsigned)tiles, hk::SEARCH_THREADS, 0, st>>>(p, q);
+        hk::hk_label_scan_tiles_kernel<<<(unsigned)blocks, hk::SEARCH_SCAN_THREADS, 0, st>>>(q, tiles);
+        hk::hk_label_scan_blocks_kernel<<<1, hk::SEARCH_SCAN_THREADS, 0, st>>>(q, blocks);
+        if (q.max_labels > 0) {
+            const long long warps = hk::SEARCH_THREADS / 32;  // one warp per tile
+            const unsigned grid = (unsigned)((tiles + warps - 1) / warps);
+            hk::hk_label_write_kernel<<<grid, hk::SEARCH_THREADS, 0, st>>>(p, q, tiles);
+        }
+        long long total = 0;
+        e = cudaGetLastError();
+        if (e == cudaSuccess) e = cudaMemcpyAsync(&total, lw.total, sizeof(total), cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+        if (e == cudaSuccess) *labels->count = total;
+        return (int)e;
+    }
     e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     return (int)e;
@@ -437,16 +521,33 @@ static int run_search_value(const void* roots, int32_t* value, int32_t* best_mas
 int hk_search_value(const void* roots, int32_t* value, int32_t* best_mask, int64_t* nodes, int8_t* status, int64_t B,
                     int32_t N, int32_t d, int32_t dtype, uint32_t ops, int32_t max_depth, int64_t max_nodes,
                     int64_t capacity, int64_t history, void* workspace, void* stream) {
-    return run_search_value(roots, value, best_mask, nodes, status, false, nullptr, nullptr, B, N, d, dtype, ops,
-                            max_depth, max_nodes, capacity, history, workspace, stream);
+    return run_search_value(roots, value, best_mask, nodes, status, false, nullptr, nullptr, nullptr, B, N, d, dtype,
+                            ops, max_depth, max_nodes, capacity, history, workspace, stream);
 }
 
 int hk_search_value_line(const void* roots, int32_t* value, int32_t* best_mask, int64_t* nodes, int8_t* status,
                          int32_t* line_mask, int32_t* line_axis, int64_t B, int32_t N, int32_t d, int32_t dtype,
                          uint32_t ops, int32_t max_depth, int64_t max_nodes, int64_t capacity, int64_t history,
                          void* workspace, void* stream) {
-    return run_search_value(roots, value, best_mask, nodes, status, true, line_mask, line_axis, B, N, d, dtype, ops,
-                            max_depth, max_nodes, capacity, history, workspace, stream);
+    return run_search_value(roots, value, best_mask, nodes, status, true, line_mask, line_axis, nullptr, B, N, d, dtype,
+                            ops, max_depth, max_nodes, capacity, history, workspace, stream);
+}
+
+int64_t hk_search_value_labels_workspace_bytes(int64_t B, int32_t N, int32_t d, int64_t capacity, int64_t history) {
+    if (!value_args_ok(B, N, d, capacity, history)) return 0;
+    LabelWorkspace w;
+    return (int64_t)(carve_labels(&w, nullptr, B, N, d, capacity, history) + 256);  // + 256: room to align the pointer
+}
+
+int hk_search_value_labels(const void* roots, int32_t* value, int32_t* best_mask, int64_t* nodes, int8_t* status,
+                           int64_t max_labels, int64_t* label_count, int32_t* label_root, int32_t* label_level,
+                           int32_t* label_value, uint64_t* label_optimal, int32_t* label_mask, int32_t* label_axis,
+                           int64_t B, int32_t N, int32_t d, int32_t dtype, uint32_t ops, int32_t max_depth,
+                           int64_t max_nodes, int64_t capacity, int64_t history, void* workspace, void* stream) {
+    const LabelOutputs labels{max_labels, label_count, label_root, label_level, label_value, label_optimal, label_mask,
+                              label_axis};
+    return run_search_value(roots, value, best_mask, nodes, status, false, nullptr, nullptr, &labels, B, N, d, dtype,
+                            ops, max_depth, max_nodes, capacity, history, workspace, stream);
 }
 
 }  // extern "C"

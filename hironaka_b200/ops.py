@@ -6,6 +6,7 @@ CPU or through torch ops, and nothing falls back: a CPU tensor or a missing libr
 """
 from __future__ import annotations
 
+import ctypes
 from typing import List, NamedTuple, Optional, Sequence, Union
 
 import torch
@@ -494,6 +495,48 @@ def search_value_line(roots: torch.Tensor, *, ops: int, max_depth: int, max_node
                                         int(max_nodes), int(capacity), int(history), _ptr(workspace), stream)
     check(rc, "hk_search_value_line")
     return value, best_mask, nodes, status, line_mask, line_axis
+
+
+def search_value_labels_workspace_bytes(B: int, N: int, d: int, capacity: int, history: int) -> int:
+    """Bytes of device workspace `search_value_labels` needs (hk_search_value_labels_workspace_bytes; 0 for refused
+    arguments)."""
+    return int(lib().hk_search_value_labels_workspace_bytes(B, N, d, capacity, history))
+
+
+def search_value_labels(roots: torch.Tensor, *, ops: int, max_depth: int, max_nodes: int, capacity: int, history: int,
+                        max_labels: int, workspace: Optional[torch.Tensor] = None):
+    """search_value with every solved state of value >= 1 as a label (hk_search_value_labels): (value [B] int32,
+    best_mask [B] int32, nodes [B] int64, status [B] int8, count, root [K] int32, level [K] int32, label_value [K]
+    int32, optimal [K] int64, mask [K, max_depth] int32, axis [K, max_depth] int32), `count` the number of labels (a
+    Python int) and K = min(count, max_labels), the first labels in history order.  Bit g of `optimal` is set when the
+    host move of action id g is optimal.  `workspace` is a uint8 tensor of at least
+    search_value_labels_workspace_bytes(B, N, d, capacity, history) bytes on the roots' device (allocated here when
+    None).  Synchronous."""
+    dt = _require_state(roots)
+    B, N, d = roots.shape
+    dev = roots.device
+    workspace = _workspace(workspace, search_value_labels_workspace_bytes(B, N, d, capacity, history), dev)
+    value = torch.empty(B, dtype=torch.int32, device=dev)
+    best_mask = torch.empty(B, dtype=torch.int32, device=dev)
+    nodes = torch.empty(B, dtype=torch.int64, device=dev)
+    status = torch.empty(B, dtype=torch.int8, device=dev)
+    L = max(int(max_labels), 0)
+    root, level, label_value = (torch.empty(L, dtype=torch.int32, device=dev) for _ in range(3))
+    optimal = torch.empty(L, dtype=torch.int64, device=dev)
+    mask = torch.empty((L, max(int(max_depth), 0)), dtype=torch.int32, device=dev)
+    axis = torch.empty_like(mask)
+    count = ctypes.c_int64(0)
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        rc = lib().hk_search_value_labels(_ptr(roots), _ptr(value), _ptr(best_mask), _ptr(nodes), _ptr(status),
+                                          int(max_labels), ctypes.addressof(count), _ptr(root), _ptr(level),
+                                          _ptr(label_value), _ptr(optimal), _ptr(mask), _ptr(axis), B, N, d, dt, ops,
+                                          int(max_depth), int(max_nodes), int(capacity), int(history),
+                                          _ptr(workspace), stream)
+    check(rc, "hk_search_value_labels")
+    K = min(count.value, L)
+    return (value, best_mask, nodes, status, count.value, root[:K], level[:K], label_value[:K], optimal[:K], mask[:K],
+            axis[:K])
 
 
 def _single_op(fn_name: str, state: torch.Tensor, inplace: bool, padding_value: float) -> Optional[torch.Tensor]:

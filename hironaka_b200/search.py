@@ -12,6 +12,10 @@ search_depth_line and search_value_line return, with the same numbers, a line of
 longest line against the fixed host, and an optimal line of the best host with the agent's best replies.  play_line
 replays lines into the states along them.  Along an optimal line the value drops by one per move, so its states with
 value - t at move t are exact value labels.
+
+search_value_labels returns far more such labels: every state the value search solved with a value of at least one,
+under resolved roots and cut ones alike, with its exact value, every optimal host move (as HostActionEncoder ids) and
+its rows.
 """
 from __future__ import annotations
 
@@ -201,3 +205,55 @@ def play_line(points: torch.Tensor, mask: torch.Tensor, axis: torch.Tensor, *, r
         if len(idx):
             out[idx, t + 1] = _ops.step(out[idx, t].contiguous(), mask[idx, t], axis[idx, t], ops=step_ops).state
     return out
+
+
+class ValueLabels(NamedTuple):
+    value: torch.Tensor        # [B] int32 as ValueResult
+    best_mask: torch.Tensor    # [B] int32
+    nodes: torch.Tensor        # [B] int64
+    status: torch.Tensor       # [B] int8 STATUS_*
+    count: int                 # labels found; the tensors below hold the first K = min(count, max_labels)
+    root: torch.Tensor         # [K] int32 the root the state lies under
+    level: torch.Tensor        # [K] int32 moves from the root (non-decreasing over the labels)
+    label_value: torch.Tensor  # [K] int32 the state's exact value, >= 1
+    optimal: torch.Tensor      # [K, 2^d - d - 1] bool column g: the host move of HostActionEncoder id g is optimal
+    mask: torch.Tensor         # [K, max_depth] int32 the host's set at each move from the root; 0 past the level
+    axis: torch.Tensor         # [K, max_depth] int32 the agent's axis at each move from the root; -1 past the level
+    state: torch.Tensor        # [K, N, d] int32 the state
+
+
+def search_value_labels(points: torch.Tensor, *, reposition: bool = True, max_depth: int = 16,
+                        max_nodes: int = 1 << 22, capacity: Optional[int] = None, history: Optional[int] = None,
+                        max_labels: int = 1 << 22) -> ValueLabels:
+    """search_value, and every state it solved with a value of at least one, as training labels.
+
+    A state of level l solved in round R has the exact value R - l: once a state is solved its subtree stops growing,
+    so nothing below it is solved later.  This holds under every root, whatever its status, so roots cut by a limit
+    contribute labels too.  The optimal host moves of such a state are exactly its groups whose children were all
+    solved; column g of `optimal` is the set of HostActionEncoder id g (the sets with |S| >= 2 in increasing bitmask
+    order, the order of host_action.action_masks).  Each label also has its root, its level, its path from the root
+    (mask, axis) and its rows, replayed from the root with the searches' step.
+
+    Labels are in the order of the search's history: level non-decreasing and, within a level, root non-decreasing.
+    `count` is the number found; the first min(count, max_labels) are returned.  Equal states reached by different
+    paths are separate labels.  Memory and limits are search_value's, plus 12 bytes per 256 history states for the
+    label scan and the outputs (about 4 * (2 * max_depth + 4) bytes per label and N * d * 4 for its rows).
+    Synchronous."""
+    B, N, d = points.shape
+    step_ops = C.HK_OP_SHIFT | C.HK_OP_NEWTON | (C.HK_OP_REPOSITION if reposition else 0)
+    cap = default_capacity(N, d) if capacity is None else int(capacity)
+    hist = default_history() if history is None else int(history)
+    (value, best_mask, nodes, status, count, root, level, label_value, optimal, mask,
+     axis) = _ops.search_value_labels(points, ops=step_ops, max_depth=max_depth, max_nodes=max_nodes, capacity=cap,
+                                      history=hist, max_labels=max_labels)
+    ids = torch.arange((1 << d) - d - 1, dtype=torch.int64, device=points.device)
+    optimal = ((optimal[:, None] >> ids) & 1).bool()
+    state = points[root.long()]
+    # the labels with level > t are a suffix: one step per level advances exactly them
+    starts = torch.searchsorted(level, torch.arange(1, max_depth + 1, dtype=torch.int32, device=points.device),
+                                right=False).tolist()
+    for t, start in enumerate(starts):
+        if start == len(level):
+            break
+        _ops.step(state[start:], mask[start:, t], axis[start:, t], ops=step_ops)
+    return ValueLabels(value, best_mask, nodes, status, count, root, level, label_value, optimal, mask, axis, state)

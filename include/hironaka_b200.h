@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define HK_VERSION 105 /* major*100 + minor */
+#define HK_VERSION 106 /* major*100 + minor */
 
 /* ---- status codes ---------------------------------------------------------------- */
 #define HK_OK 0
@@ -318,6 +318,34 @@ int hk_search_value_line(const void* roots, int32_t* value, int32_t* best_mask, 
                          int32_t* line_mask, int32_t* line_axis, int64_t B, int32_t N, int32_t d, int32_t dtype,
                          uint32_t ops, int32_t max_depth, int64_t max_nodes, int64_t capacity, int64_t history,
                          void* workspace, void* stream);
+
+/* ---- value labels from the game-value search ---------------------------------------------------
+ * hk_search_value_labels: hk_search_value, then every state of its history that was SOLVED with value >= 1, whatever
+ * its root's status.  A state of level l solved in round R has the exact value R - l (no state below a solved state is
+ * solved in a later round), and its OPTIMAL host moves are exactly its groups whose children are all solved (a group
+ * with an unsolved child has a value above R - l).  value, best_mask, nodes and status equal hk_search_value's.
+ * Outputs:
+ *   *label_count   HOST int64: the number of labels, also when it exceeds max_labels
+ *   the first min(count, max_labels) labels in history order (level non-decreasing, within a level root
+ *   non-decreasing); entries past them are not written:
+ *   label_root     [max_labels] int32: the root the state lies under
+ *   label_level    [max_labels] int32: its level, the moves from the root
+ *   label_value    [max_labels] int32: its value
+ *   label_optimal  [max_labels] uint64: bit g is set when the host move with action id g (the sets with |S| >= 2 in
+ *                  increasing bitmask order: 57 at d = 6) is optimal
+ *   label_mask, label_axis [max_labels, max_depth] int32: the moves from the root to the state; mask 0 and axis -1
+ *                  past the label's level, as the lines.
+ * Equal states reached by different paths are separate labels.  max_labels == 0 counts only; the label pointers may
+ * then be null.  workspace: hk_search_value_labels_workspace_bytes(B, N, d, capacity, history) bytes: hk_search_value's
+ * and 12 bytes per 256 history states; it returns 0 for arguments hk_search_value refuses.  SYNCHRONOUS.
+ * Errors: those of hk_search_value; max_labels < 0, a null label_count, a null label output with max_labels > 0:
+ * HK_ERR_BAD_ARG. */
+int64_t hk_search_value_labels_workspace_bytes(int64_t B, int32_t N, int32_t d, int64_t capacity, int64_t history);
+int hk_search_value_labels(const void* roots, int32_t* value, int32_t* best_mask, int64_t* nodes, int8_t* status,
+                           int64_t max_labels, int64_t* label_count, int32_t* label_root, int32_t* label_level,
+                           int32_t* label_value, uint64_t* label_optimal, int32_t* label_mask, int32_t* label_axis,
+                           int64_t B, int32_t N, int32_t d, int32_t dtype, uint32_t ops, int32_t max_depth,
+                           int64_t max_nodes, int64_t capacity, int64_t history, void* workspace, void* stream);
 
 /* ---- multi-step rollout ------------------------------------------------------------------
  * T consecutive steps with the state held on chip between steps: one read and one write of
